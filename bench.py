@@ -19,6 +19,9 @@ scaling), the batch replicated, GPI's max over policies exchanged as packed int6
   gpu_eager_baseline : the port's eager-PyTorch op sequence on cuda:0 -- the honest GPU comparator (SURVEY 8d)
   configs      secondary lines for BASELINE configs 1, 4 (i)/(ii), 5 (config 3 = gpi_eval), each with its CPU figure
   shard_check  (world > 1) sharded == unsharded: GPI keys bit-equal, losses / weights within the mode's tolerance
+
+--dump-outputs DIR writes the last timed step's losses and updated parameters as .npy files (seeded inputs: two builds run with
+the same arguments can be compared output for output).
 """
 import argparse
 import contextlib
@@ -636,6 +639,38 @@ def shard_check(cfg, n_local, precision, rank, world, dev, K=3):
     return res
 
 
+DUMP_MAX_BYTES = 60 << 20          # --dump-outputs: array data; with the .npy headers the files stay under 64 MB
+
+
+def step_outputs(losses, lib, n_local):
+    """
+    What one all-task step computed, as float32 host arrays: the losses update_successor_all returned ([n_local][3]: loss,
+    psi loss, phi loss) and the parameters it updated -- the packed online psi rows, w, g of the local policies and the shared h.
+    """
+    out = {'losses': losses, 'psi_online': lib.online[:n_local], 'w': lib.w[:n_local], 'g': lib.g[:n_local], 'h': lib.h}
+    return {k: v.detach().float().cpu().numpy() for k, v in out.items()}
+
+
+def write_outputs(arrays, dirname, max_bytes=DUMP_MAX_BYTES):
+    """
+    DIR/<name>.npy per array.  When the arrays hold more than max_bytes in all, the largest ones are cut down to a fixed, seeded
+    sample of their elements (flattened, in index order) so the total fits: the same shapes always give the same sample.
+    """
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    sizes = {k: a.nbytes for k, a in arrays.items()}
+    budget = max_bytes
+    for i, k in enumerate(sorted(arrays, key=lambda k: sizes[k])):          # smallest first: each takes at most a fair share
+        a = arrays[k]
+        share = budget // (len(arrays) - i)
+        if a.nbytes > share:
+            keep = share // a.itemsize
+            idx = np.sort(np.random.default_rng(SEED).choice(a.size, keep, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(dirname, k + '.npy'), a)
+        budget -= a.nbytes
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -651,7 +686,12 @@ def main():
                     help='flush: 256 MiB write between timed steps (everything cold, weights included); inputs: cycle through '
                          'more distinct resident batches than fit in L2 (inputs cold, weights stay L2-resident)')
     ap.add_argument('--precision', default='bf16', choices=['bf16', 'fp32', 'tf32', 'tf32x3'])
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one computed (losses, updated parameters; rank 0\'s policies) '
+                         'as DIR/<name>.npy, float32, at most 64 MB in all; inputs are seeded, so two builds compare output for output')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     cfg = dict(WORKLOADS[args.workload])
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
@@ -705,6 +745,7 @@ def main():
     plan_key = lib.last_plan_key
     launches = None
     stream_ms = None
+    outputs = None                                                  # --dump-outputs: the last timed step's results
     if args.l2 == 'inputs':
         # The K timed steps as ONE stream of work between two events (inputs larger than L2: n_res distinct resident batches are
         # cycled, > 160 MB): what a training loop sees -- the kernels of consecutive steps chain through programmatic dependent
@@ -714,11 +755,13 @@ def main():
         barrier()
         e0.record()
         for k in range(args.steps):
-            ag.update_successor_all(resident[(n_warm + k) % n_res], use_gpi=True)
+            losses = ag.update_successor_all(resident[(n_warm + k) % n_res], use_gpi=True)
         e1.record()
         barrier()
         launches = _lib.launch_count - l0
         stream_ms = e0.elapsed_time(e1)
+        if args.dump_outputs:                                       # before the bracketed steps below move the weights on
+            outputs = step_outputs(losses, lib, n_local)
     # per-step brackets: an event pair around every step and probes around the dominant kernel (the one-launch fused forward:
     # online psi(s) + GPI(s') + target psi(s')), recorded by the command list itself inside the step.  'flush' mode: these ARE
     # the timed steps (256 MiB write between them, outside the brackets).
@@ -732,10 +775,12 @@ def main():
             flush.fill_(k & 0xFF)
         lib.set_probe(plan_key, *kev[k])
         ev[k][0].record()
-        ag.update_successor_all(resident[(n_warm + k) % n_res], use_gpi=True)
+        losses = ag.update_successor_all(resident[(n_warm + k) % n_res], use_gpi=True)
         ev[k][1].record()
     barrier()
     lib.set_probe(plan_key, None, None)
+    if args.dump_outputs and outputs is None:                       # --l2 flush: these were the timed steps
+        outputs = step_outputs(losses, lib, n_local)
     if launches is None:
         launches = _lib.launch_count - l0
     step_ms = [a.elapsed_time(b) for a, b in ev]
@@ -938,6 +983,8 @@ def main():
             except Exception as e:
                 out['secondary_error'] = f'{type(e).__name__}: {e}'
     if rank == 0:
+        if args.dump_outputs:
+            write_outputs(outputs, args.dump_outputs)
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()

@@ -5,6 +5,7 @@ and cannot be built, or a call returns non-zero, a RuntimeError is raised.
 """
 import ctypes as C
 import os
+import shutil
 import subprocess
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -17,6 +18,17 @@ ACT = {'none': 0, 'relu': 1, 'tanh': 2}
 PREC = {'fp32': 0, 'bf16': 1, 'tf32': 2, 'tf32x3': 3}
 
 
+def nvcc_path():
+    """nvcc on PATH, else the one of the CUDA toolkit torch locates (CUDA_HOME / CUDA_PATH, /usr/local/cuda)."""
+    found = shutil.which('nvcc')
+    if found:
+        return found
+    from torch.utils.cpp_extension import CUDA_HOME
+    if CUDA_HOME and os.path.isfile(os.path.join(CUDA_HOME, 'bin', 'nvcc')):
+        return os.path.join(CUDA_HOME, 'bin', 'nvcc')
+    raise RuntimeError('nvcc not found: put the CUDA toolkit\'s bin directory on PATH or set CUDA_HOME')
+
+
 def build(force=False, verbose=False):
     """nvcc -> libsfgpi.so, sm_100a only (cross-compiles without a GPU)."""
     srcs = [os.path.join(CSRC, s) for s in SOURCES if os.path.exists(os.path.join(CSRC, s))]
@@ -24,7 +36,7 @@ def build(force=False, verbose=False):
     deps += [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith('.cuh')]
     if not force and os.path.exists(LIB_PATH) and all(os.path.getmtime(LIB_PATH) >= os.path.getmtime(d) for d in deps):
         return LIB_PATH
-    cmd = ['nvcc', '-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17', '-Xcompiler', '-fPIC',
+    cmd = [nvcc_path(), '-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17', '-Xcompiler', '-fPIC',
            '-shared', '-o', LIB_PATH] + srcs
     if verbose:
         cmd.insert(1, '-Xptxas=-v')
