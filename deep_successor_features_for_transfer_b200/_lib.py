@@ -60,7 +60,7 @@ class ForwardArgs(C.Structure):
                 ('sel_actions', C.c_void_p), ('sel_keys', C.c_void_p), ('sel_key_stride', C.c_int32),
                 ('sel_out', C.c_void_p), ('w', C.c_void_p), ('n_w', C.c_int32), ('w_diag', C.c_int32),
                 ('key_action', C.c_void_p), ('key_task', C.c_void_p), ('task_base', C.c_int32), ('q_out', C.c_void_p),
-                ('mode', C.c_int32), ('acts_bf16_out', C.c_void_p), ('relu_mask_out', C.c_void_p), ('key_stage', C.c_void_p)]
+                ('mode', C.c_int32), ('acts_bf16_out', C.c_void_p), ('relu_mask_out', C.c_void_p)]
 
 
 class TdArgs(C.Structure):
@@ -120,9 +120,9 @@ class Cmd(C.Structure):
 
 
 OP = dict(H2D=1, D2H=2, D2D=3, KEYS_FILL=4, PACK_BF16=5, FOLD_GPI=6, FORWARD=7, FORWARD_TC_JOBS=8, TD=9, BACKWARD=10,
-          BACKWARD_TC=11, ADAM=12, EVENT=13, PEER_KEYS=14, SHARD_PACK=15, PEER_UNPACK=16, STEP_PREP=17, KEYS_REDUCE=18,
-          PACK_F32=19, FOLD_GPI_F32=20, FORWARD_STREAM=21, BACKWARD_STREAM=22, KEYS_DECODE=23)
-OP_LAUNCHES = {13: 0, 0: 0, 1: 0, 2: 0, 3: 0, 4: 1, 5: 1, 6: 1, 7: 1, 8: 1, 9: 1, 10: 2, 11: 3, 12: 2, 14: 1, 15: 1, 16: 1, 17: 1, 18: 1,
+          BACKWARD_TC=11, ADAM=12, EVENT=13, PEER_KEYS=14, SHARD_PACK=15, PEER_UNPACK=16, STEP_PREP=17, PACK_F32=19,
+          FOLD_GPI_F32=20, FORWARD_STREAM=21, BACKWARD_STREAM=22, KEYS_DECODE=23)
+OP_LAUNCHES = {13: 0, 0: 0, 1: 0, 2: 0, 3: 0, 4: 1, 5: 1, 6: 1, 7: 1, 8: 1, 9: 1, 10: 2, 11: 3, 12: 2, 14: 1, 15: 1, 16: 1, 17: 1,
                19: 1, 20: 1, 21: 1, 22: 3, 23: 1}
 MAX_PEERS = 16
 PEER_CHANNELS = 4
@@ -177,7 +177,6 @@ class G4Args(C.Structure):
 SYMBOLS = {
     'sfgpi_mlp_forward': (C.c_int, [C.POINTER(ForwardArgs), C.c_void_p]),
     'sfgpi_keys_fill': (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p]),
-    'sfgpi_keys_reduce': (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p]),
     'sfgpi_keys_decode': (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     'sfgpi_gpi_from_psi': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -4,7 +4,6 @@
 // Gradients arrive as split partials (wgrad split-K, TD per-CTA partials) and are summed here in a fixed order, so the
 // whole step is deterministic.  HBM-bound: 16 B read + 12 B written per parameter (+ 4 B * n_part of partials).
 #include "common.cuh"
-#include <stdlib.h>
 
 namespace sfgpi {
 
@@ -363,8 +362,7 @@ extern "C" int sfgpi_adam_step(const sfgpi_adam_args *args, void *stream) {
     }
     cudaStream_t st = (cudaStream_t)stream;
     // flattened fast path (see adam_flat_kernel): the train steps' shape -- double-buffered corrections, 128-bit aligned segments
-    static const bool flat_off = getenv("SFGPI_ADAM_FLAT") != nullptr && atoi(getenv("SFGPI_ADAM_FLAT")) == 0;
-    if (!flat_off && !a.fresh && a.consts != nullptr && a.consts_next != nullptr) {
+    if (!a.fresh && a.consts != nullptr && a.consts_next != nullptr) {
         AdamFlat f;
         bool ok = true;
         int nb = 0, shared_len = 0;
@@ -394,8 +392,7 @@ extern "C" int sfgpi_adam_step(const sfgpi_adam_args *args, void *stream) {
     }
     int blocks = (max_len + kAdamThreads - 1) / kAdamThreads;
     if (blocks < 1) blocks = 1;
-    static const int ctas_per_sm = getenv("SFGPI_ADAM_CTAS") ? atoi(getenv("SFGPI_ADAM_CTAS")) : 8;       // (experiment knob)
-    const int cap = (148 * ctas_per_sm + a.n_pol - 1) / a.n_pol;       // ~8 CTAs per SM over the whole launch
+    const int cap = (148 * 8 + a.n_pol - 1) / a.n_pol;                 // ~8 CTAs per SM over the whole launch
     if (blocks > cap) blocks = cap < 1 ? 1 : cap;
     dim3 grid(blocks, a.n_pol);
     launch_pdl(adam_kernel, grid, dim3(kAdamThreads), 0, st, a, blocks);

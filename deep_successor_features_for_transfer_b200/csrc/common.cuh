@@ -58,22 +58,14 @@ __device__ __forceinline__ void trace_exit(int trace_slot) { trace_mark(trace_sl
 bool pdl_enabled();
 
 template <typename... KArgs, typename... Args>
-inline void launch_pdl_cluster(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, int cluster_x,
-                               Args &&...args) {
+inline void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args &&...args) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
     cfg.blockDim = block;
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
-    cudaLaunchAttribute attr[2];
+    cudaLaunchAttribute attr[1];
     int n = 0;
-    if (cluster_x > 1) {
-        attr[n].id = cudaLaunchAttributeClusterDimension;
-        attr[n].val.clusterDim.x = cluster_x;
-        attr[n].val.clusterDim.y = 1;
-        attr[n].val.clusterDim.z = 1;
-        ++n;
-    }
     if (pdl_enabled()) {
         attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         attr[n].val.programmaticStreamSerializationAllowed = 1;
@@ -82,10 +74,6 @@ inline void launch_pdl_cluster(void (*kernel)(KArgs...), dim3 grid, dim3 block, 
     cfg.attrs = attr;
     cfg.numAttrs = n;
     cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-template <typename... KArgs, typename... Args>
-inline void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args &&...args) {
-    launch_pdl_cluster(kernel, grid, block, smem, st, 1, static_cast<Args &&>(args)...);
 }
 
 __device__ __forceinline__ void cp_async16(void *smem, const void *gmem) {

@@ -1,4 +1,4 @@
-// Definitions shared by the tensor-core forward kernels (mlp_forward_tc.cu: ping-pong pairs / 2-CTA pairs;
+// Definitions shared by the tensor-core forward kernels (mlp_forward_tc.cu: ping-pong pairs;
 // mlp_chain_tc.cu: the single-tile layer-pipelined chain): job / launch parameter blocks, the item (layer) table, the hidden-layer epilogue.
 #pragma once
 #include "tc_common.cuh"
@@ -341,7 +341,7 @@ struct TmapSet { CUtensorMap w[kMaxJobs]; CUtensorMap q[kMaxJobs]; CUtensorMap a
 // entry = job << 30 | has_y << 29 | policy << 16 | first tile.
 constexpr int kMaxUnits = 1024;
 struct UnitTable { uint32_t u[kMaxUnits]; };
-struct Unit { int jb, pl, pip, tile0, tstep; bool has_y; };
+struct Unit { int jb, pl, tile0; bool has_y; };
 
 
 // role 0 = epilogue X (thread 0), 1 = MMA issuer, 2 = producer warp 0, 3 = epilogue Y (thread 0); 64 slots each

@@ -156,7 +156,7 @@ __global__ void __launch_bounds__(256) gpi_from_psi_kernel(const float *__restri
 using namespace sfgpi;
 
 extern "C" const char *sfgpi_last_error(void) { return g_err; }
-extern "C" int sfgpi_version(void) { return 100; }
+extern "C" int sfgpi_version(void) { return 101; }
 
 extern "C" int sfgpi_keys_fill(int64_t *keys, int64_t n, void *stream) {
     if (n <= 0) return SFGPI_OK;
@@ -164,48 +164,6 @@ extern "C" int sfgpi_keys_fill(int64_t *keys, int64_t n, void *stream) {
     if (blocks > 148 * 8) blocks = 148 * 8;
     launch_pdl(keys_fill_kernel, dim3(blocks), dim3(256), 0, (cudaStream_t)stream, reinterpret_cast<long long *>(keys), (long long)n);
     return check_launch("sfgpi_keys_fill");
-}
-
-namespace sfgpi {
-// keys_out[i] = max_p stage[p][i]: two keys (16 B) per thread, 4 policies' loads in flight per trip; HBM-bound streaming pass
-__global__ void __launch_bounds__(256) keys_reduce_kernel(const long long *__restrict__ stage, int n_pol, long long n,
-                                                          long long *__restrict__ keys_out) {
-    pdl_launch_dependents();
-    pdl_wait();
-    const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 2;
-    if (i >= n) return;
-    if (i + 1 < n && (n & 1) == 0 && ((reinterpret_cast<uintptr_t>(stage) | reinterpret_cast<uintptr_t>(keys_out)) & 15) == 0) {
-        longlong2 m = make_longlong2(LLONG_MIN, LLONG_MIN);
-        int p = 0;
-        for (; p + 4 <= n_pol; p += 4) {
-            longlong2 v[4];
-#pragma unroll
-            for (int q = 0; q < 4; ++q) v[q] = *reinterpret_cast<const longlong2 *>(stage + (size_t)(p + q) * n + i);
-#pragma unroll
-            for (int q = 0; q < 4; ++q) { m.x = max(m.x, v[q].x); m.y = max(m.y, v[q].y); }
-        }
-        for (; p < n_pol; ++p) {
-            const longlong2 v = *reinterpret_cast<const longlong2 *>(stage + (size_t)p * n + i);
-            m.x = max(m.x, v.x); m.y = max(m.y, v.y);
-        }
-        *reinterpret_cast<longlong2 *>(keys_out + i) = m;
-    } else {
-        for (long long k = i; k < min(i + 2, n); ++k) {
-            long long m = LLONG_MIN;
-            for (int p = 0; p < n_pol; ++p) m = max(m, stage[(size_t)p * n + k]);
-            keys_out[k] = m;
-        }
-    }
-}
-}  // namespace sfgpi
-
-extern "C" int sfgpi_keys_reduce(const int64_t *stage, int32_t n_pol, int64_t n, int64_t *keys_out, void *stream) {
-    if (n_pol < 1 || n < 0 || !stage || !keys_out) { set_error("sfgpi_keys_reduce: invalid arguments"); return SFGPI_E_INVALID; }
-    if (n == 0) return SFGPI_OK;
-    const long long blocks = ((n + 1) / 2 + 255) / 256;
-    launch_pdl(keys_reduce_kernel, dim3((unsigned)blocks), dim3(256), 0, (cudaStream_t)stream, reinterpret_cast<const long long *>(stage),
-               (int)n_pol, (long long)n, reinterpret_cast<long long *>(keys_out));
-    return check_launch("sfgpi_keys_reduce");
 }
 
 extern "C" int sfgpi_keys_decode(const int64_t *keys, int64_t n, int64_t *index_out, float *value_out, void *stream) {

@@ -1,5 +1,5 @@
-// Folded-GPI column order and the blocked running (max, argmax) scan, shared by the tensor-core forward kernels
-// (mlp_forward_tc.cu: bf16; mlp_stream_tc.cu: tf32 / tf32x3).
+// Folded-GPI column order, shared by the tensor-core forward kernels (mlp_forward_tc.cu: bf16; mlp_stream_tc.cu: tf32 / tf32x3),
+// and the blocked running (max, argmax) scan of the tf32 kernel.
 #pragma once
 #include "tc_common.cuh"
 
@@ -25,7 +25,7 @@ __device__ __forceinline__ void gpi_row_to_wa(int row, int nw, int A, int &wi, i
 template <int WB, int OFF>
 __device__ __forceinline__ void gpi_scan_blocked(const uint32_t (&v)[32], const float (&bv)[8], int col, int ncol, int A_, int nw, float (&bb)[8],
                                                  int (&ba)[8], int &act_i, int &g, long long *&kp, long long *&tp, uint32_t kstep,
-                                                 bool k_staged, bool k_has, bool t_has, bool row_ok, uint32_t task_id, float *q_row) {
+                                                 bool k_has, bool t_has, bool row_ok, uint32_t task_id, float *q_row) {
 #pragma unroll
     for (int j = 0; j < 8 / WB; ++j) {
         if (col + j * WB < ncol) {                           // (ncol is a multiple of WB)
@@ -39,9 +39,7 @@ __device__ __forceinline__ void gpi_scan_blocked(const uint32_t (&v)[32], const 
 #pragma unroll
                 for (int ws = 0; ws < WB; ++ws) {
                     if (row_ok && g * WB + ws < nw) {
-                        const long long key = pack_key(bb[ws], (uint32_t)ba[ws]);
-                        if (k_staged) kp[(size_t)ws * kstep] = key;
-                        else if (k_has) atomicMax(kp + (size_t)ws * kstep, key);
+                        if (k_has) atomicMax(kp + (size_t)ws * kstep, pack_key(bb[ws], (uint32_t)ba[ws]));
                         if (t_has) atomicMax(tp + (size_t)ws * kstep, pack_key(bb[ws], task_id));
                     }
                     bb[ws] = -INFINITY;

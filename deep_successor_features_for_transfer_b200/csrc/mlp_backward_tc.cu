@@ -677,8 +677,7 @@ extern "C" int sfgpi_mlp_backward_tc(const sfgpi_backward_tc_args *args, void *s
     dp.n_items = dp.n_chunks + (L - 2);
     dp.tiles_per_policy = (a.B + kTM - 1) / kTM;
     const int total_tiles = dp.tiles_per_policy * a.n_pol;
-    static const int pair_min = getenv("SFGPI_PAIR_MIN") ? atoi(getenv("SFGPI_PAIR_MIN")) : 148;
-    dp.paired = total_tiles > pair_min ? 1 : 0;
+    dp.paired = total_tiles > 148 ? 1 : 0;
     dp.pairs_per_policy = dp.paired ? (dp.tiles_per_policy + 1) / 2 : dp.tiles_per_policy;
     dp.total_pairs = dp.pairs_per_policy * a.n_pol;
     CUtensorMap tmap_w;

@@ -467,7 +467,6 @@ mlp_chain_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__ T
 bool forward_chain_supported(const TcMulti &m) {
     for (int j = 0; j < m.n_jobs; ++j) {
         const sfgpi_forward_args &a = m.job[j].a;
-        if (a.key_stage != nullptr) return false;
         for (int l = 0; l < SFGPI_MAX_LAYERS; ++l)
             if (a.acts_out[l] != nullptr) return false;
     }

@@ -218,7 +218,6 @@ extern "C" int sfgpi_mlp_forward(const sfgpi_forward_args *args, void *stream) {
         return SFGPI_E_INVALID;
     }
     if (a.mode != 0) { set_error("sfgpi_mlp_forward: mode %d not built into this entry point", a.mode); return SFGPI_E_INVALID; }
-    if (a.key_stage != nullptr) { set_error("sfgpi_mlp_forward: key_stage is an output of the tensor-core path only"); return SFGPI_E_INVALID; }
     if (a.B == 0 || a.n_pol == 0) return SFGPI_OK;
     const bool gpi = a.w != nullptr;
     if (gpi && (net.n_features > kNC || a.n_w < 1)) {

@@ -32,33 +32,26 @@ __device__ __forceinline__ int job_of_pair(const TcMulti &m, int pair) {
     return j;
 }
 
-// TWO = true: 2-CTA pairs (cluster of 2, tcgen05 cta_group::2).  The pair runs ONE MMA stream with M = 256 (128 rows from each
-// CTA) and each CTA stores only its half of every weight block, so per SM the weight traffic (TMA in, MMA read) halves and a
-// 16 KB ring stage feeds a whole 256-column k-block.  Work unit = 4 row tiles of one policy: CTA r handles tile 4q + r in slot
-// X and tile 4q + 2 + r in slot Y.  Rank 0 issues all MMAs; producers and epilogues run in both CTAs.
-template <bool TWO>
 __global__ void __launch_bounds__(kThreadsTc, 1)
 mlp_forward_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__ TmapSet maps, const __grid_constant__ UnitTable ut) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t cta_rank = TWO ? cluster_ctarank() : 0u;
-    const int unit0 = TWO ? (int)(blockIdx.x >> 1) : (int)blockIdx.x, unit_stride = TWO ? (int)(gridDim.x >> 1) : (int)gridDim.x;
-    // work unit g -> job, policy slot, the tile this CTA handles in slot X (slot Y: tile0 + tstep), whether it has a Y slot
+    const int unit0 = (int)blockIdx.x, unit_stride = (int)gridDim.x;
+    // work unit g -> job, policy slot, the tile this CTA handles in slot X (slot Y: tile0 + 1), whether it has a Y slot
     auto unit_at = [&](int g) {
         Unit u;
-        if (!TWO && m.sched) {
+        if (m.sched) {
             const uint32_t e = ut.u[g];
             u.jb = (int)(e >> 30); u.has_y = (e >> 29) & 1u; u.pl = (int)((e >> 16) & 0x1FFFu); u.tile0 = (int)(e & 0xFFFFu);
-            u.pip = 0; u.tstep = 1;
             return u;
         }
         u.jb = job_of_pair(m, g);
         const TcParams &p = m.job[u.jb];
         const int pair = g - m.pair_start[u.jb];
         u.pl = pair / p.pairs_per_policy;
-        u.pip = pair - u.pl * p.pairs_per_policy;
-        if (TWO) { u.tile0 = 4 * u.pip + (int)cta_rank; u.tstep = 2; u.has_y = 4 * u.pip + 2 < p.tiles_per_policy; }
-        else { u.tile0 = p.paired ? 2 * u.pip : u.pip; u.tstep = 1; u.has_y = p.paired && (2 * u.pip + 1 < p.tiles_per_policy); }
+        const int pip = pair - u.pl * p.pairs_per_policy;
+        u.tile0 = p.paired ? 2 * pip : pip;
+        u.has_y = p.paired && (2 * pip + 1 < p.tiles_per_policy);
         return u;
     };
     pdl_launch_dependents(SFGPI_TR_FWD);
@@ -85,16 +78,16 @@ mlp_forward_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < 8; ++s) { mbar_init(W_FULL(s), 1); mbar_init(W_EMPTY(s), 1); }
-        for (int s = 0; s < 2; ++s) { mbar_init(SLOT_READY(s), TWO ? 2 : 256); mbar_init(ACC_FULL(s), 1); }
+        for (int s = 0; s < 2; ++s) { mbar_init(SLOT_READY(s), 256); mbar_init(ACC_FULL(s), 1); }
         fence_mbar_init();
         for (int j = 0; j < m.n_jobs; ++j) {
             tma_prefetch_desc(&maps.w[j]);
             if (m.job[j].gpi) tma_prefetch_desc(&maps.q[j]);
         }
     }
-    if (warp == kMmaWarp) { if (TWO) tmem_alloc2(holder_addr, 512); else tmem_alloc(holder_addr, 512); }
+    if (warp == kMmaWarp) tmem_alloc(holder_addr, 512);
     tc_fence_before();
-    if (TWO) cluster_sync_all(); else __syncthreads();       // (pair: the peer's barriers must exist before anything arrives on them)
+    __syncthreads();
     tc_fence_after();
     uint32_t tmem_base;
     asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(holder_addr));
@@ -119,11 +112,10 @@ mlp_forward_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__
                 const bool has_y = un.has_y;
                 for (int it = 0; it < p.n_items; ++it) {
                     const ItemInfo ii = item_info(p, it);
-                    const int nblocks = TWO ? 1 : (ii.n_cols + kNB - 1) / kNB;
+                    const int nblocks = (ii.n_cols + kNB - 1) / kNB;
                     const bool folded = ii.kind == 2 && p.gpi;
                     const void *tm = folded ? (const void *)&maps.q[jb] : (const void *)&maps.w[jb];
-                    // pair: this CTA stores weight rows [rank * n_cols / 2, ...) of the block (its half of the B operand)
-                    const int rbase = (folded ? pl * p.n_final + ii.row_base : row0 + ii.row_base) + (TWO ? (int)cta_rank * (ii.n_cols >> 1) : 0);
+                    const int rbase = folded ? pl * p.n_final + ii.row_base : row0 + ii.row_base;
                     for (int slot = 0; slot < (has_y ? 2 : 1); ++slot)
                         for (int kb = 0; kb < ii.n_kb; ++kb)
                             for (int nb = 0; nb < nblocks; ++nb, ++n) {
@@ -131,13 +123,8 @@ mlp_forward_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__
                                 if ((s & 3) != warp) continue;
                                 mbar_wait_warp(W_EMPTY(s), ((n >> ns_log) & 1) ^ 1);
                                 if (warp == 0 && leader) TL_STAMP(2, tlc);
-                                if (TWO) {                       // both halves are counted on the pair leader's barrier
-                                    if (cta_rank == 0) mbar_arrive_expect_tx_e(W_FULL(s), 2 * kStageBytes, leader);
-                                    tma_load_2d_2cta_e(W_addr + stage_off(s), tm, W_FULL(s), kb * kKB, rbase, leader);
-                                } else {
-                                    mbar_arrive_expect_tx_e(W_FULL(s), kStageBytes, leader);
-                                    tma_load_2d_e(W_addr + stage_off(s), tm, W_FULL(s), kb * kKB, rbase + nb * kNB, leader);
-                                }
+                                mbar_arrive_expect_tx_e(W_FULL(s), kStageBytes, leader);
+                                tma_load_2d_e(W_addr + stage_off(s), tm, W_FULL(s), kb * kKB, rbase + nb * kNB, leader);
                             }
                 }
             }
@@ -145,98 +132,77 @@ mlp_forward_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__
     } else if (warp == kMmaWarp) {
         // =========================== MMA issuer ===========================
         // Whole warp runs the loop (operands stay in uniform registers), the elected lane issues: see tc_common.cuh.
-        if (!TWO || cta_rank == 0) {
-            const uint32_t leader = elect_one();
-            uint32_t n = 0, ready_cnt[2] = {0, 0};
-            int tlc = 0;
-            const uint64_t adesc_x = umma_desc_k_sw128(sbase), adesc_y = umma_desc_k_sw128(sbase + kABytes);
-            const uint64_t bdesc0 = umma_desc_k_sw128(W_addr);
-            for (int gpair = unit0; gpair < m.total_pairs; gpair += unit_stride) {
-                const Unit un = unit_at(gpair);
-                const int jb = un.jb;
-                const TcParams &p = m.job[jb];
-                const bool has_y = un.has_y;
-                for (int it = 0; it < p.n_items; ++it) {
-                    const ItemInfo ii = item_info(p, it);
-                    const int nblocks = (ii.n_cols + kNB - 1) / kNB;
-                    const uint32_t idesc_full = umma_idesc_bf16(kTM, kNB);
-                    const uint32_t idesc_last = umma_idesc_bf16(kTM, (uint32_t)(ii.n_cols - (nblocks - 1) * kNB));
-                    for (int slot = 0; slot < (has_y ? 2 : 1); ++slot) {
-                        if (TWO) mbar_wait_warp_cluster(SLOT_READY(slot), ready_cnt[slot] & 1);
-                        else mbar_wait_warp(SLOT_READY(slot), ready_cnt[slot] & 1);
-                        ++ready_cnt[slot];
-                        tc_fence_after();
-                        if (leader) TL_STAMP(1, tlc);                         // slot ready
-                        const uint32_t d_base = tmem_base + (uint32_t)slot * 256u;
-                        if (TWO) {
-                            // pair: one ring stage (this CTA's half of the weight block) per k-block, M = 256, N = n_cols
-                            const uint32_t idesc2 = umma_idesc_bf16(256, (uint32_t)ii.n_cols);
-                            for (int kb = 0; kb < ii.n_kb; ++kb, ++n) {
-                                const uint64_t ad = (slot ? adesc_y : adesc_x) + (uint64_t)(kb * ((kTM * 128) >> 4));
-                                const int s = n & ns_mask;
-                                mbar_wait_warp(W_FULL(s), (n >> ns_log) & 1);
-                                tc_fence_after();
-                                if (leader && kb == 0) TL_STAMP(1, tlc);
-                                const uint64_t bd = bdesc0 + (uint64_t)(int64_t)(stage_off(s) >> 4);
+        const uint32_t leader = elect_one();
+        uint32_t n = 0, ready_cnt[2] = {0, 0};
+        int tlc = 0;
+        const uint64_t adesc_x = umma_desc_k_sw128(sbase), adesc_y = umma_desc_k_sw128(sbase + kABytes);
+        const uint64_t bdesc0 = umma_desc_k_sw128(W_addr);
+        for (int gpair = unit0; gpair < m.total_pairs; gpair += unit_stride) {
+            const Unit un = unit_at(gpair);
+            const int jb = un.jb;
+            const TcParams &p = m.job[jb];
+            const bool has_y = un.has_y;
+            for (int it = 0; it < p.n_items; ++it) {
+                const ItemInfo ii = item_info(p, it);
+                const int nblocks = (ii.n_cols + kNB - 1) / kNB;
+                const uint32_t idesc_full = umma_idesc_bf16(kTM, kNB);
+                const uint32_t idesc_last = umma_idesc_bf16(kTM, (uint32_t)(ii.n_cols - (nblocks - 1) * kNB));
+                for (int slot = 0; slot < (has_y ? 2 : 1); ++slot) {
+                    mbar_wait_warp(SLOT_READY(slot), ready_cnt[slot] & 1);
+                    ++ready_cnt[slot];
+                    tc_fence_after();
+                    if (leader) TL_STAMP(1, tlc);                         // slot ready
+                    const uint32_t d_base = tmem_base + (uint32_t)slot * 256u;
+                    // A full 256-column layer is issued as N=256 MMAs over a PAIR of adjacent ring stages (rows 0-127 | 128-255
+                    // of the weight block are contiguous in shared memory): half as many instructions for the same math --
+                    // the single issuing thread needs ~107 cycles per tcgen05.mma, more than the 64 an N=128 MMA executes.
+                    const bool wide = nblocks == 2 && ii.n_cols == 256 && !(n & 1);
+                    const uint32_t idesc_wide = umma_idesc_bf16(kTM, 256);
+                    for (int kb = 0; kb < ii.n_kb; ++kb) {
+                        const uint64_t ad = (slot ? adesc_y : adesc_x) + (uint64_t)(kb * ((kTM * 128) >> 4));
+                        if (wide) {
+                            const int s = n & ns_mask;
+                            mbar_wait_warp(W_FULL(s), (n >> ns_log) & 1);
+                            mbar_wait_warp(W_FULL(s + 1), (n >> ns_log) & 1);
+                            tc_fence_after();
+                            if (leader && kb == 0) TL_STAMP(1, tlc);              // first weight stages landed
+                            const uint64_t bd = bdesc0 + (uint64_t)(int64_t)(stage_off(s) >> 4);
+                            if (ii.n_k16 == 4) {
+                                umma_bf16_e(d_base, ad, bd, idesc_wide, kb ? 1u : 0u, leader);
+                                umma_bf16_e(d_base, ad + 2, bd + 2, idesc_wide, 1u, leader);
+                                umma_bf16_e(d_base, ad + 4, bd + 4, idesc_wide, 1u, leader);
+                                umma_bf16_e(d_base, ad + 6, bd + 6, idesc_wide, 1u, leader);
+                            } else {
                                 for (int k16 = 0; k16 < ii.n_k16; ++k16)
-                                    umma_bf16_2cta_e(d_base, ad + 2 * k16, bd + 2 * k16, idesc2, (kb | k16) ? 1u : 0u, leader);
-                                umma_commit_2cta_e(W_EMPTY(s), leader);
+                                    umma_bf16_e(d_base, ad + 2 * k16, bd + 2 * k16, idesc_wide, (kb | k16) ? 1u : 0u, leader);
                             }
-                            umma_commit_2cta_e(ACC_FULL(slot), leader);
-                            if (leader) TL_STAMP(1, tlc);
+                            umma_commit_e(W_EMPTY(s), leader);
+                            umma_commit_e(W_EMPTY(s + 1), leader);
+                            n += 2;
                             continue;
                         }
-                        // A full 256-column layer is issued as N=256 MMAs over a PAIR of adjacent ring stages (rows 0-127 | 128-255
-                        // of the weight block are contiguous in shared memory): half as many instructions for the same math --
-                        // the single issuing thread needs ~107 cycles per tcgen05.mma, more than the 64 an N=128 MMA executes.
-                        const bool wide = nblocks == 2 && ii.n_cols == 256 && !(n & 1);
-                        const uint32_t idesc_wide = umma_idesc_bf16(kTM, 256);
-                        for (int kb = 0; kb < ii.n_kb; ++kb) {
-                            const uint64_t ad = (slot ? adesc_y : adesc_x) + (uint64_t)(kb * ((kTM * 128) >> 4));
-                            if (wide) {
-                                const int s = n & ns_mask;
-                                mbar_wait_warp(W_FULL(s), (n >> ns_log) & 1);
-                                mbar_wait_warp(W_FULL(s + 1), (n >> ns_log) & 1);
-                                tc_fence_after();
-                                if (leader && kb == 0) TL_STAMP(1, tlc);              // first weight stages landed
-                                const uint64_t bd = bdesc0 + (uint64_t)(int64_t)(stage_off(s) >> 4);
-                                if (ii.n_k16 == 4) {
-                                    umma_bf16_e(d_base, ad, bd, idesc_wide, kb ? 1u : 0u, leader);
-                                    umma_bf16_e(d_base, ad + 2, bd + 2, idesc_wide, 1u, leader);
-                                    umma_bf16_e(d_base, ad + 4, bd + 4, idesc_wide, 1u, leader);
-                                    umma_bf16_e(d_base, ad + 6, bd + 6, idesc_wide, 1u, leader);
-                                } else {
-                                    for (int k16 = 0; k16 < ii.n_k16; ++k16)
-                                        umma_bf16_e(d_base, ad + 2 * k16, bd + 2 * k16, idesc_wide, (kb | k16) ? 1u : 0u, leader);
-                                }
-                                umma_commit_e(W_EMPTY(s), leader);
-                                umma_commit_e(W_EMPTY(s + 1), leader);
-                                n += 2;
-                                continue;
+                        for (int nb = 0; nb < nblocks; ++nb, ++n) {
+                            const int s = n & ns_mask;
+                            mbar_wait_warp(W_FULL(s), (n >> ns_log) & 1);
+                            tc_fence_after();
+                            if (leader && kb == 0 && nb == 0) TL_STAMP(1, tlc);   // first weight stage landed
+                            const uint32_t idesc = (nb == nblocks - 1) ? idesc_last : idesc_full;
+                            const uint64_t bd = bdesc0 + (uint64_t)(int64_t)(stage_off(s) >> 4);
+                            const uint32_t d = d_base + nb * kNB;
+                            if (ii.n_k16 == 4) {
+                                umma_bf16_e(d, ad, bd, idesc, kb ? 1u : 0u, leader);
+                                umma_bf16_e(d, ad + 2, bd + 2, idesc, 1u, leader);
+                                umma_bf16_e(d, ad + 4, bd + 4, idesc, 1u, leader);
+                                umma_bf16_e(d, ad + 6, bd + 6, idesc, 1u, leader);
+                            } else {
+                                for (int k16 = 0; k16 < ii.n_k16; ++k16)
+                                    umma_bf16_e(d, ad + 2 * k16, bd + 2 * k16, idesc, (kb | k16) ? 1u : 0u, leader);
                             }
-                            for (int nb = 0; nb < nblocks; ++nb, ++n) {
-                                const int s = n & ns_mask;
-                                mbar_wait_warp(W_FULL(s), (n >> ns_log) & 1);
-                                tc_fence_after();
-                                if (leader && kb == 0 && nb == 0) TL_STAMP(1, tlc);   // first weight stage landed
-                                const uint32_t idesc = (nb == nblocks - 1) ? idesc_last : idesc_full;
-                                const uint64_t bd = bdesc0 + (uint64_t)(int64_t)(stage_off(s) >> 4);
-                                const uint32_t d = d_base + nb * kNB;
-                                if (ii.n_k16 == 4) {
-                                    umma_bf16_e(d, ad, bd, idesc, kb ? 1u : 0u, leader);
-                                    umma_bf16_e(d, ad + 2, bd + 2, idesc, 1u, leader);
-                                    umma_bf16_e(d, ad + 4, bd + 4, idesc, 1u, leader);
-                                    umma_bf16_e(d, ad + 6, bd + 6, idesc, 1u, leader);
-                                } else {
-                                    for (int k16 = 0; k16 < ii.n_k16; ++k16)
-                                        umma_bf16_e(d, ad + 2 * k16, bd + 2 * k16, idesc, (kb | k16) ? 1u : 0u, leader);
-                                }
-                                umma_commit_e(W_EMPTY(s), leader);           // stage free once these MMAs have read it
-                            }
+                            umma_commit_e(W_EMPTY(s), leader);           // stage free once these MMAs have read it
                         }
-                        umma_commit_e(ACC_FULL(slot), leader);                // accumulator of this item complete
-                        if (leader) TL_STAMP(1, tlc);                         // all MMAs of the item issued
                     }
+                    umma_commit_e(ACC_FULL(slot), leader);                // accumulator of this item complete
+                    if (leader) TL_STAMP(1, tlc);                         // all MMAs of the item issued
                 }
             }
         }
@@ -259,16 +225,6 @@ mlp_forward_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__
 #define TL_EPI() do { if (tl_role >= 0) TL_STAMP(tl_role, tlc); } while (0)
         TL_EPI();                                            // set-up done
 
-        // pair: SLOT_READY lives in the leader CTA and takes ONE cluster-scope release arrive per CTA -- 256 per-thread
-        // release.cluster arrives cost ~1000 cycles per epilogue (measured); a CTA barrier orders the others' writes before it.
-        auto slot_ready = [&](int slot) {
-            if (TWO) {
-                asm volatile("bar.sync 1, 256;" ::: "memory");
-                if (et == 0) mbar_arrive_leader(SLOT_READY(slot));
-            } else {
-                mbar_arrive(SLOT_READY(slot));
-            }
-        };
         for (int gpair = unit0; gpair < m.total_pairs; gpair += unit_stride) {
             const Unit un = unit_at(gpair);
             const int jb = un.jb;
@@ -324,7 +280,7 @@ mlp_forward_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__
 #pragma unroll
             for (int slot = 0; slot < 2; ++slot) {
                 if (slot >= n_slots) break;
-                const int b = (un.tile0 + slot * un.tstep) * kTM + r;                   // global state index of this thread's row
+                const int b = (un.tile0 + slot) * kTM + r;                             // global state index of this thread's row
                 bs[slot] = b;
                 if (a.sel_out != nullptr && b < B)
                     sidx_v[slot] = a.sel_actions ? (int)a.sel_actions[b] : (int)key_index(a.sel_keys[(size_t)pl * a.sel_key_stride + b]);
@@ -351,7 +307,7 @@ mlp_forward_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__
                     }
                     fence_proxy_async();                      // generic-proxy smem writes -> visible to the UMMA (async proxy)
                 }
-                slot_ready(slot);
+                mbar_arrive(SLOT_READY(slot));
                 sel_base[slot] = (a.sel_out != nullptr && row_ok) ? sidx_v[slot] * D : -(1 << 30);
             }
             TL_EPI();                                         // state tiles staged
@@ -377,13 +333,6 @@ mlp_forward_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__
                 cur_policy = jb * 65536 + pl;
             }
 
-            // GPI running state (folded form): columns are (reward vector wi, action act); group g scans slot g
-            float best = -INFINITY;
-            int best_a = 0, wi = 0, act_i = 0;               // (blocked order: wi counts blocks of WB reward vectors)
-            float bb[8];
-            int ba[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) { bb[i] = -INFINITY; ba[i] = 0; }
             // GPI output chunks: the generic item loop below spends as long on its per-(chunk, slot) set-up -- job fields re-read
             // through register-indexed constant loads, slot-indexed state in local memory, a page of straight-line code that runs
             // once per chunk and is therefore never in the 32 KB instruction cache -- as on the scan itself (ncu source page at 256
@@ -391,12 +340,11 @@ mlp_forward_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__
             // stamps at 4 vectors: 3.3 k cycles of set-up ahead of a 5-trip scan).  GPI jobs that write action / task keys only
             // take their output chunks through the lean loop further down: everything chunk-invariant in registers, slots unrolled.
             const int Lh_u = p.Lh, n_items_u = p.n_items;
-            const int ncol_u = p.gpi ? gpi_ncols(p.nw, A_) : 0;
-            const bool lean_gpi = p.gpi != 0 && !a.w_diag && a.key_stage == nullptr && a.q_out == nullptr;
+            const bool lean_gpi = p.gpi != 0 && !a.w_diag && a.q_out == nullptr;
             const bool lean_psi = p.gpi == 0;
             for (int it = 0; it < n_items_u; ++it) {
                 if (lean_gpi && it == 1 + Lh_u) {
-                    const int nw_u = p.nw, n_final_u = p.n_final, wblk_u = gpi_wblock(nw_u);
+                    const int nw_u = p.nw, n_final_u = p.n_final, wblk_u = gpi_wblock(nw_u), ncol_u = gpi_ncols(nw_u, A_);
                     const bool wide_u = wblk_u == 8 && ncol_u >= m.wide_min;
                     const uint32_t bias_u = bias_addr + 4u * ((1 + Lh_u) * kH);        // folded biases, indexed by absolute column
                     const uint32_t tid_u = (uint32_t)(a.task_base + pl), kstep_u = (uint32_t)B;
@@ -430,7 +378,7 @@ mlp_forward_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__
                                 else gpi_scan_rolled<1>(t_lane, bias_u, col0, cm, ce, A_, nw_u, ka_b, kt_b, kstep_u, b < B, tid_u, nullptr);
                             }
                             tc_fence_before();
-                            if (more) slot_ready(slot);                                     // next chunk may overwrite the accumulator
+                            if (more) mbar_arrive(SLOT_READY(slot));                                     // next chunk may overwrite the accumulator
                             TL_EPI();
                         }
                     }
@@ -460,7 +408,7 @@ mlp_forward_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__
                                            psi_u ? psi_u + ((size_t)b * n_pol_u + pl) * AD : nullptr, AD,
                                            sel_u ? sel_u + ((size_t)pl * B + b) * D : nullptr, slot ? sb1_u : sb0_u, D, b < B);
                             tc_fence_before();
-                            if (more) slot_ready(slot);                                     // next chunk may overwrite the accumulator
+                            if (more) mbar_arrive(SLOT_READY(slot));                                     // next chunk may overwrite the accumulator
                             TL_EPI();
                         }
                     }
@@ -486,18 +434,23 @@ mlp_forward_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__
                             ? reinterpret_cast<uint32_t *>(a.relu_mask_out) + (((size_t)it * a.n_pol + pl) * B + b) * 8
                             : nullptr;
                         if (store_pending[slot]) { a_slot_guard(!store_pending[slot ^ 1]); store_pending[slot] = false; }
+                        // An opaque copy of the row index: ptxas then derives the swizzled store addresses inside each epilogue
+                        // instead of keeping values of r live across the work-unit loop (measured on B200, 1000 W: 52 instead of
+                        // 80 B of spills, forward 37.6 instead of 38.6 us at the bench's headline size).
+                        int rr = r;
+                        asm volatile("" : "+r"(rr));
                         if (act == SFGPI_ACT_RELU) {
-                            if (a.relu_mask_out) hidden_epilogue<SFGPI_ACT_RELU, 4, true>(t_lane, bias, Arow, r, save, mask_out, group * 128);
-                            else hidden_epilogue<SFGPI_ACT_RELU, 4, false>(t_lane, bias, Arow, r, save, nullptr, group * 128);
-                        } else if (act == SFGPI_ACT_NONE) hidden_epilogue<SFGPI_ACT_NONE, 4, false>(t_lane, bias, Arow, r, save, nullptr, group * 128);
-                        else hidden_epilogue<SFGPI_ACT_TANH, 4, false>(t_lane, bias, Arow, r, save, nullptr, group * 128);
+                            if (a.relu_mask_out) hidden_epilogue<SFGPI_ACT_RELU, 4, true>(t_lane, bias, Arow, rr, save, mask_out, group * 128);
+                            else hidden_epilogue<SFGPI_ACT_RELU, 4, false>(t_lane, bias, Arow, rr, save, nullptr, group * 128);
+                        } else if (act == SFGPI_ACT_NONE) hidden_epilogue<SFGPI_ACT_NONE, 4, false>(t_lane, bias, Arow, rr, save, nullptr, group * 128);
+                        else hidden_epilogue<SFGPI_ACT_TANH, 4, false>(t_lane, bias, Arow, rr, save, nullptr, group * 128);
                         tc_fence_before();
                         fence_proxy_async();
-                        slot_ready(slot);
+                        mbar_arrive(SLOT_READY(slot));
                         if (saving) {                         // tile complete in shared memory -> one thread stores it
-                            if (!TWO) asm volatile("bar.sync 1, 256;" ::: "memory");      // (pair: slot_ready just did)
+                            asm volatile("bar.sync 1, 256;" ::: "memory");
                             if (et == 0) {
-                                const int row0 = (un.tile0 + slot * un.tstep) * kTM;
+                                const int row0 = (un.tile0 + slot) * kTM;
 #pragma unroll
                                 for (int kb = 0; kb < kH / kKB; ++kb)
                                     tma_store_3d(&maps.acts[jb], Arow + kb * (kTM * 128), kb * kKB, row0, it * a.n_pol + pl);
@@ -506,151 +459,28 @@ mlp_forward_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__
                             store_pending[slot] = true;
                         }
                     } else {
-                        // ------ output layer chunk ------
+                        // ------ output layer chunk, GPI form (psi-form chunks always take the lean loop above) ------
+                        // Rolled 8-column scan (gpi_scan_rolled, forward_tc.cuh): this code runs once per tile, so it is
+                        // instruction-FETCH bound -- unrolled 32-column windows cost 9-13 k cycles per tile for 36 columns
+                        // (profiles/r02_forward_chain.md), the rolled loop ~2.5 k.  Every emission is an atomicMax, so a chunk
+                        // needs no state from the previous one and each group takes one 128-column half.
                         const uint32_t bias = bias_addr + 4u * ((1 + p.Lh) * kH + ii.col0);
-                        // 8 columns per trip in a rolled loop: this code runs once per tile, so it is instruction-fetch bound
-                        // and compact beats wide.  psi form: column groups alternate between the two epilogue groups; GPI form:
-                        // a running (max, argmax) is carried along the columns, so ONE group scans a slot (group g: slot g).
-                        const int c_first = p.gpi ? (group == slot ? 0 : ii.n_cols) : group * 8;
-                        const int c_step = p.gpi ? 8 : 16;
-                        const int ncol = p.gpi ? gpi_ncols(p.nw, A_) : 0;
-                        const int wblk = p.gpi ? gpi_wblock(p.nw) : 1;
-                        const int sb = sel_base[slot];
-                        // Everything the column loop needs of the job's arguments, in REGISTERS: `p` / `a` are slices of the kernel
-                        // parameters selected by a runtime job index, so each field read is a register-indexed constant load
-                        // (LDC c[0][R+off], ~100 cycles) that the "memory"-clobbering tcgen05 waits force the compiler to repeat
-                        // per column -- ~1600 cycles per 8-column trip (measured: 8.3 ms forward at 256 reward vectors).
-                        const bool gpi_form = p.gpi != 0;
-                        const int n_cols_it = ii.n_cols, col0_it = ii.col0, n_pol_job = a.n_pol, task_base = a.task_base;
-                        float *const q_out = a.q_out, *const psi_out = a.psi_out, *const sel_out = a.sel_out;
-                        // where this row emits the key of reward vector wi: destination pointers that advance by a fixed step per
-                        // vector (no 64-bit index arithmetic in the column loop); rebuilt from wi at every chunk so that they are
-                        // not live across the hidden-layer epilogues.  kp: staged store / action-key atomic, tp: task-key atomic.
-                        uint32_t kstep = 0;
-                        bool k_staged = false, k_has = false, t_has = false;
-                        long long *kp = nullptr, *tp = nullptr;
-                        if (gpi_form) {
-                            kstep = a.w_diag ? 0u : (uint32_t)B;
-                            k_staged = a.key_stage != nullptr;
-                            k_has = k_staged || a.key_action != nullptr;
-                            t_has = a.key_task != nullptr;
-                            kp = k_staged ? reinterpret_cast<long long *>(a.key_stage) + (size_t)pl * (a.w_diag ? 1 : p.nw) * B
-                                          : reinterpret_cast<long long *>(a.key_action) + (a.w_diag ? (size_t)pl * B : 0);
-                            tp = reinterpret_cast<long long *>(a.key_task) + (a.w_diag ? (size_t)pl * B : 0);
-                            kp += (size_t)(wi * wblk) * kstep + b;
-                            tp += (size_t)(wi * wblk) * kstep + b;
-                        }
-                        const int nw_job = p.nw;
-                        float *const q_row = (q_out != nullptr && row_ok) ? q_out + ((size_t)b * n_pol_job + pl) * A_ : nullptr;
-                        if (gpi_form && !k_staged) {
-                            // Rolled 8-column scan (gpi_scan_rolled, forward_tc.cuh): this code runs once per tile, so it is
-                            // instruction-FETCH bound -- the unrolled 32-column windows below cost 9-13 k cycles per tile for 36
-                            // columns (profiles/r02_forward_chain.md), the rolled loop ~2.5 k.  Every emission is an atomicMax,
-                            // so a chunk needs no state from the previous one and each group takes one 128-column half.
-                            long long *ka = a.key_action ? reinterpret_cast<long long *>(a.key_action) + (a.w_diag ? (size_t)pl * B : 0) + b : nullptr;
-                            long long *kt = a.key_task ? reinterpret_cast<long long *>(a.key_task) + (a.w_diag ? (size_t)pl * B : 0) + b : nullptr;
-                            const int c_hi = min(col0_it + n_cols_it, ncol);
-                            const int cb = wblk > 1 ? col0_it + group * 128 : (group == slot ? col0_it : c_hi);
-                            const int ce = wblk > 1 ? min(cb + 128, c_hi) : c_hi;
-                            const uint32_t tid_ = (uint32_t)(task_base + pl);
-                            if (cb < ce) {
-                                if (wblk == 8) gpi_scan_rolled<8>(t_lane, bias - 4u * col0_it, col0_it, cb, ce, A_, nw_job, ka, kt, kstep, row_ok, tid_, q_row);
-                                else if (wblk == 4) gpi_scan_rolled<4>(t_lane, bias - 4u * col0_it, col0_it, cb, ce, A_, nw_job, ka, kt, kstep, row_ok, tid_, q_row);
-                                else gpi_scan_rolled<1>(t_lane, bias - 4u * col0_it, col0_it, cb, ce, A_, nw_job, ka, kt, kstep, row_ok, tid_, q_row);
-                            }
-                        } else if (gpi_form && wblk > 1) {
-                            // (staged keys only) blocked GPI scan: 32 columns per TMEM load, then four 8-column sub-trips out of registers.  (Double-
-                            // buffering the loads was tried: no gain at 256 reward vectors and the extra 32 live registers cost the
-                            // hidden-layer epilogues ~5 us per launch in spills.)
-                            if (group == slot) {
-                                const uint32_t tid_ = (uint32_t)(task_base + pl);
-#pragma unroll 1
-                                for (int c0 = 0; c0 < n_cols_it; c0 += 32) {
-                                    uint32_t v[32];
-                                    tmem_ld32(t_lane + c0, v);
-                                    tmem_wait_ld();
-#define SFGPI_SCAN(WB, OFF)                                                                                                            \
-    do {                                                                                                                                \
-        const float4 b0_ = lds128(bias + 4u * (c0 + OFF)), b1_ = lds128(bias + 4u * (c0 + OFF + 4));                                    \
-        const float bv_[8] = {b0_.x, b0_.y, b0_.z, b0_.w, b1_.x, b1_.y, b1_.z, b1_.w};                                                  \
-        gpi_scan_blocked<WB, OFF>(v, bv_, col0_it + c0 + OFF, ncol, A_, nw_job, bb, ba, act_i, wi, kp, tp, kstep, k_staged, k_has,      \
-                                  t_has, row_ok, tid_, q_row);                                                                          \
-    } while (0)
-                                    if (wblk == 8) { SFGPI_SCAN(8, 0); SFGPI_SCAN(8, 8); SFGPI_SCAN(8, 16); SFGPI_SCAN(8, 24); }
-                                    else { SFGPI_SCAN(4, 0); SFGPI_SCAN(4, 8); SFGPI_SCAN(4, 16); SFGPI_SCAN(4, 24); }
-#undef SFGPI_SCAN
-                                }
-                            }
-                        } else
-#pragma unroll 1
-                        for (int c0 = c_first; c0 < n_cols_it; c0 += c_step) {
-                            uint32_t v[8];
-                            tmem_ld8(t_lane + c0, v);
-                            const float4 b0 = lds128(bias + 4u * c0), b1 = lds128(bias + 4u * (c0 + 4));
-                            const float bv[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-                            tmem_wait_ld();
-                            if (gpi_form) {
-                                // folded GPI: column = wi * A + act.  The scan is instruction-bound (one thread per row walks every
-                                // column), so the per-column work is kept to add / compare / two selects / count; the key of a
-                                // finished reward vector goes out through the pre-computed pointers.
-                                auto emit = [&]() {
-                                    if (row_ok) {
-                                        if (k_staged) *kp = pack_key(best, (uint32_t)best_a);
-                                        else if (k_has) atomicMax(kp, pack_key(best, (uint32_t)best_a));
-                                        if (t_has) atomicMax(tp, pack_key(best, (uint32_t)(task_base + pl)));
-                                    }
-                                    kp += kstep; tp += kstep;
-                                    act_i = 0; ++wi; best = -INFINITY; best_a = 0;
-                                };
-                                if (col0_it + c0 + 8 <= ncol && !(wi == 0 && q_out != nullptr)) {        // fast path: whole trip valid
-#pragma unroll
-                                    for (int i = 0; i < 8; ++i) {
-                                        const float q = __uint_as_float(v[i]) + bv[i];
-                                        if (q > best) { best = q; best_a = act_i; }
-                                        if (++act_i == A_) emit();
-                                    }
-                                } else {
-#pragma unroll
-                                    for (int i = 0; i < 8; ++i) {
-                                        if (col0_it + c0 + i < ncol) {
-                                            const float q = __uint_as_float(v[i]) + bv[i];
-                                            if (wi == 0 && q_out != nullptr && row_ok)
-                                                q_out[((size_t)b * n_pol_job + pl) * A_ + act_i] = q;
-                                            if (q > best) { best = q; best_a = act_i; }
-                                            if (++act_i == A_) emit();
-                                        }
-                                    }
-                                }
-                            } else {
-                                const int colb = col0_it + c0;
-                                float val[8];
-#pragma unroll
-                                for (int i = 0; i < 8; ++i) val[i] = __uint_as_float(v[i]) + bv[i];
-                                if (row_ok) {
-                                    if (psi_out != nullptr) {
-                                        float *po = psi_out + ((size_t)b * n_pol_job + pl) * AD + colb;
-                                        if ((AD & 3) == 0) {                  // rows are 16-byte aligned: 128-bit stores
-                                            if (colb < AD) *reinterpret_cast<float4 *>(po) = make_float4(val[0], val[1], val[2], val[3]);
-                                            if (colb + 4 < AD) *reinterpret_cast<float4 *>(po + 4) = make_float4(val[4], val[5], val[6], val[7]);
-                                        } else {
-#pragma unroll
-                                            for (int i = 0; i < 8; ++i)
-                                                if (colb + i < AD) po[i] = val[i];
-                                        }
-                                    }
-                                    if ((unsigned)(colb + 7 - sb) < (unsigned)(D + 7)) {         // group overlaps [sel, sel + D)
-                                        float *so = sel_out + ((size_t)pl * B + b) * D;
-#pragma unroll
-                                        for (int i = 0; i < 8; ++i) {
-                                            const unsigned off = (unsigned)(colb + i - sb);
-                                            if (off < (unsigned)D) so[off] = val[i];
-                                        }
-                                    }
-                                }
-                            }
+                        const int col0_it = ii.col0, ncol = gpi_ncols(p.nw, A_), wblk = gpi_wblock(p.nw);
+                        const uint32_t kstep = a.w_diag ? 0u : (uint32_t)B;
+                        float *const q_row = (a.q_out != nullptr && row_ok) ? a.q_out + ((size_t)b * a.n_pol + pl) * A_ : nullptr;
+                        long long *ka = a.key_action ? reinterpret_cast<long long *>(a.key_action) + (a.w_diag ? (size_t)pl * B : 0) + b : nullptr;
+                        long long *kt = a.key_task ? reinterpret_cast<long long *>(a.key_task) + (a.w_diag ? (size_t)pl * B : 0) + b : nullptr;
+                        const int c_hi = min(col0_it + ii.n_cols, ncol);
+                        const int cb = wblk > 1 ? col0_it + group * 128 : (group == slot ? col0_it : c_hi);
+                        const int ce = wblk > 1 ? min(cb + 128, c_hi) : c_hi;
+                        const uint32_t tid_ = (uint32_t)(a.task_base + pl);
+                        if (cb < ce) {
+                            if (wblk == 8) gpi_scan_rolled<8>(t_lane, bias - 4u * col0_it, col0_it, cb, ce, A_, p.nw, ka, kt, kstep, row_ok, tid_, q_row);
+                            else if (wblk == 4) gpi_scan_rolled<4>(t_lane, bias - 4u * col0_it, col0_it, cb, ce, A_, p.nw, ka, kt, kstep, row_ok, tid_, q_row);
+                            else gpi_scan_rolled<1>(t_lane, bias - 4u * col0_it, col0_it, cb, ce, A_, p.nw, ka, kt, kstep, row_ok, tid_, q_row);
                         }
                         tc_fence_before();
-                        if (it + 1 < p.n_items) slot_ready(slot);                  // next chunk may overwrite the accumulator
+                        if (it + 1 < p.n_items) mbar_arrive(SLOT_READY(slot));                  // next chunk may overwrite the accumulator
                     }
                     TL_EPI();                                 // epilogue of (item, slot) done
                 }
@@ -665,11 +495,11 @@ mlp_forward_tc_kernel(const __grid_constant__ TcMulti m, const __grid_constant__
         unsigned long long gt; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt)); m.timeline[1024 + blockIdx.x] = (long long)gt;
     }
     tc_fence_before();
-    if (TWO) cluster_sync_all(); else __syncthreads();       // (pair: nobody retires while the peer may still touch it)
+    __syncthreads();
     if (warp == kMmaWarp) {
         __syncwarp();
         tc_fence_after();
-        if (TWO) tmem_dealloc2(tmem_base, 512); else tmem_dealloc(tmem_base, 512);
+        tmem_dealloc(tmem_base, 512);
     }
     trace_exit(SFGPI_TR_FWD);
 }
@@ -984,9 +814,8 @@ static int make_tmap_acts(CUtensorMap *tm, const void *base, uint64_t slabs, uin
     return SFGPI_OK;
 }
 
-static int g_two_cta_min = getenv("SFGPI_2CTA_MIN") ? atoi(getenv("SFGPI_2CTA_MIN")) : 0x7fffffff;
-static int g_forward_chain = getenv("SFGPI_CHAIN") ? atoi(getenv("SFGPI_CHAIN")) : 1;
-static int g_wide_min = getenv("SFGPI_WIDE_MIN") ? atoi(getenv("SFGPI_WIDE_MIN")) : 256;
+static int g_forward_chain = 1;
+static int g_wide_min = 256;
 
 // developer aid (SFGPI_TIMELINE=1): dump CTA 0's role timelines (cycles since the first stamp)
 static void dump_timeline(long long *tl_buf, cudaStream_t st, int n_jobs, int units, int grid, const char *mode) {
@@ -1026,14 +855,10 @@ static bool tc_shape_ok(const sfgpi_net_desc &net, const char **why) {
 using namespace sfgpi;
 using namespace sfgpi::tc;
 
-// Runtime options of the tensor-core path.  "2cta_min_tiles": launches with more row tiles than this use 2-CTA pairs
-// (default: never); returns the previous value, or -1 for an unknown option.
+// Runtime options of the tensor-core forward.  Each moves a choice between two code paths that give the same bits, which the
+// code otherwise makes from the launch size, so that tests can run the other path and compare.  Returns the previous value,
+// or -1 for an unknown option.
 extern "C" int sfgpi_set_option(const char *name, int32_t value) {
-    if (name != nullptr && strcmp(name, "2cta_min_tiles") == 0) {
-        const int old = g_two_cta_min;
-        g_two_cta_min = value;
-        return old;
-    }
     if (name != nullptr && strcmp(name, "forward_chain") == 0) {      // 0: never, 1 (default): launches of <= 148 tiles, 2: always
         const int old = g_forward_chain;
         g_forward_chain = value;
@@ -1185,7 +1010,6 @@ extern "C" int sfgpi_mlp_forward_tc_jobs(const sfgpi_forward_tc_job *jobs, int32
         TcParams &p = m.job[m.n_jobs];
         p.a = a;
         p.gpi = a.w != nullptr ? 1 : 0;
-        { static const bool dry = getenv("SFGPI_GPI_DRY") != nullptr; if (dry && p.gpi) { p.a.key_action = nullptr; p.a.key_task = nullptr; } }   // developer aid: scan without emissions
         if (p.gpi && (a.psi_out || a.sel_out)) {
             set_error("sfgpi_mlp_forward_tc: the GPI form cannot also emit psi / gathered rows (use a separate job)");
             return SFGPI_E_INVALID;
@@ -1226,19 +1050,13 @@ extern "C" int sfgpi_mlp_forward_tc_jobs(const sfgpi_forward_tc_job *jobs, int32
     if (tl_on) cudaMemsetAsync(tl_buf, 0, 1280 * sizeof(long long), (cudaStream_t)stream);
     m.timeline = tl_on ? tl_buf : nullptr;
     m.wide_min = g_wide_min;
-    static const int pair_min = getenv("SFGPI_PAIR_MIN") ? atoi(getenv("SFGPI_PAIR_MIN")) : 148;
-    // 2-CTA pairs are opt-in (sfgpi_set_option("2cta_min_tiles", n) or env SFGPI_2CTA_MIN): measured on B200 they remove the
-    // shared-memory bound of the MMA phase (3100-3300 -> 2300-2600 cycles per tile-layer) but the cluster-scope hand-off makes
-    // every epilogue ~500 cycles longer, and the epilogue chain is then the critical path: 0.506 ms vs 0.448 ms at N=64, B=16384.
-    const int two_min = g_two_cta_min;
-    const int paired = total_tiles > pair_min ? 1 : 0;           // small launches: one tile per CTA, no ping-pong partner
-    const bool two = paired && total_tiles > two_min;            // >= 2 row tiles per SM: 2-CTA pairs (4 tiles per work unit)
+    const int paired = total_tiles > 148 ? 1 : 0;                // small launches: one tile per CTA, no ping-pong partner
     // Launches that fit in ONE wave (<= 148 row tiles: every CTA has a single tile, nothing to ping-pong with) take the layer-
     // pipelined single-tile kernel (mlp_chain_tc.cu): measured 84 vs 90 us per B = 32 step.  Larger launches keep the ping-pong
     // pairs: with the MMA phase shared-memory-bound at ~3 k cycles per tile-layer, overlapping it with ANOTHER tile's epilogue
     // (3.1 k per tile-layer) beats overlapping it with its own tile's previous epilogue (~5 k), 50 vs 52 us at 384 tiles.
     // sfgpi_set_option("forward_chain", 0 / 1 / 2) = never / one-wave launches (default) / always.
-    if (g_forward_chain && (g_forward_chain > 1 || total_tiles <= 148) && !two && forward_chain_supported(m)) {
+    if (g_forward_chain && (g_forward_chain > 1 || total_tiles <= 148) && forward_chain_supported(m)) {
         for (int j = m.n_jobs; j < kMaxJobs; ++j) { m.job[j] = m.job[0]; maps.w[j] = maps.w[0]; maps.q[j] = maps.q[0]; maps.acts[j] = maps.acts[0]; }
         const int grid = launch_forward_chain(m, maps, total_tiles, (cudaStream_t)stream);
         if (tl_on) dump_timeline(tl_buf, (cudaStream_t)stream, m.n_jobs, m.total_pairs, grid, "chain (one tile, layer-pipelined)");
@@ -1249,7 +1067,7 @@ extern "C" int sfgpi_mlp_forward_tc_jobs(const sfgpi_forward_tc_job *jobs, int32
     for (int j = 0; j < m.n_jobs; ++j) {
         TcParams &p = m.job[j];
         p.paired = paired;
-        p.pairs_per_policy = two ? (p.tiles_per_policy + 3) / 4 : (paired ? (p.tiles_per_policy + 1) / 2 : p.tiles_per_policy);
+        p.pairs_per_policy = paired ? (p.tiles_per_policy + 1) / 2 : p.tiles_per_policy;
         p.total_pairs = p.pairs_per_policy * p.a.n_pol;
         m.pair_start[j] = m.total_pairs;
         m.total_pairs += p.total_pairs;
@@ -1260,13 +1078,12 @@ extern "C" int sfgpi_mlp_forward_tc_jobs(const sfgpi_forward_tc_job *jobs, int32
     // and singles dearest first (jobs that save activations have the longer epilogues), so CTA c -- which takes units
     // c, c + G, ... -- combines a cheap pair with a single, and the dear pairs at the end of the round get no second unit.
     static UnitTable ut;                                         // (host scratch; the launch copies it into the kernel parameters)
-    static const bool sched_off = getenv("SFGPI_SCHED_OFF") != nullptr;
     m.sched = 0;
     {
         const int G = 148, rounds = total_tiles / (2 * G), left = total_tiles - 2 * rounds * G;
         int q_total = 0;
         for (int j = 0; j < m.n_jobs; ++j) q_total += m.job[j].a.n_pol;
-        if (!sched_off && paired && !two && rounds >= 1 && left > 0 && left <= G && q_total <= 0x1FFF) {
+        if (paired && rounds >= 1 && left > 0 && left <= G && q_total <= 0x1FFF) {
             const int p_target = rounds * G;
             int order[kMaxJobs], nj = m.n_jobs;
             for (int j = 0; j < nj; ++j) order[j] = j;
@@ -1277,26 +1094,19 @@ extern "C" int sfgpi_mlp_forward_tc_jobs(const sfgpi_forward_tc_job *jobs, int32
             int n_units = 0;
             bool ok = true;
             // Which tiles run as singles: a lone tile costs ~1.6x a paired one (nothing hides its MMA phase) and the jobs that save
-            // activations have the longer epilogues, so the singles are taken from the CHEAPEST jobs first (env SFGPI_SCHED_EVEN=1:
-            // an even share of every job, the round-1 rule) and every other tile is paired.
+            // activations have the longer epilogues, so the singles are taken from the CHEAPEST jobs first and every other tile
+            // is paired.
             static int np_buf[0x2000];
-            static const bool even = getenv("SFGPI_SCHED_EVEN") != nullptr;
             int qi = 0, given = 0;
             int singles_left = total_tiles - 2 * p_target;
             for (int oi = 0; oi < nj && ok; ++oi) {
                 const TcParams &p = m.job[order[oi]];
                 if (p.tiles_per_policy > 0xFFFF) { ok = false; break; }
                 for (int pl = 0; pl < p.a.n_pol; ++pl, ++qi) {
-                    int share;
-                    if (even) {
-                        share = (int)((long long)p_target * (qi + 1) / q_total - (long long)p_target * qi / q_total);
-                        if (share > p.tiles_per_policy / 2) share = p.tiles_per_policy / 2;
-                    } else {
-                        int s1 = singles_left < p.tiles_per_policy ? singles_left : p.tiles_per_policy;
-                        if ((p.tiles_per_policy - s1) & 1) s1 += (s1 < p.tiles_per_policy) ? 1 : -1;      // the rest pairs up
-                        singles_left -= s1;
-                        share = (p.tiles_per_policy - s1) / 2;
-                    }
+                    int s1 = singles_left < p.tiles_per_policy ? singles_left : p.tiles_per_policy;
+                    if ((p.tiles_per_policy - s1) & 1) s1 += (s1 < p.tiles_per_policy) ? 1 : -1;      // the rest pairs up
+                    singles_left -= s1;
+                    const int share = (p.tiles_per_policy - s1) / 2;
                     np_buf[qi] = share;
                     given += share;
                 }
@@ -1327,14 +1137,12 @@ extern "C" int sfgpi_mlp_forward_tc_jobs(const sfgpi_forward_tc_job *jobs, int32
     const int smem_bytes = 2 * kABytes + kNStage * kStageBytes + kBiasFloatsMax * 4 + 256;
     static bool cfg = false;
     if (!cfg) {
-        cudaFuncSetAttribute(mlp_forward_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-        cudaFuncSetAttribute(mlp_forward_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
+        cudaFuncSetAttribute(mlp_forward_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
         cfg = true;
     }
-    const int grid = two ? (m.total_pairs < 74 ? 2 * m.total_pairs : 148) : (m.total_pairs < 148 ? m.total_pairs : 148);
-    if (two) launch_pdl_cluster(mlp_forward_tc_kernel<true>, dim3(grid), dim3(kThreadsTc), smem_bytes, (cudaStream_t)stream, 2, m, maps, ut);
-    else launch_pdl(mlp_forward_tc_kernel<false>, dim3(grid), dim3(kThreadsTc), smem_bytes, (cudaStream_t)stream, m, maps, ut);
-    if (tl_on) dump_timeline(tl_buf, (cudaStream_t)stream, m.n_jobs, m.total_pairs, grid, two ? "2-CTA pairs" : (m.sched ? "pairs + singles (unit table)" : (paired ? "paired" : "one-tile")));
+    const int grid = m.total_pairs < 148 ? m.total_pairs : 148;
+    launch_pdl(mlp_forward_tc_kernel, dim3(grid), dim3(kThreadsTc), smem_bytes, (cudaStream_t)stream, m, maps, ut);
+    if (tl_on) dump_timeline(tl_buf, (cudaStream_t)stream, m.n_jobs, m.total_pairs, grid, m.sched ? "pairs + singles (unit table)" : (paired ? "paired" : "one-tile"));
     return check_launch("sfgpi_mlp_forward_tc");
 }
 

@@ -409,7 +409,7 @@ mlp_forward_stream_kernel(const __grid_constant__ SMulti m, const __grid_constan
     do {                                                                                                                                \
         const float4 b0_ = lds128(bias + 4u * (c0 + OFF)), b1_ = lds128(bias + 4u * (c0 + OFF + 4));                                    \
         const float bv_[8] = {b0_.x, b0_.y, b0_.z, b0_.w, b1_.x, b1_.y, b1_.z, b1_.w};                                                  \
-        gpi_scan_blocked<WB, OFF>(v, bv_, col0_it + c0 + OFF, ncol, A_, nw_job, bb, ba, act_i, wi, kp, tp, kstep, false, k_has,         \
+        gpi_scan_blocked<WB, OFF>(v, bv_, col0_it + c0 + OFF, ncol, A_, nw_job, bb, ba, act_i, wi, kp, tp, kstep, k_has,                \
                                   t_has, row_ok, tid_, q_row);                                                                          \
     } while (0)
                             if (wblk == 8) { SFGPI_SCAN(8, 0); SFGPI_SCAN(8, 8); SFGPI_SCAN(8, 16); SFGPI_SCAN(8, 24); }
@@ -867,7 +867,6 @@ extern "C" int sfgpi_mlp_forward_stream(const sfgpi_forward_tc_job *jobs, int32_
             return SFGPI_E_INVALID;
         }
         if (p.gpi && (!jobs[j].wq || !jobs[j].bq)) { set_error("sfgpi_mlp_forward_stream: GPI form needs the folded weights"); return SFGPI_E_INVALID; }
-        if (a.key_stage != nullptr) { set_error("sfgpi_mlp_forward_stream: key_stage is not supported in the tf32 modes"); return SFGPI_E_INVALID; }
         p.nw = p.gpi ? (a.w_diag ? 1 : a.n_w) : 0;
         p.Lh = net.n_layers - 2;
         p.rows_per_policy = sfgpi_bf16_rows_per_policy(&net);

@@ -58,9 +58,6 @@ extern "C" int sfgpi_run(const sfgpi_cmd *cmds, int32_t n, void *stream) {
             case SFGPI_OP_STEP_PREP:
                 rc = sfgpi_step_prep(reinterpret_cast<const sfgpi_step_prep_args *>(c.p[0]), stream);
                 break;
-            case SFGPI_OP_KEYS_REDUCE:
-                rc = sfgpi_keys_reduce(reinterpret_cast<const int64_t *>(c.p[0]), (int32_t)c.i[0], c.i[1], reinterpret_cast<int64_t *>(c.p[1]), stream);
-                break;
             case SFGPI_OP_PACK_F32:
                 rc = sfgpi_pack_f32(reinterpret_cast<const sfgpi_net_desc *>(c.p[0]), reinterpret_cast<const float *>(c.p[1]), (int32_t)c.i[0],
                                     (int32_t)c.i[1], (int32_t)c.i[2], (int32_t)c.i[3], reinterpret_cast<float *>(c.p[2]),

@@ -137,20 +137,6 @@ __device__ __forceinline__ void mbar_wait_warp(uint32_t bar, uint32_t parity) {
         if (spin > (1u << 26)) __trap();
     }
 }
-// same, acquire at cluster scope: the waiter consumes shared memory written by the PEER CTA (2-CTA pairs)
-__device__ __forceinline__ void mbar_wait_warp_cluster(uint32_t bar, uint32_t parity) {
-    uint32_t done = 0;
-    for (uint32_t spin = 0; !done; ++spin) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(done)
-            : "r"(bar), "r"(parity)
-            : "memory");
-        if (spin > (1u << 26)) __trap();
-    }
-}
 __device__ __forceinline__ void mbar_arrive_expect_tx_e(uint32_t bar, uint32_t bytes, uint32_t leader) {
     asm volatile(
         "{\n\t.reg .pred q;\n\t"
@@ -175,62 +161,6 @@ __device__ __forceinline__ void tma_load_3d_e(uint32_t smem_dst, const void *tma
         "@q cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];\n\t}"
         ::"r"(smem_dst), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(bar), "r"(crd0), "r"(crd1), "r"(crd2), "r"(leader)
         : "memory");
-}
-
-// ---------------------------------------------------------------- 2-CTA pairs (cta_group::2)
-// Two CTAs of a cluster (one TPC) share every MMA: M = 256 = 128 rows of A from each CTA, and each CTA holds only HALF of the
-// B operand (N/2 weight rows) -- TMA-in and MMA-read traffic of B halve per SM, which is what bounds the paired forward
-// (DESIGN.md: 384 KB of shared-memory traffic per tile-layer at 128 B/cycle).  Only the leader (cluster rank 0) issues.
-constexpr uint32_t kPeerBitMask = 0xFEFFFFFFu;           // shared::cluster address -> the same offset in CTA 0 of the pair
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_alloc2(uint32_t smem_result, uint32_t ncols) {      // whole warp, in BOTH CTAs
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_result), "r"(ncols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc2(uint32_t taddr, uint32_t ncols) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void umma_bf16_2cta_e(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate,
-                                                 uint32_t leader) {
-    asm volatile(
-        "{\n\t.reg .pred p, q;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "setp.ne.b32 q, %5, 0;\n\t"
-        "@q tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate), "r"(leader)
-        : "memory");
-}
-// arrives (once all prior MMAs of this thread completed) on the barrier at the same offset in BOTH CTAs of the pair
-__device__ __forceinline__ void umma_commit_2cta_e(uint32_t bar, uint32_t leader) {
-    asm volatile(
-        "{\n\t.reg .pred q;\n\t.reg .b16 m;\n\t"
-        "setp.ne.b32 q, %1, 0;\n\t"
-        "mov.b16 m, 3;\n\t"
-        "@q tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], m;\n\t}"
-        ::"r"(bar), "r"(leader)
-        : "memory");
-}
-// TMA load into THIS CTA's shared memory whose bytes are counted on the pair leader's barrier (bar = shared::cta offset)
-__device__ __forceinline__ void tma_load_2d_2cta_e(uint32_t smem_dst, const void *tmap, uint32_t bar, int crd0, int crd1,
-                                                   uint32_t leader) {
-    asm volatile(
-        "{\n\t.reg .pred q;\n\t"
-        "setp.ne.b32 q, %5, 0;\n\t"
-        "@q cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];\n\t}"
-        ::"r"(smem_dst), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(bar & kPeerBitMask), "r"(crd0), "r"(crd1), "r"(leader)
-        : "memory");
-}
-// arrive on the barrier at offset `bar` in CTA 0 of the pair (local or remote), cluster-scope release
-__device__ __forceinline__ void mbar_arrive_leader(uint32_t bar) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar & kPeerBitMask) : "memory");
 }
 
 // mbarrier arrives once all previously issued MMAs of this thread have completed (implies fence::before_thread_sync)

@@ -16,7 +16,6 @@ the agents hold VIEWS of row i, so `.parameters()`, `state_dict()`, `update_mode
 working.  No torch op is on the compute path; torch only owns the memory and the stream.
 """
 import ctypes as C
-import os
 import math
 
 import numpy as np
@@ -442,8 +441,7 @@ class PackedSFLibrary:
                 ws['dzo16'], ws['xo16'] = bf(n_pol, B, adp), bf(B, 64)
                 ws['masks'] = torch.zeros(L - 1, n_pol, B, 8, dtype=torch.int32, device=self.device)   # ReLU sign bits
                 items = (sp.dims[-1] + 127) // 128 + 2 * (L - 1)
-                want = int(os.environ.get('SFGPI_WGRAD_SPLIT', '0')) or max(1, 148 // (items * n_pol))       # (env: experiment knob)
-                n_split = _lib.lib().sfgpi_bwd_tc_splits(B, want)                                # one wave of CTAs
+                n_split = _lib.lib().sfgpi_bwd_tc_splits(B, max(1, 148 // (items * n_pol)))      # one wave of CTAs
             ws['n_split'] = n_split
             ws['grad_part'] = torch.zeros(n_pol, n_split, sp.row_stride, dtype=torch.float32, device=self.device)
             if self.G is not None:
@@ -611,15 +609,6 @@ class PackedSFLibrary:
             a2 = self._fwd_args(self.online, lo, n_pol, None, B)
             a2.w, a2.n_w, a2.w_diag = P(self.w), n_pol, 1
         a2.key_action = ptr(keys)
-        # Staged keys (tensor-core mode, GPI over the library; opt-in through SFGPI_STAGE_MIN = smallest n_w * n_pol that uses it):
-        # the epilogue stores per-policy keys and one streaming pass (sfgpi_keys_reduce) takes the MAX over the local policies,
-        # instead of one int64 atomicMax per (policy, vector, state).  Measured on B200 the atomics are NOT the bound even at
-        # 32 policies x 256 reward vectors (33 M atomics per step: 5.48 ms forward with atomics, 5.55 ms staged), and the extra
-        # launch costs ~4 us on the small configurations, so the default keeps the atomics.
-        stage = None
-        if tc and not st_mode and use_gpi and not a2.w_diag and a2.n_w * a2.n_pol >= int(os.environ.get('SFGPI_STAGE_MIN', str(1 << 62))):
-            stage = ws.setdefault(('key_stage', a2.n_w), torch.empty(a2.n_pol, a2.n_w, B, dtype=torch.int64, device=self.device))
-            a2.key_stage = stage.data_ptr()
         # (3) target forward on s', gather psi^-(s')[a*]                                sfdqn.py:330-331
         a3 = self._fwd_args(self.target, lo, n_pol, None, B)
         if tc:
@@ -658,7 +647,7 @@ class PackedSFLibrary:
             b.policy_lo, b.n_pol, b.B, b.d_out = lo, n_pol, B, ptr(ws['d_out'])
             b.acts_bf16, b.dz_bf16, b.dzo_bf16, b.xo_bf16 = (ptr(ws[k]) for k in ('acts16', 'dz16', 'dzo16', 'xo16'))
             b.relu_masks = ptr(ws['masks'])
-            if variant == 2 and os.environ.get('SFGPI_RIDE_EXPAND', '1') != '0':
+            if variant == 2:
                 t.defer_expand, b.expand_td = 1, C.addressof(t)        # TSF expand rides in the dgrad launch (idle SMs)
         else:
             b = _lib.BackwardArgs()
@@ -702,7 +691,7 @@ class PackedSFLibrary:
         ad.beta_loss = (float(beta) if variant == 2 else 1.0) if variant >= 1 else 0.0
         ad.sequential_shared = 1
         return dict(ws=ws, a1=a1, a2=a2, a3=a3, t=t, b=b, ad=ad, n_pol=n_pol, lo=lo, tc=tc, st=st_mode, B=B, ring=0, keys=keys, w_all=w_all, sharded=sharded,
-                    peer=peer, variant=variant, stage=stage,
+                    peer=peer, variant=variant,
                     losses=torch.zeros(64, n_pol, 3, dtype=torch.float32, device=self.device))
 
     def train_step(self, transitions, policy, use_gpi=True, variant=1, beta=1.0, host_losses=None):
@@ -818,9 +807,7 @@ class PackedSFLibrary:
                 ka.keys_all[r] = karena.ptrs[r] + koff
                 ua.x[r] = base.ptrs[r] + xoff
             a2.key_action = karena.local + koff
-            if peer['reduce_cmd'] is not None:
-                peer['reduce_cmd'].p[1] = karena.local + koff
-            elif plan['prep'] is not None:
+            if plan['prep'] is not None:
                 plan['prep'].keys = karena.local + koff
             else:
                 peer['fill_cmd'].p[0] = karena.local + koff
@@ -927,9 +914,6 @@ class PackedSFLibrary:
         st_mode = plan['st']
         merged = plan['tc'] and not st_mode and not (plan['sharded'] and peer is None)
         plan['prep'] = None
-        stage = plan.get('stage')
-        if stage is not None:
-            n_keys = 0                                        # every key is written by the reduction: no fill
         if plan['tc']:
             dref = C.addressof(plan['desc'])
             nw = 1 if a2.w_diag else a2.n_w
@@ -971,8 +955,7 @@ class PackedSFLibrary:
             elif plan['tc']:
                 cmd(seg0, 'PACK_BF16', (dref, self.online.data_ptr(), self._shadow_for('online').data_ptr()), (0, self.n))
                 cmd(seg0, 'PACK_BF16', (dref, self.target.data_ptr(), self._shadow_for('target').data_ptr()), (a3.policy_lo, a3.n_pol))
-            if stage is None:
-                cmd(seg0, 'KEYS_FILL', (keys_ptr,), (n_keys,))
+            cmd(seg0, 'KEYS_FILL', (keys_ptr,), (n_keys,))
             if st_mode:
                 cmd(seg1, 'FOLD_GPI_F32', (dref, self.online.data_ptr(), a2.w, plan['wq'].data_ptr(), plan['bq'].data_ptr()),
                     (a2.policy_lo, a2.n_pol, a2.n_w | (a2.w_diag << 31), self._prec))
@@ -990,9 +973,6 @@ class PackedSFLibrary:
             else:
                 cmd(seg1, 'FORWARD_TC_JOBS', (C.addressof(jobs),), (3,))
             cmd(seg1, 'NOP')                                  # probe slot: event after it
-            if stage is not None:
-                cmd(seg1, 'KEYS_REDUCE', (stage.data_ptr(), keys_ptr), (a2.n_pol, a2.n_w * B))
-                n_reduce = len(seg0) + len(seg1) - 1
         else:
             cmd(seg1, 'FORWARD', (C.addressof(a1),))
             cmd(seg1, 'NOP')
@@ -1048,7 +1028,6 @@ class PackedSFLibrary:
         if peer is not None:
             arr = plan['segments'][0][0]
             peer['fill_cmd'] = arr[n_fill]
-            peer['reduce_cmd'] = arr[n_reduce] if stage is not None else None
 
     def set_probe(self, plan_key, start_event=None, end_event=None):
         """

@@ -86,11 +86,6 @@ typedef struct {
                                        the operands of sfgpi_mlp_backward_tc */
     void *relu_mask_out;            /* tensor-core mode only: [L-1][n_pol][B][8] uint32, bit c%32 of word c/32 = (activation c > 0)
                                        for ReLU layers: all the dgrad chain needs of them */
-    int64_t *key_stage;             /* tensor-core mode only, optional: [n_pol][n_rows][B] (n_rows = 1 if w_diag else n_w).  Given it,
-                                       the GPI epilogue STORES policy p's per-vector action keys here instead of doing an int64
-                                       atomicMax per (policy, vector, state) into key_action; sfgpi_keys_reduce then takes the MAX
-                                       over policies.  (Measured on B200: the atomics are not the bound even at 33 M per launch, so
-                                       the host mirror keeps this opt-in.) */
 } sfgpi_forward_args;
 
 int sfgpi_mlp_forward(const sfgpi_forward_args *args, void *stream);
@@ -102,8 +97,6 @@ int sfgpi_mlp_forward(const sfgpi_forward_args *args, void *stream);
  */
 int sfgpi_keys_fill(int64_t *keys, int64_t n, void *stream);
 int sfgpi_keys_decode(const int64_t *keys, int64_t n, int64_t *index_out, float *value_out, void *stream);
-/* keys_out[i] = max over p < n_pol of stage[p * n + i], i < n: the reduction over policies of staged keys (key_stage above) */
-int sfgpi_keys_reduce(const int64_t *stage, int32_t n_pol, int64_t n, int64_t *keys_out, void *stream);
 
 /*
  * Unfused GPI epilogue on a materialised psi [B][N][A][D] (GPI_w, sfdqn.py:236-239): q_out [B][N][A] (nullable),
@@ -503,7 +496,6 @@ int sfgpi_replay_gather(const sfgpi_replay_args *args, void *stream);
 #define SFGPI_OP_SHARD_PACK 15      /* p0 = w, p1 = h, p2 = h_prev, p3 = x_local, i0 = nw, i1 = nh */
 #define SFGPI_OP_PEER_UNPACK 16     /* p0 = sfgpi_peer_unpack_args */
 #define SFGPI_OP_STEP_PREP 17       /* p0 = sfgpi_step_prep_args */
-#define SFGPI_OP_KEYS_REDUCE 18     /* p0 = stage, p1 = keys_out, i0 = n_pol, i1 = n */
 #define SFGPI_OP_PACK_F32 19        /* p0 = net desc, p1 = params, p2 = shadow, p3 = shadow_t, p4 = wout_t, i0 = policy_lo, i1 = n_pol, i2 = n_policies_total, i3 = precision */
 #define SFGPI_OP_FOLD_GPI_F32 20    /* p0 = net desc, p1 = params, p2 = w, p3 = wq, p4 = bq, i0 = policy_lo, i1 = n_pol, i2 = n_w | w_diag << 31, i3 = precision */
 #define SFGPI_OP_FORWARD_STREAM 21  /* p0 = sfgpi_forward_tc_job[], i0 = n_jobs, i1 = precision */
@@ -570,9 +562,9 @@ int sfgpi_peer_free(void *dptr);
 int sfgpi_peer_reduce_keys(const sfgpi_peer_keys_args *args, void *stream);
 int sfgpi_peer_unpack(const sfgpi_peer_unpack_args *args, void *stream);
 
-/* Runtime options.  Returns the previous value or -1 (unknown option).
- *   "2cta_min_tiles"  tensor-core forward launches with more 128-row tiles than this run as 2-CTA pairs (tcgen05
- *                     cta_group::2, each CTA holds half of every weight block); default: never.
+/* Runtime options.  Returns the previous value or -1 (unknown option).  Both move a choice the library otherwise makes
+ * from the launch size between two code paths that compute the same bits; the tests set them to run the other path and
+ * compare the two.
  *   "forward_chain"   which bf16 forward kernel runs: 0 = ping-pong tile pairs always (csrc/mlp_forward_tc.cu), 1 (default) =
  *                     the layer-pipelined single-tile kernel (csrc/mlp_chain_tc.cu) for launches of <= 148 tiles, 2 = always.
  *   "gpi_wide_min"    folded GPI output layers (n_w * A columns, n_w >= 8) of at least this many columns are scanned by the
