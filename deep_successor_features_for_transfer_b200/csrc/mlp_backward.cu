@@ -1,17 +1,23 @@
 // Backward of the psi MLP, fp32 CUDA-core path: (1) fused dgrad chain, (2) split-K wgrad + bias grad.
 //
-// The loss touches psi(s)[b, a_b, :] only (sfdqn.py:334-335: merge[indices, actions,:] = targets), so dZ of the last layer
-// is D-sparse per row; it is kept as d_out [B][D] in HBM and expanded on the fly while staging shared-memory chunks.
+// The TD loss touches psi(s)[b, a_b, :] only (sfdqn.py:334-335: merge[indices, actions,:] = targets), so dZ of the last layer
+// is D-sparse per row; it is kept as d_out [n_pol][B][D] in HBM and expanded on the fly while staging shared-memory chunks.
+// A general loss (autograd through PackedSFLibrary.psi) has a dense dZ of the last layer: actions == NULL, d_out is
+// [B][n_pol][A*D] (the forward's psi_out layout).  Both are template instantiations (kDense), so the sparse kernels are
+// exactly the train step's.
 #include "common.cuh"
 
 namespace sfgpi {
 
 // acc[r][c] += sum_n A[row ty*8+r][n] * W[n][kout0 + c*32+tx],  n in [0, nred)   (NN: reduction index = weight row)
 // dense:  A = As (smem tile, stride lda).   sparse (last layer): A[row][n] = dsel[row][n - sel[row]*D] inside the action's
-// D columns, else 0 -- materialised per 32-wide chunk into dzc.
+// D columns, else 0 -- materialised per 32-wide chunk into dzc.  kDense (last layer of a dense d_out): A[row][n] =
+// dsel[row * dld + n] for the rows_ok rows inside the batch, dsel pointing into d_out in global memory.
+template <bool kDense>
 __device__ __forceinline__ void cta_gemm_nn(float (&acc)[8][8], const float *As, int lda, int nred,
                                             const float *__restrict__ W, int ldw, int kcols, float *Ws, bool sparse,
-                                            float *dzc, const float *dsel, const int *sel_s, int D) {
+                                            float *dzc, const float *dsel, const int *sel_s, int D,
+                                            size_t dld, int rows_ok) {
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5, tid = threadIdx.x;
     const int nc8 = (kcols + 31) >> 5;
     const bool aligned = ((ldw & 3) == 0) && ((reinterpret_cast<uintptr_t>(W) & 15) == 0);
@@ -33,8 +39,12 @@ __device__ __forceinline__ void cta_gemm_nn(float (&acc)[8][8], const float *As,
         if (sparse) {
             for (int e = tid; e < kBM * nlen4; e += kThreads) {
                 int r = e / nlen4, nn = e - r * nlen4;
-                unsigned off = (unsigned)(n0 + nn - sel_s[r] * D);
-                dzc[r * kWsNT + nn] = (nn < nlen && off < (unsigned)D) ? dsel[r * D + off] : 0.0f;
+                if constexpr (kDense) {
+                    dzc[r * kWsNT + nn] = (nn < nlen && r < rows_ok) ? dsel[(size_t)r * dld + n0 + nn] : 0.0f;
+                } else {
+                    unsigned off = (unsigned)(n0 + nn - sel_s[r] * D);
+                    dzc[r * kWsNT + nn] = (nn < nlen && off < (unsigned)D) ? dsel[r * D + off] : 0.0f;
+                }
             }
         }
         if (ch + 1 < nchunks) cp_async_wait<1>(); else cp_async_wait<0>();
@@ -83,7 +93,8 @@ __host__ __device__ inline BwdSmem bwd_smem_layout(const sfgpi_net_desc &net) {
     return s;
 }
 
-// ---- (1) dgrad chain: dZ_{L-1} (sparse) -> dZ_{L-2} -> ... -> dZ_0, all inside one CTA per (policy, 64-row tile) ----
+// ---- (1) dgrad chain: dZ_{L-1} (sparse or dense) -> dZ_{L-2} -> ... -> dZ_0, all inside one CTA per (policy, 64-row tile) ----
+template <bool kDense>
 __global__ void __launch_bounds__(kThreads, 1) mlp_dgrad_kernel(const __grid_constant__ sfgpi_backward_args a) {
     extern __shared__ __align__(16) float smem[];
     const sfgpi_net_desc &net = a.net;
@@ -97,11 +108,17 @@ __global__ void __launch_bounds__(kThreads, 1) mlp_dgrad_kernel(const __grid_con
     const int pl = blockIdx.y, row0 = blockIdx.x * kBM;
     const float *P = a.params + (size_t)(a.policy_lo + pl) * net.row_stride;
 
-    for (int e = tid; e < kBM * D; e += kThreads) {
-        int r = e / D;
-        dsel[e] = (row0 + r < B) ? a.d_out[((size_t)pl * B + row0) * D + e] : 0.0f;
+    const int AD = net.dims[L];
+    const float *dsrc = dsel;
+    if constexpr (kDense) {
+        dsrc = a.d_out + ((size_t)row0 * a.n_pol + pl) * AD;
+    } else {
+        for (int e = tid; e < kBM * D; e += kThreads) {
+            int r = e / D;
+            dsel[e] = (row0 + r < B) ? a.d_out[((size_t)pl * B + row0) * D + e] : 0.0f;
+        }
+        if (tid < kBM) sel_s[tid] = (row0 + tid < B) ? (int)a.actions[row0 + tid] : 0;
     }
-    if (tid < kBM) sel_s[tid] = (row0 + tid < B) ? (int)a.actions[row0 + tid] : 0;
     __syncthreads();
 
     for (int l = L - 1; l >= 1; --l) {
@@ -117,7 +134,8 @@ __global__ void __launch_bounds__(kThreads, 1) mlp_dgrad_kernel(const __grid_con
             for (int r = 0; r < 8; ++r)
 #pragma unroll
                 for (int c = 0; c < 8; ++c) acc[r][c] = 0.0f;
-            cta_gemm_nn(acc, cur, lda, nred, W + k0, K, kcols, Ws, l == L - 1, dzc, dsel, sel_s, D);
+            cta_gemm_nn<kDense>(acc, cur, lda, nred, W + k0, K, kcols, Ws, l == L - 1, dzc, dsrc, sel_s, D,
+                                (size_t)a.n_pol * AD, B - row0);
 #pragma unroll
             for (int c = 0; c < 8; ++c) {
                 const int cc = c * 32 + tx, k = k0 + cc;
@@ -155,6 +173,7 @@ __device__ __forceinline__ int wg_tiles_of_layer(const sfgpi_net_desc &net, int 
     return ((net.dims[l + 1] + kWgN - 1) / kWgN) * ((net.dims[l] + kNC - 1) / kNC);
 }
 
+template <bool kDense>
 __global__ void __launch_bounds__(kThreads, 1) mlp_wgrad_kernel(const __grid_constant__ sfgpi_backward_args a, int tiles_per_split) {
     extern __shared__ __align__(16) float smem[];
     const sfgpi_net_desc &net = a.net;
@@ -200,6 +219,11 @@ __global__ void __launch_bounds__(kThreads, 1) mlp_wgrad_kernel(const __grid_con
         stage_rows(ins, kWsNN, in + (size_t)b0 * K + k0, K, blen, kKC, kcols, nc8 * 32, in_aligned);
         if (!last) {
             stage_rows(dzs, kWgLdz, dz + (size_t)b0 * N + n0, N, blen, kKC, nrows, kWgN, dz_aligned);
+        } else if constexpr (kDense) {                   // dense d_out [B][n_pol][A*D]: row b of policy pl is strided
+            const int ldd = a.n_pol * N;
+            const float *src = a.d_out + ((size_t)b0 * a.n_pol + pl) * N + n0;
+            const bool al = ((ldd & 3) == 0) && ((reinterpret_cast<uintptr_t>(src) & 15) == 0);
+            stage_rows(dzs, kWgLdz, src, ldd, blen, kKC, nrows, kWgN, al);
         } else {
             for (int e = tid; e < kKC * kWgN; e += kThreads) {
                 int r = e / kWgN, nn = e - r * kWgN;
@@ -275,14 +299,21 @@ extern "C" int sfgpi_mlp_backward(const sfgpi_backward_args *args, void *stream)
         return SFGPI_E_INVALID;
     }
     if (a.B == 0 || a.n_pol == 0) return SFGPI_OK;
+    if (!a.d_out) { set_error("sfgpi_mlp_backward: d_out is NULL"); return SFGPI_E_INVALID; }
+    const bool dense = a.actions == nullptr;             // d_out [B][n_pol][A*D] instead of [n_pol][B][D]
     cudaStream_t st = (cudaStream_t)stream;
     if (net.n_layers > 1) {
         const BwdSmem lay = bwd_smem_layout(net);
         if (lay.total_bytes > kMaxSmem) { set_error("sfgpi_mlp_backward: needs %d B shared memory", lay.total_bytes); return SFGPI_E_SMEM; }
         static bool cfg = false;
-        if (!cfg) { cudaFuncSetAttribute(mlp_dgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem); cfg = true; }
+        if (!cfg) {
+            cudaFuncSetAttribute(mlp_dgrad_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem);
+            cudaFuncSetAttribute(mlp_dgrad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem);
+            cfg = true;
+        }
         dim3 grid((a.B + kBM - 1) / kBM, a.n_pol);
-        mlp_dgrad_kernel<<<grid, kThreads, lay.total_bytes, st>>>(a);
+        if (dense) mlp_dgrad_kernel<true><<<grid, kThreads, lay.total_bytes, st>>>(a);
+        else mlp_dgrad_kernel<false><<<grid, kThreads, lay.total_bytes, st>>>(a);
         int rc = check_launch("sfgpi_mlp_backward(dgrad)");
         if (rc) return rc;
     }
@@ -291,8 +322,13 @@ extern "C" int sfgpi_mlp_backward(const sfgpi_backward_args *args, void *stream)
         tiles += ((net.dims[l + 1] + kWgN - 1) / kWgN) * ((net.dims[l] + kNC - 1) / kNC);
     static bool cfg2 = false;
     const int wg_bytes = 2 * kWgStage * (int)sizeof(float);
-    if (!cfg2) { cudaFuncSetAttribute(mlp_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, wg_bytes); cfg2 = true; }
+    if (!cfg2) {
+        cudaFuncSetAttribute(mlp_wgrad_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, wg_bytes);
+        cudaFuncSetAttribute(mlp_wgrad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, wg_bytes);
+        cfg2 = true;
+    }
     dim3 grid(tiles * a.n_split, a.n_pol);
-    mlp_wgrad_kernel<<<grid, kThreads, wg_bytes, st>>>(a, tiles);
+    if (dense) mlp_wgrad_kernel<true><<<grid, kThreads, wg_bytes, st>>>(a, tiles);
+    else mlp_wgrad_kernel<false><<<grid, kThreads, wg_bytes, st>>>(a, tiles);
     return check_launch("sfgpi_mlp_backward(wgrad)");
 }

@@ -5,8 +5,9 @@
 //     tiles ping-ponging on 2 x 256 TMEM columns).  dA_{l-1}[b][k] = sum_n dZ_l[b][n] W_l[n][k]: A = dZ_l is K-major in
 //     shared memory exactly like a forward activation; B = W_l is read from the SAME bf16 shadow as the forward, as an
 //     MN-major operand (its rows are the reduction index), so no transposed copy of the weights exists.  The last layer's
-//     dZ is D-sparse (sfdqn.py:334-335: only psi(s)[b, a_b, :] is in the loss); the epilogue threads expand d_out[b][D] into
-//     the dense row on the fly.  Each epilogue multiplies by the activation derivative (from the bf16 activations the forward
+//     dZ is D-sparse in the train step (sfdqn.py:334-335: only psi(s)[b, a_b, :] is in the loss); the epilogue threads expand
+//     d_out[b][D] into the dense row on the fly.  Autograd through PackedSFLibrary.psi passes a dense dZ instead (actions
+//     NULL, d_out [B][n_pol][A*D]): the same threads read it and convert it to bf16 (the kDense instantiation).  Each epilogue multiplies by the activation derivative (from the bf16 activations the forward
 //     saved), writes the next A operand in place and the row-major bf16 dZ_l to HBM for the wgrad kernel.
 //
 // (2) mlp_wgrad_tc_kernel -- dW_l[n][k] = sum_b dZ_l[b][n] in_l[b][k] and db_l[n] = sum_b dZ_l[b][n], split-K over the batch.
@@ -34,7 +35,7 @@ struct DgParams {
     sfgpi_net_desc net;
     int policy_lo, n_pol, B;
     const long long *actions;        // [B]
-    const float *d_out;              // [n_pol][B][D]
+    const float *d_out;              // [n_pol][B][D]; dense (kDense): [B][n_pol][AD]
     const __nv_bfloat16 *acts;       // [L-1][n_pol][B][256]
     const uint32_t *masks;           // [L-1][n_pol][B][8] ReLU sign bits written by the forward (NULL: derive from acts)
     __nv_bfloat16 *dz;               // [L-1][n_pol][B][256]
@@ -93,7 +94,9 @@ __device__ __forceinline__ DgItem dg_item(const DgParams &p, int it) {
 }
 
 // Expanded dense chunk c of this row's dZ_{L-1}: columns [256c, 256c+256) of a row that is zero except d_out[0..D) at
-// [sel, sel+D).  Written to the A slot (K-major SW128) and, as the wgrad operand, to dzo (row-major bf16).
+// [sel, sel+D) -- or, kDense, the row drow[0..AD) itself, zero past AD.  Written to the A slot (K-major SW128) and, as the
+// wgrad operand, to dzo (row-major bf16).
+template <bool kDense>
 __device__ __forceinline__ void build_dzo_chunk(const DgParams &p, int c, uint32_t Arow, int r, bool row_ok, int sel,
                                                 const float *drow, __nv_bfloat16 *dzo_row, int j0, int jstep) {
     const int D = p.net.n_features;
@@ -104,8 +107,12 @@ __device__ __forceinline__ void build_dzo_chunk(const DgParams &p, int c, uint32
         float v[8];
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
-            const unsigned off = (unsigned)(col0 + i - sel);
-            v[i] = (row_ok && off < (unsigned)D) ? drow[off] : 0.0f;
+            if constexpr (kDense) {
+                v[i] = (row_ok && col0 + i < p.AD) ? drow[col0 + i] : 0.0f;
+            } else {
+                const unsigned off = (unsigned)(col0 + i - sel);
+                v[i] = (row_ok && off < (unsigned)D) ? drow[off] : 0.0f;
+            }
         }
         const uint32_t q0 = pack_bf16x2(v[0], v[1]), q1 = pack_bf16x2(v[2], v[3]), q2 = pack_bf16x2(v[4], v[5]),
                        q3 = pack_bf16x2(v[6], v[7]);
@@ -170,6 +177,7 @@ __device__ __forceinline__ void dgrad_epilogue(uint32_t t_lane, uint32_t Arow, i
     }
 }
 
+template <bool kDense>
 __global__ void __launch_bounds__(kThreadsDg, 1)
 mlp_dgrad_tc_kernel(const __grid_constant__ DgParams p, const __grid_constant__ CUtensorMap tmap_w,
                     const __grid_constant__ CUtensorMap tmap_dz, const __grid_constant__ CUtensorMap tmap_dzo,
@@ -363,10 +371,11 @@ mlp_dgrad_tc_kernel(const __grid_constant__ DgParams p, const __grid_constant__ 
                 bs[slot] = b;
                 const bool row_ok = b < B;
                 const size_t prow = (size_t)pl * B + (row_ok ? b : 0);
-                const int sel = row_ok ? (int)p.actions[b] * D : 0;
+                const int sel = (!kDense && row_ok) ? (int)p.actions[b] * D : 0;
+                const float *drow = kDense ? p.d_out + ((size_t)(row_ok ? b : 0) * p.n_pol + pl) * p.AD : p.d_out + prow * D;
                 guard_slot(slot);
-                build_dzo_chunk(p, 0, sbase + (uint32_t)slot * kABytes, r, row_ok, sel, p.d_out + prow * D, p.dzo + prow * p.ADp,
-                                group, 2);
+                build_dzo_chunk<kDense>(p, 0, sbase + (uint32_t)slot * kABytes, r, row_ok, sel, drow, p.dzo + prow * p.ADp,
+                                        group, 2);
                 fence_proxy_async();
                 mbar_arrive(SLOT_READY(slot));
                 store_tile(&tmap_dzo, slot, (min(256, p.ADp) + kKB - 1) / kKB, 0, pl);
@@ -387,8 +396,9 @@ mlp_dgrad_tc_kernel(const __grid_constant__ DgParams p, const __grid_constant__ 
                     guard_slot(slot);
                     if (it + 1 < p.n_chunks) {                   // more output-layer chunks: refill the A slot
                         const size_t prow = (size_t)pl * B + (row_ok ? b : 0);
-                        const int sel = row_ok ? (int)p.actions[b] * D : 0;
-                        build_dzo_chunk(p, it + 1, Arow, r, row_ok, sel, p.d_out + prow * D, p.dzo + prow * p.ADp, group, 2);
+                        const int sel = (!kDense && row_ok) ? (int)p.actions[b] * D : 0;
+                        const float *drow = kDense ? p.d_out + ((size_t)(row_ok ? b : 0) * p.n_pol + pl) * p.AD : p.d_out + prow * D;
+                        build_dzo_chunk<kDense>(p, it + 1, Arow, r, row_ok, sel, drow, p.dzo + prow * p.ADp, group, 2);
                         fence_proxy_async();
                         mbar_arrive(SLOT_READY(slot));
                         store_tile(&tmap_dzo, slot, (min(256, p.ADp - (it + 1) * 256) + kKB - 1) / kKB, (it + 1) * 256, pl);
@@ -647,6 +657,8 @@ extern "C" int sfgpi_mlp_backward_tc(const sfgpi_backward_tc_args *args, void *s
         if (net.dims[l] != kH) { set_error("sfgpi_mlp_backward_tc: every hidden width must be 256"); return SFGPI_E_INVALID; }
     if (a.B < 0 || a.n_pol < 0 || a.n_split < 1) { set_error("sfgpi_mlp_backward_tc: invalid sizes"); return SFGPI_E_INVALID; }
     if (a.B == 0 || a.n_pol == 0) return SFGPI_OK;
+    if (!a.d_out) { set_error("sfgpi_mlp_backward_tc: d_out is NULL"); return SFGPI_E_INVALID; }
+    const bool dense = a.actions == nullptr;                        // d_out [B][n_pol][A*D] instead of [n_pol][B][D]
     if (sfgpi_bwd_tc_splits(a.B, a.n_split) != a.n_split) {
         set_error("sfgpi_mlp_backward_tc: n_split %d leaves empty batch splits for B=%d (use sfgpi_bwd_tc_splits)", a.n_split, a.B);
         return SFGPI_E_INVALID;
@@ -697,7 +709,11 @@ extern "C" int sfgpi_mlp_backward_tc(const sfgpi_backward_tc_args *args, void *s
     }
     const int dg_smem = 2 * kABytes + kNStage * kStageBytes + 256;
     static bool cfg = false;
-    if (!cfg) { cudaFuncSetAttribute(mlp_dgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, dg_smem); cfg = true; }
+    if (!cfg) {
+        cudaFuncSetAttribute(mlp_dgrad_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, dg_smem);
+        cudaFuncSetAttribute(mlp_dgrad_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dg_smem);
+        cfg = true;
+    }
     dp.n_main = dp.total_pairs < 148 ? dp.total_pairs : 148;
     sfgpi_td_args ex = {};
     int ex_nclu = 0, riders = 0;
@@ -718,7 +734,8 @@ extern "C" int sfgpi_mlp_backward_tc(const sfgpi_backward_tc_args *args, void *s
         cudaMemcpyToSymbol(g_dg_tl_on, &on, sizeof(on));
         cudaMemcpyToSymbol(g_dg_tl, z, sizeof(z));
     }
-    launch_pdl(mlp_dgrad_tc_kernel, dim3(dp.n_main + riders), dim3(kThreadsDg), dg_smem, st, dp, tmap_w, tm_dz_st, tm_dzo_st, ex, ex_nclu);
+    if (dense) launch_pdl(mlp_dgrad_tc_kernel<true>, dim3(dp.n_main + riders), dim3(kThreadsDg), dg_smem, st, dp, tmap_w, tm_dz_st, tm_dzo_st, ex, ex_nclu);
+    else launch_pdl(mlp_dgrad_tc_kernel<false>, dim3(dp.n_main + riders), dim3(kThreadsDg), dg_smem, st, dp, tmap_w, tm_dz_st, tm_dzo_st, ex, ex_nclu);
     rc = check_launch("sfgpi_mlp_backward_tc(dgrad)");
     if (rc) return rc;
     if (dg_tl) {                                                 // developer aid: CTA 0's timeline (cycles since its entry)

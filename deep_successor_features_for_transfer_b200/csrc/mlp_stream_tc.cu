@@ -488,7 +488,8 @@ mlp_forward_stream_kernel(const __grid_constant__ SMulti m, const __grid_constan
 }
 
 // ------------------------------------------------------------------------------------------------------------------------
-// dgrad chain in the same streaming structure: dZ_{L-1} (the D-sparse d_out of the TD step, expanded on the fly) -> dZ_{L-2} ->
+// dgrad chain in the same streaming structure: dZ_{L-1} (the D-sparse d_out of the TD step, expanded on the fly, or with kDense
+// the dense d_out [B][n_pol][A*D] of a general loss, read as it is) -> dZ_{L-2} ->
 // ... -> dZ_0 for one 128-row tile.  dA_{l-1}[b][k] = sum_n dZ_l[b][n] W_l[n][k]: A = dZ_l k-blocks (produced by the epilogue
 // threads exactly like forward activations), B = W_l^T read K-major from the TRANSPOSED operand shadows that sfgpi_pack_f32
 // writes next to the forward ones (so the forward's verified operand path is reused; fp32 MN-major would need the BASE32B
@@ -499,7 +500,7 @@ struct SDg {
     sfgpi_net_desc net;
     int policy_lo, n_pol, B;
     const long long *actions;        // [B]
-    const float *d_out;              // [n_pol][B][D]
+    const float *d_out;              // [n_pol][B][D]; dense (kDense): [B][n_pol][AD]
     const uint32_t *masks;           // [L-1][n_pol][B][8] ReLU sign bits written by the forward
     const float *acts;               // fp32 [parts][L-1][n_pol][B][256] (tanh layers: derivative from the stored outputs)
     int L, Lh, AD, ADp, n_kb0;       // ADp = A*D padded to 32, n_kb0 = ADp / 32
@@ -508,7 +509,7 @@ struct SDg {
     int acts_part_stride;            // floats between the hi and lo activation tensors
 };
 
-template <int PARTS>
+template <int PARTS, bool kDense>
 __global__ void __launch_bounds__(kSThreads, 1)
 mlp_dgrad_stream_kernel(const __grid_constant__ SDg p, const __grid_constant__ CUtensorMap tmap_wt, const __grid_constant__ CUtensorMap tmap_wo,
                         const __grid_constant__ CUtensorMap tmap_dz, const __grid_constant__ CUtensorMap tmap_dzo) {
@@ -616,9 +617,11 @@ mlp_dgrad_stream_kernel(const __grid_constant__ SDg p, const __grid_constant__ C
             const int pl = g / p.tiles_per_policy, tile = g - pl * p.tiles_per_policy;
             const int b = tile * kTM + r;
             const bool row_ok = b < B;
-            const int sel = row_ok ? (int)p.actions[b] * D : 0;
-            const float *drow = p.d_out + ((size_t)pl * B + (row_ok ? b : 0)) * D;
-            // ---- item 0's A operand: the expanded dense dZ_{L-1} row, zero except d_out[0..D) at [sel, sel + D) ----
+            const int sel = (!kDense && row_ok) ? (int)p.actions[b] * D : 0;
+            const float *drow = kDense ? p.d_out + ((size_t)(row_ok ? b : 0) * p.n_pol + pl) * p.AD
+                                       : p.d_out + ((size_t)pl * B + (row_ok ? b : 0)) * D;
+            // ---- item 0's A operand: the expanded dense dZ_{L-1} row, zero except d_out[0..D) at [sel, sel + D) (kDense: the
+            //      row of the dense d_out, zero past AD) ----
 #pragma unroll 1
             for (int kb = 0; kb < p.n_kb0; ++kb, ++n) {
                 const int s = n % NS;
@@ -627,8 +630,12 @@ mlp_dgrad_stream_kernel(const __grid_constant__ SDg p, const __grid_constant__ C
                 const int col0 = kb * kK32 + group * 16;
 #pragma unroll
                 for (int i = 0; i < 16; ++i) {
-                    const unsigned off = (unsigned)(col0 + i - sel);
-                    h[i] = (row_ok && off < (unsigned)D) ? drow[off] : 0.0f;
+                    if constexpr (kDense) {
+                        h[i] = (row_ok && col0 + i < p.AD) ? drow[col0 + i] : 0.0f;
+                    } else {
+                        const unsigned off = (unsigned)(col0 + i - sel);
+                        h[i] = (row_ok && off < (unsigned)D) ? drow[off] : 0.0f;
+                    }
                 }
                 s_write_a16<PARTS>(h, A_addr + s * PARTS * kAPart, r, group * 16);
                 publish(s, &tmap_dzo, kb * kK32, tile * kTM, pl, p.n_pol);
@@ -943,10 +950,11 @@ extern "C" int sfgpi_mlp_backward_stream(const sfgpi_backward_stream_args *args,
     }
     bool relu = false;
     for (int l = 0; l < L - 1; ++l) relu = relu || net.acts[l] == SFGPI_ACT_RELU;
-    if (!a.shadow_t || !a.wout_t || !a.x || !a.acts || !a.actions || !a.d_out || !a.dz || !a.dzo || !a.xo || !a.grad_part || (relu && !a.relu_masks)) {
+    if (!a.shadow_t || !a.wout_t || !a.x || !a.acts || !a.d_out || !a.dz || !a.dzo || !a.xo || !a.grad_part || (relu && !a.relu_masks)) {
         set_error("sfgpi_mlp_backward_stream: missing buffers");
         return SFGPI_E_INVALID;
     }
+    const bool dense = a.actions == nullptr;                          // d_out [B][n_pol][A*D] instead of [n_pol][B][D]
     cudaStream_t st = (cudaStream_t)stream;
     const int S = net.dims[0], AD = net.n_actions * net.n_features, ADp = sfgpi_f32_out_pad(&net), Lh = L - 2;
     launch_pdl(build_xo_f32_kernel, dim3((a.B * 32 + 255) / 256), dim3(256), 0, st, a.x, a.B, S, parts, a.xo);
@@ -983,13 +991,16 @@ extern "C" int sfgpi_mlp_backward_stream(const sfgpi_backward_stream_args *args,
     const int smem = NS * parts * (kAPart + kBPart) + 256;
     static bool cfg = false;
     if (!cfg) {
-        cudaFuncSetAttribute(mlp_dgrad_stream_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        cudaFuncSetAttribute(mlp_dgrad_stream_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        cudaFuncSetAttribute(mlp_dgrad_stream_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        cudaFuncSetAttribute(mlp_dgrad_stream_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        cudaFuncSetAttribute(mlp_dgrad_stream_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        cudaFuncSetAttribute(mlp_dgrad_stream_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         cfg = true;
     }
     const int grid = dp.total_units < 148 ? dp.total_units : 148;
-    if (parts == 2) launch_pdl(mlp_dgrad_stream_kernel<2>, dim3(grid), dim3(kSThreads), smem, st, dp, tm_wt, tm_wo, tm_dz, tm_dzo);
-    else launch_pdl(mlp_dgrad_stream_kernel<1>, dim3(grid), dim3(kSThreads), smem, st, dp, tm_wt, tm_wo, tm_dz, tm_dzo);
+    auto kern = parts == 2 ? (dense ? mlp_dgrad_stream_kernel<2, true> : mlp_dgrad_stream_kernel<2, false>)
+                           : (dense ? mlp_dgrad_stream_kernel<1, true> : mlp_dgrad_stream_kernel<1, false>);
+    launch_pdl(kern, dim3(grid), dim3(kSThreads), smem, st, dp, tm_wt, tm_wo, tm_dz, tm_dzo);
     rc = check_launch("sfgpi_mlp_backward_stream(dgrad)");
     if (rc) return rc;
     return sfgpi_wgrad_tf32_launch(net, parts, a.n_pol, a.B, a.dz, a.dzo, a.acts, a.xo, ADp, a.grad_part, a.n_split, st);

@@ -20,6 +20,7 @@ import math
 
 import numpy as np
 import torch
+from torch.autograd.function import once_differentiable
 
 from . import _lib
 from ._lib import ACT, MAX_LAYERS, ptr
@@ -117,8 +118,34 @@ def _stream():
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
+class _PsiFunction(torch.autograd.Function):
+    """psi_j(x), j in [lo, lo+n_pol), as a function of the packed ONLINE rows (PackedSFLibrary.psi)."""
+
+    @staticmethod
+    def forward(ctx, online, lib, x, lo, n_pol):
+        out, acts, masks = lib._psi_forward(x, lo, n_pol)
+        # saved through save_for_backward: freed by the backward (unless retain_graph), a second backward raises
+        ctx.save_for_backward(x, acts, masks)
+        ctx.lib, ctx.lo, ctx.n_pol, ctx.gen, ctx.precision = lib, lo, n_pol, lib.weights_gen, lib.precision
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, d_psi):
+        lib = ctx.lib
+        if lib.weights_gen != ctx.gen:
+            raise RuntimeError('one of the variables needed for gradient computation has been modified by an inplace operation: '
+                               'the library\'s online psi rows were written (train step, optimizer step, add_policy or reset) '
+                               'after this psi forward')
+        if lib.precision != ctx.precision:       # the saved activations have the layout of the forward's mode
+            raise RuntimeError(f'the library\'s precision mode changed from {ctx.precision!r} to {lib.precision!r} between this psi '
+                               'forward and its backward')
+        x, acts, masks = ctx.saved_tensors
+        return lib._psi_backward(x, ctx.lo, ctx.n_pol, acts, masks, d_psi), None, None, None, None
+
+
 class PackedSFLibrary:
-    def __init__(self, device=None, lr=None, wd=None, tsf_dim=None, capacity=4, precision='fp32'):
+    def __init__(self, device=None, lr=None, wd=None, tsf_dim=None, capacity=4, precision='fp32', autograd=False):
         if not torch.cuda.is_available():
             raise RuntimeError('deep_successor_features_for_transfer_b200 needs a CUDA device (sm_100a); there is no CPU path')
         _lib.lib()                                   # fail loudly right here if the native library is missing
@@ -137,6 +164,12 @@ class PackedSFLibrary:
         self.shard = None           # dist.ShardContext once enable_sharding() was called
         self._xchg = None
         self._peer = None           # peer-memory exchange state (enable_sharding on an NVLink node)
+        # autograd: the online storage is a leaf that requires grad, psi() records a differentiable forward and the packed
+        # gradient [cap][row_stride] accumulates in online.grad.  weights_gen counts library-side writes of the online rows.
+        self.autograd = bool(autograd)
+        self.weights_gen = 0
+        self._grad_rows = set()     # rows whose gradient psi() backward has written since their optimizer's zero_grad
+        self._bound_rows = set()    # ... of which the psi Linear modules' .grad are bound to their view of online.grad
         self.set_precision(precision)
 
     def set_precision(self, precision):
@@ -290,21 +323,35 @@ class PackedSFLibrary:
             gl = self.G * sp.dims[0] + self.G + self.n_flows * (2 * sp.dims[0] + 1)      # W | b | K x (weight | bias | scale)
             hl = sp.n_features * self.G + sp.n_features
             new.update(g=z(cap, gl), g_m=z(cap, gl), g_v=z(cap, gl), h_m=z(cap, hl), h_v=z(cap, hl))
-        for k, t in new.items():
-            old = getattr(self, k, None)
-            if old is not None and self.n > 0:
-                t[:self.n].copy_(old[:self.n])
-            setattr(self, k, t)
+        old_grad = getattr(self, 'online', None)
+        old_grad = None if old_grad is None else old_grad.grad
+        with torch.no_grad():
+            for k, t in new.items():
+                old = getattr(self, k, None)
+                if old is not None and self.n > 0:
+                    t[:self.n].copy_(old[:self.n])
+                setattr(self, k, t)
+        if self.autograd:
+            self.online.requires_grad_(True)
+            self.online.register_post_accumulate_grad_hook(PackedSFLibrary._grad_hook(self))
+            if old_grad is not None:
+                self.online.grad = torch.zeros_like(self.online)
+                self.online.grad[:self.n].copy_(old_grad[:self.n])
+            self._bound_rows = set()
         self.cap = cap
         self._adam_par = (getattr(self, '_adam_par', None) or []) + [0] * (cap - len(getattr(self, '_adam_par', None) or []))
         self._ws = {}
         self.invalidate_exchange()
         for i, mods in enumerate(self._views):
             self._point_views(i, mods)
+        if self.autograd:
+            self._bind_grads()
 
     def _point_views(self, i, mods):
-        for (W, b), lin in zip(self.spec.views(self.online[i]), mods['online']):
+        for (W, b), lin in zip(self.spec.views(self.online.detach()[i]), mods['online']):
             lin.weight.data, lin.bias.data = W, b
+            if self.autograd:                                # (re)bound to online.grad by _bind_grads
+                lin.weight.grad = lin.bias.grad = None
         for (W, b), lin in zip(self.spec.views(self.target[i]), mods['target']):
             lin.weight.data, lin.bias.data = W, b
         mods['w'].weight.data = self.w[i].view(1, -1)
@@ -371,6 +418,7 @@ class PackedSFLibrary:
         self._views.append(mods)
         self._point_views(i, mods)
         self.n += 1
+        self.weights_gen += 1
         # cached train-step plans hard-code the policy count (GPI range, pack range, 'all' = n policies): drop them
         self._drop_plans()
         self.invalidate_exchange()
@@ -397,6 +445,8 @@ class PackedSFLibrary:
         self._close_peer()
         self.spec, self.n, self.cap, self._views, self._ws, self.h = None, 0, 0, [], {}, None
         self._adam_par = []
+        self.weights_gen += 1
+        self._grad_rows, self._bound_rows = set(), set()
         for k in ('online', 'target', 'm', 'v', 'w', 'w_m', 'w_v', 'step', 'adam_consts', 'adam_consts2', 'g', 'g_m', 'g_v', 'h_m', 'h_v'):
             if hasattr(self, k):
                 delattr(self, k)
@@ -483,6 +533,125 @@ class PackedSFLibrary:
         a.psi_out = ptr(out)
         self._forward(a, 'target' if target else 'online')
         return out
+
+    def psi(self, x, lo=0, n_pol=None):
+        """
+        Differentiable psi_j(x), j in [lo, lo+n_pol) of the ONLINE nets: [B][n_pol][A][D], equal to forward_psi bit for bit.
+        Under grad mode the result carries a backward that runs the precision mode's backward kernels on the dense dL/dpsi and
+        accumulates dL/d(row) into online.grad ([cap][row_stride], library row layout); every psi Linear of a row that received
+        a gradient then has its .grad bound to its view of that buffer.  Needs a library built with autograd=True.  The
+        backward raises if the library wrote the online rows after this forward (weights_gen).  Inputs that require grad are
+        refused: there is no input gradient.
+        """
+        if not self.autograd:
+            raise RuntimeError('psi() needs a library built with autograd=True')
+        if self._sharded:
+            raise NotImplementedError('psi() does not support sharded libraries')
+        if isinstance(x, torch.Tensor) and x.requires_grad:
+            raise ValueError('psi() has no gradient with respect to the states: pass x.detach()')
+        x = self._check_x(x)
+        n_pol = self.n - lo if n_pol is None else n_pol
+        if not (0 <= lo and n_pol >= 1 and lo + n_pol <= self.n):
+            raise IndexError('policy range out of bounds')
+        return _PsiFunction.apply(self.online, self, x, lo, n_pol)
+
+    def _psi_forward(self, x, lo, n_pol):
+        """forward_psi that also keeps what the backward needs: activations (and ReLU masks) allocated for this call alone,
+        because several recorded forwards (e.g. psi(s) and psi(s')) can be alive at once.  Returns (psi, acts, masks): fp32
+        mode, acts is one flat buffer holding every hidden layer's [n_pol][B][width] (see _fp32_acts) and masks is None.
+        torch.empty: the forward kernels store every activation the backward reads (every row < B, all 256 columns of the
+        tensor-core layouts, the mask words of every ReLU layer; masks of other layers are never read)."""
+        sp, B = self.spec, x.shape[0]
+        L = len(sp.acts)
+        out = self._f(B, n_pol, sp.n_actions, sp.n_features)
+        a = self._fwd_args(self.online, lo, n_pol, x)
+        a.psi_out = ptr(out)
+        masks = None
+        if self.precision == 'fp32':
+            acts = self._f(n_pol * B * sum(sp.dims[1:L]))
+            for l, t in enumerate(self._fp32_acts(acts, n_pol, B)):
+                a.acts_out[l] = t.data_ptr()
+        else:
+            shape = (self._parts, L - 1, n_pol, B, 256) if self._stream else (L - 1, n_pol, B, 256)
+            acts = torch.empty(*shape, dtype=torch.float32 if self._stream else torch.bfloat16, device=self.device)
+            masks = torch.empty(L - 1, n_pol, B, 8, dtype=torch.int32, device=self.device)
+            a.acts_bf16_out, a.relu_mask_out = acts.data_ptr(), masks.data_ptr()
+        self._forward(a, 'online')
+        return out, acts, masks
+
+    def _fp32_acts(self, flat, n_pol, B):
+        """Per-layer [n_pol][B][dims[l+1]] views of the fp32 mode's flat activation buffer."""
+        sp, out, off = self.spec, [], 0
+        for l in range(len(sp.acts) - 1):
+            n = n_pol * B * sp.dims[l + 1]
+            out.append(flat[off:off + n].view(n_pol, B, sp.dims[l + 1]))
+            off += n
+        return out
+
+    def _psi_backward(self, x, lo, n_pol, acts, masks, d_psi):
+        """Dense-d_out backward of one psi() forward -> gradient w.r.t. the whole online storage (rows outside zero)."""
+        sp, B = self.spec, x.shape[0]
+        d_psi = d_psi.to(torch.float32).contiguous()                 # [B][n_pol][A][D]: the psi_out layout the kernels read
+        ws = self._workspace(B, n_pol, n_pol)
+        if self._stream:
+            self._pack('online', lo, n_pol, transposed=True)
+            b = _lib.BackwardStreamArgs()
+            sh_t, wo_t = self._shadow_t()
+            b.net, b.precision, b.shadow_t, b.wout_t, b.n_policies_total = sp.desc(), self._prec, ptr(sh_t), ptr(wo_t), self.cap
+            b.acts, b.dz, b.dzo, b.xo = ptr(acts), ptr(ws['dz32']), ptr(ws['dzo32']), ptr(ws['xo32'])
+            b.relu_masks = ptr(masks)
+            name = 'sfgpi_mlp_backward_stream'
+        elif self.precision != 'fp32':
+            self._pack('online', lo, n_pol)
+            b = _lib.BackwardTcArgs()
+            b.net, b.params_bf16, b.n_policies_total = sp.desc(), ptr(self._shadow_for('online')), self.cap
+            b.acts_bf16, b.dz_bf16, b.dzo_bf16, b.xo_bf16 = ptr(acts), ptr(ws['dz16']), ptr(ws['dzo16']), ptr(ws['xo16'])
+            b.relu_masks = ptr(masks)
+            name = 'sfgpi_mlp_backward_tc'
+        else:
+            b = _lib.BackwardArgs()
+            b.net, b.params = sp.desc(), ptr(self.online)
+            for l, t in enumerate(self._fp32_acts(acts, n_pol, B)):
+                b.acts[l] = t.data_ptr()
+                b.dz[l] = ws['dz'][l].data_ptr()
+            name = 'sfgpi_mlp_backward'
+        b.policy_lo, b.n_pol, b.B = lo, n_pol, B
+        b.x, b.actions, b.d_out = x.data_ptr(), None, d_psi.data_ptr()          # actions NULL: d_out is dense
+        b.grad_part, b.n_split = ptr(ws['grad_part']), ws['n_split']
+        _lib.call(name, C.byref(b), _stream())
+        if self.online.grad is not None:
+            # rows whose psi .grad a stock torch optimizer's zero_grad() set to None: start their accumulation afresh
+            for i in sorted(self._bound_rows & set(range(lo, lo + n_pol))):
+                if all(p.grad is None for lin in self._views[i]['online'] for p in (lin.weight, lin.bias)):
+                    self.online.grad[i].zero_()
+                    self._bound_rows.discard(i)
+        grad = torch.zeros(self.online.shape, dtype=torch.float32, device=self.device)
+        torch.sum(ws['grad_part'], dim=1, out=grad[lo:lo + n_pol])
+        self._grad_rows.update(range(lo, lo + n_pol))
+        return grad
+
+    @staticmethod
+    def _grad_hook(lib):
+        """post-accumulate-grad hook of the online storage: bind the psi Linear .grad of every row with a gradient to its view
+        of online.grad, so that stock torch code (clip_grad_norm_, torch.optim over sf.psi[i][0][0].parameters()) reads the
+        packed gradient and its in-place changes reach it."""
+        import weakref
+        ref = weakref.ref(lib)
+
+        def hook(online):
+            self = ref()
+            if self is not None:
+                self._bind_grads()
+        return hook
+
+    def _bind_grads(self):
+        if self.online.grad is None:
+            return
+        g = self.online.grad.detach()
+        for i in sorted(self._grad_rows - self._bound_rows):
+            for (W, b), lin in zip(self.spec.views(g[i]), self._views[i]['online']):
+                lin.weight.grad, lin.bias.grad = W, b
+            self._bound_rows.add(i)
 
     def gpi(self, x, w_vec, lo=0, n_pol=None, want_q=True, task_base=None, keys_out=None, reduce=True):
         """
@@ -730,6 +899,7 @@ class PackedSFLibrary:
         if variant == 2 and self.G is None:
             raise Exception('Affine Function (h) is not initialized')          # tsfdqn.py:592-593
         key = ('plan', B, policy, bool(use_gpi), variant, float(beta))
+        self.weights_gen += 1
         plan = self._ws.get(key)
         if plan is None:
             plan = self._ws[key] = self._build_plan(B, policy, use_gpi, variant, beta)
@@ -1117,6 +1287,7 @@ class PackedSFLibrary:
         i = int(policy)
         if not (0 <= i < self.n):
             raise IndexError('policy index out of range')
+        self.weights_gen += 1
         psp = phi_lib.spec
         if psp.n_features != D or psp.n_actions != 1:
             raise ValueError('the phi network must map cat[s, a, s\'] to n_features values')
@@ -1209,4 +1380,5 @@ class PackedSFLibrary:
 
     def target_sync(self, i):
         """update_models_weights(psi_model, target_psi_model) (utils/torch.py:31-33): one contiguous D2D row copy."""
-        self.target[i].copy_(self.online[i])
+        with torch.no_grad():
+            self.target[i].copy_(self.online.detach()[i])

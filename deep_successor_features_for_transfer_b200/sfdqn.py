@@ -157,14 +157,24 @@ class PackedPsi(torch.nn.Module):
 
     def forward(self, state):
         lib = self._lib_ref[0]
+        if lib.autograd and not self.is_target and torch.is_grad_enabled():
+            return lib.psi(state, self.index, 1)[:, 0]
         return lib.forward_psi(state, self.index, 1, target=self.is_target)[:, 0]
 
 
 class PackedAdamView:
-    """Read-only view of optimizer i's state in the packed buffers, shaped like torch.optim.Adam's `state` / `param_groups`."""
+    """
+    Optimizer i's Adam in the packed buffers, shaped like torch.optim.Adam's `state` / `param_groups`.  The fused train step
+    steps it inside update_successor.  On a library built with autograd=True, step() / zero_grad() also work the reference's
+    eager way (optim.zero_grad(); loss.backward(); optim.step()): one sfgpi_adam_step launch over the groups that have
+    gradients -- the psi row from the packed gradient online.grad[i], w, and for TSF g and the shared h -- sharing `step`
+    and the bias corrections with the fused step, so both kinds of step can be mixed.
+    """
 
-    def __init__(self, library, index, groups):
+    def __init__(self, library, index, groups, eager_unsupported=None):
         self._library, self.index, self._groups = library, index, groups
+        self._eager_unsupported = eager_unsupported
+        self._skipped = set()        # groups left out of an eager step while others were stepped
 
     @property
     def param_groups(self):
@@ -186,14 +196,113 @@ class PackedAdamView:
         return out
 
     def zero_grad(self, set_to_none=True):
-        pass
+        """Clears optimizer i's psi row of the packed gradient and the .grad of every parameter it steps (w, g and the
+        shared h included, as torch.optim.Adam.zero_grad does for its groups)."""
+        L = self._library
+        if not L.autograd:
+            return
+        i = self.index
+        if L.online.grad is not None:
+            L.online.grad[i].zero_()
+        L._grad_rows.discard(i)
+        L._bound_rows.discard(i)
+        for _, params in self._groups:
+            for p in params:
+                if p.grad is None:
+                    continue
+                if set_to_none:
+                    p.grad = None
+                else:
+                    p.grad.detach_().zero_()
 
     def step(self):
-        raise RuntimeError('the packed Adam is stepped inside update_successor (fused kernel); it has no standalone step()')
+        L, i = self._library, self.index
+        if not L.autograd:
+            raise RuntimeError('the packed Adam is stepped inside update_successor (fused kernel); it has no standalone step()')
+        if self._eager_unsupported is not None or L.n_flows > 0:
+            raise NotImplementedError(f'optim.step() is not supported for {self._eager_unsupported or "normalising-flow g functions"}; '
+                                      'use the fused update_successor')
+        if L._sharded:
+            raise NotImplementedError('optim.step() does not support sharded libraries')
+        have = {}
+        for k, params in self._groups:
+            n_grad = sum(p.grad is not None for p in params)
+            if 0 < n_grad < len(params):
+                raise RuntimeError(f"optimizer {i}: only some parameters of the '{k}' group have gradients; the packed Adam "
+                                   'steps a group as a whole')
+            have[k] = n_grad > 0
+        have.setdefault('g', False)
+        have.setdefault('h', False)
+        for k in self._skipped:
+            if have[k]:
+                raise RuntimeError(f"optimizer {i}: the '{k}' group was skipped by an earlier step and now has gradients; the "
+                                   'packed per-optimizer step counter cannot represent a per-parameter step')
+        if not any(have.values()):
+            return
+        self._skipped |= {k for k, h in have.items() if not h}
+        self._launch(have)
+
+    def _launch(self, have):
+        import ctypes as C
+        from . import _lib
+        from .library import _stream
+        L, i = self._library, self.index
+        sp = L.spec
+        keep = []                                    # tensors that must outlive the launch call
+
+        def grad_of(p):
+            g = p.grad.detach()
+            if g.dtype != torch.float32 or not g.is_contiguous() or g.device != L.device:
+                g = g.to(device=L.device, dtype=torch.float32).contiguous()
+            keep.append(g)
+            return g.data_ptr()
+
+        ad = _lib.AdamArgs()
+        ad.n_pol, ad.step = 1, L.step[i:].data_ptr()
+        ad.beta1, ad.beta2, ad.eps = 0.9, 0.999, 1e-8
+        ad.sequential_shared = 1
+        segs = []
+        if have['sf']:
+            rs = sp.row_stride
+            row = L.online.grad[i]
+            for (W, b), lin in zip(sp.views(row), L._views[i]['online']):      # .grad rebound by the user: copy it back
+                for view, p in ((W, lin.weight), (b, lin.bias)):
+                    if p.grad.data_ptr() != view.data_ptr():
+                        view.copy_(p.grad)
+            segs.append((L.online.detach()[i].data_ptr(), 0, L.m[i].data_ptr(), L.v[i].data_ptr(), row.data_ptr(), rs, 'sf'))
+        if have['w']:
+            segs.append((L.w[i].data_ptr(), 0, L.w_m[i].data_ptr(), L.w_v[i].data_ptr(), grad_of(self._groups[1][1][0]), sp.n_features, 'w'))
+        if L.G is not None:
+            S, G, D = sp.dims[0], L.G, sp.n_features
+            if have['g']:
+                gW, gb = self._groups[2][1]
+                segs.append((L.g[i].data_ptr(), 0, L.g_m[i].data_ptr(), L.g_v[i].data_ptr(), grad_of(gW), G * S, 'g'))
+                o = 4 * G * S
+                segs.append((L.g[i].data_ptr() + o, 0, L.g_m[i].data_ptr() + o, L.g_v[i].data_ptr() + o, grad_of(gb), G, 'g'))
+            if have['h']:
+                hW, hb = self._groups[3][1]
+                segs.append((L.h.data_ptr(), 0, L.h_m[i].data_ptr(), L.h_v[i].data_ptr(), grad_of(hW), D * G, 'h'))
+                o = 4 * D * G
+                segs.append((L.h.data_ptr() + o, 0, L.h_m[i].data_ptr() + o, L.h_v[i].data_ptr() + o, grad_of(hb), D, 'h'))
+        for k, (param, pstride, m, v, grad, length, kind) in enumerate(segs):
+            s = ad.seg[k]
+            s.param, s.param_stride, s.m, s.m_stride, s.v, s.v_stride = param, pstride, m, 0, v, 0
+            s.grad_part, s.grad_pol_stride, s.grad_part_stride, s.n_part = grad, 0, length, 1
+            s.len, s.lr, s.weight_decay = length, L.lr[kind], L.wd[kind]
+        ad.n_seg = len(segs)
+        # bias corrections: the same double-buffered pair the fused step reads and advances (library.train_step)
+        par = L._adam_par[i]
+        cur, nxt = (L.adam_consts, L.adam_consts2) if par == 0 else (L.adam_consts2, L.adam_consts)
+        ad.consts, ad.consts_next = cur[i:].data_ptr(), nxt[i:].data_ptr()
+        _lib.call('sfgpi_adam_step', C.byref(ad), _stream())
+        L._adam_par[i] = par ^ 1
+        L.weights_gen += 1
 
 
 class DeepSF:
     """Successor-feature library, G2 ("sequential") semantics  [sfdqn.py:94-371]."""
+
+    _eager_step_unsupported = None
 
     def __init__(self, pytorch_model_handle, use_true_reward=False, target_update_ev=1000, **kwargs):
         self.use_true_reward = use_true_reward
@@ -205,6 +314,9 @@ class DeepSF:
         self._tsf_dim = None
         self._library = None
         self.precision = kwargs.get('precision', self.hyperparameters.get('precision', 'fp32'))
+        # autograd=True: get_successor(s) and the online psi modules record a differentiable forward under grad mode, and the
+        # optimizers' step() / zero_grad() work, so the reference's eager update code runs on the packed library
+        self.autograd = bool(kwargs.get('autograd', self.hyperparameters.get('autograd', False)))
 
     # ---- library construction -------------------------------------------------------------------------------------
     def _hyper(self, kind, default):
@@ -212,7 +324,7 @@ class DeepSF:
 
     def _new_library(self):
         lr, wd = self._hyper('learning_rate', 1e-3), self._hyper('weight_decay', 0.0)
-        return PackedSFLibrary(self.device, lr=lr, wd=wd, tsf_dim=self._tsf_dim, precision=self.precision)
+        return PackedSFLibrary(self.device, lr=lr, wd=wd, tsf_dim=self._tsf_dim, precision=self.precision, autograd=self.autograd)
 
     def reset(self):
         self.n_tasks = 0
@@ -264,14 +376,18 @@ class DeepSF:
         groups = [('sf', list(model.parameters())), ('w', list(w_approx.parameters()))]
         if g_function is not None:
             groups += [('g', list(g_function.parameters())), ('h', list(h_function.parameters()))]
-        optim = PackedAdamView(self._library, index, groups)
+        optim = PackedAdamView(self._library, index, groups, eager_unsupported=self._eager_step_unsupported)
         return (online, loss, optim), (target, None, None)
 
     # ---- forwards ---------------------------------------------------------------------------------------------------
     def get_successor(self, state, policy_index):
+        if self.autograd and torch.is_grad_enabled():
+            return self._library.psi(state, policy_index, 1)[:, 0]
         return self._library.forward_psi(state, policy_index, 1)[:, 0]
 
     def get_successors(self, state):
+        if self.autograd and torch.is_grad_enabled():
+            return self._library.psi(state, 0, self.n_tasks)
         return self._library.forward_psi(state, 0, self.n_tasks)
 
     # ---- GPI ----------------------------------------------------------------------------------------------------------

@@ -244,6 +244,8 @@ class DeepSF_PHI(DeepSF):
     torch.optim.Adam per call.
     """
 
+    _eager_step_unsupported = 'DeepSF_PHI (its step is the joint psi / phi update)'
+
     def add_training_task(self, task, source=None):
         n_features = task.feature_dim()
         self.psi.append(None)                                                     # (reference order: psi nets first, then fit_w, :262-270)

@@ -162,6 +162,8 @@ int sfgpi_td_step(const sfgpi_td_args *args, void *stream);
  * Backward of the psi MLP for n_pol policies: fused dgrad chain (dZ_l for every layer, activations' derivative from the
  * saved outputs) followed by split-K wgrad + bias grad.  The last layer's dZ is the sparse d_out (only the taken
  * action's D columns are non-zero, sfdqn.py:334-335).
+ * actions == NULL: d_out is DENSE, dL/dpsi of a general loss in the layout of the forward's psi_out, [B][n_pol][A*D] fp32
+ * (the same rule holds for sfgpi_mlp_backward_tc and sfgpi_mlp_backward_stream).
  *   dz [l][n_pol][B][dims[l+1]] for l = 0..L-2 (scratch, caller-allocated);
  *   grad_part [n_pol][n_split][row_stride]: split-K partial gradients in library row layout.
  */
@@ -172,8 +174,8 @@ typedef struct {
     const float *x;                 /* [B][S] */
     int32_t B;
     const float *acts[SFGPI_MAX_LAYERS];
-    const int64_t *actions;         /* [B] */
-    const float *d_out;             /* [n_pol][B][D] */
+    const int64_t *actions;         /* [B]; NULL: d_out is dense */
+    const float *d_out;             /* [n_pol][B][D]; dense: [B][n_pol][A*D] */
     float *dz[SFGPI_MAX_LAYERS];
     float *grad_part;
     int32_t n_split;
@@ -267,7 +269,8 @@ int sfgpi_mlp_forward_tc_jobs(const sfgpi_forward_tc_job *jobs, int32_t n_jobs, 
 /*
  * Tensor-core backward (bf16 operands, fp32 accumulate), the mode-1 twin of sfgpi_mlp_backward: dgrad chain + split-K wgrad of
  * autograd's backward through psi (sfdqn.py:345, tsfdqn.py:645).  Reads the online rows' bf16 shadow (sfgpi_pack_bf16), the
- * bf16 activations saved by sfgpi_mlp_forward_tc (acts_bf16_out) and the sparse d_out of sfgpi_td_step; writes fp32 split
+ * bf16 activations saved by sfgpi_mlp_forward_tc (acts_bf16_out) and the sparse d_out of sfgpi_td_step (or, actions == NULL, a
+ * dense d_out [B][n_pol][A*D] fp32, rounded to bf16 like every other operand); writes fp32 split
  * partials in library row layout for sfgpi_adam_step.  Scratch (caller-allocated, bf16): dz_bf16 [L-1][n_pol][B][256],
  * dzo_bf16 [n_pol][B][sfgpi_bwd_tc_out_pad()], xo_bf16 [B][64].  n_split must equal sfgpi_bwd_tc_splits(B, wanted).
  * Same shape limits and stated tolerance as sfgpi_mlp_forward_tc, and S <= 63.
@@ -281,8 +284,8 @@ typedef struct {
     int32_t B;
     const void *acts_bf16;          /* [L-1][n_pol][B][256] */
     const void *relu_masks;         /* [L-1][n_pol][B][8] uint32 from sfgpi_mlp_forward_tc (relu_mask_out); NULL: signs from acts */
-    const int64_t *actions;         /* [B] */
-    const float *d_out;             /* [n_pol][B][D] */
+    const int64_t *actions;         /* [B]; NULL: d_out is dense */
+    const float *d_out;             /* [n_pol][B][D]; dense: [B][n_pol][A*D] */
     void *dz_bf16;
     void *dzo_bf16;
     void *xo_bf16;
@@ -323,6 +326,7 @@ int sfgpi_mlp_forward_stream(const sfgpi_forward_tc_job *jobs, int32_t n_jobs, i
  * Backward of the psi MLP in the tf32 modes (the twin of sfgpi_mlp_backward_tc): streaming dgrad chain on the transposed operand
  * shadows + split-K wgrad with MN-major fp32 operands (csrc/mlp_stream_tc.cu, csrc/mlp_wgrad_tf32.cu).  Scratch (caller-allocated
  * fp32, parts = 1 / 2): dz [parts][L-1][n_pol][B][256], dzo [parts][n_pol][B][sfgpi_f32_out_pad()], xo [parts][B][32].
+ * actions == NULL: d_out is dense, [B][n_pol][A*D] fp32 (split into hi / lo like the sparse one).
  */
 typedef struct {
     sfgpi_net_desc net;
@@ -334,8 +338,8 @@ typedef struct {
     int32_t B;
     const float *acts;              /* [parts][L-1][n_pol][B][256] from sfgpi_mlp_forward_stream (acts_bf16_out) */
     const void *relu_masks;         /* [L-1][n_pol][B][8] uint32 from the forward (required for ReLU layers) */
-    const int64_t *actions;         /* [B] */
-    const float *d_out;             /* [n_pol][B][D] */
+    const int64_t *actions;         /* [B]; NULL: d_out is dense */
+    const float *d_out;             /* [n_pol][B][D]; dense: [B][n_pol][A*D] */
     float *dz, *dzo, *xo;
     float *grad_part;               /* [n_pol][n_split][row_stride] */
     int32_t n_split;                /* == sfgpi_bwd_tc_splits(B, wanted) */
