@@ -11,7 +11,7 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB_PATH = os.environ.get('SFGPI_LIB_PATH') or os.path.join(HERE, 'libsfgpi.so')      # (override: A/B runs of two builds)
-SOURCES = ['mlp_forward.cu', 'gpi.cu', 'td.cu', 'mlp_backward.cu', 'adam.cu', 'mlp_forward_tc.cu', 'mlp_chain_tc.cu', 'mlp_backward_tc.cu', 'run.cu', 'replay.cu', 'peer.cu', 'phi.cu', 'mlp_stream_tc.cu', 'mlp_wgrad_tf32.cu', 'g4.cu', 'target.cu']
+SOURCES = ['mlp_forward.cu', 'gpi.cu', 'td.cu', 'mlp_backward.cu', 'adam.cu', 'mlp_forward_tc.cu', 'mlp_chain_tc.cu', 'mlp_backward_tc.cu', 'run.cu', 'replay.cu', 'peer.cu', 'phi.cu', 'mlp_stream_tc.cu', 'mlp_wgrad_tf32.cu', 'g4.cu', 'target.cu', 'input_grad.cu']
 MAX_LAYERS = 8
 MAX_SEGMENTS = 8
 ACT = {'none': 0, 'relu': 1, 'tanh': 2}
@@ -97,6 +97,11 @@ class BackwardStreamArgs(C.Structure):
                 ('n_policies_total', C.c_int32), ('policy_lo', C.c_int32), ('n_pol', C.c_int32), ('x', C.c_void_p), ('B', C.c_int32),
                 ('acts', C.c_void_p), ('relu_masks', C.c_void_p), ('actions', C.c_void_p), ('d_out', C.c_void_p), ('dz', C.c_void_p),
                 ('dzo', C.c_void_p), ('xo', C.c_void_p), ('grad_part', C.c_void_p), ('n_split', C.c_int32)]
+
+
+class InputGradArgs(C.Structure):
+    _fields_ = [('net', NetDesc), ('precision', C.c_int32), ('params', C.c_void_p), ('policy_lo', C.c_int32), ('n_pol', C.c_int32),
+                ('B', C.c_int32), ('dz0', C.c_void_p), ('dz0_part_stride', C.c_int64), ('dx', C.c_void_p)]
 
 
 class StepPrepArgs(C.Structure):
@@ -202,6 +207,7 @@ SYMBOLS = {
                                      C.c_void_p, C.c_void_p, C.c_void_p]),
     'sfgpi_mlp_forward_stream': (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
     'sfgpi_mlp_backward_stream': (C.c_int, [C.POINTER(BackwardStreamArgs), C.c_void_p]),
+    'sfgpi_mlp_input_grad': (C.c_int, [C.POINTER(InputGradArgs), C.c_void_p]),
     'sfgpi_g4_head': (C.c_int, [C.POINTER(G4Args), C.c_void_p]),
     'sfgpi_target_q': (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     'sfgpi_target_adapt': (C.c_int, [C.POINTER(TargetArgs), C.c_void_p]),

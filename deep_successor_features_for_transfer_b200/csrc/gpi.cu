@@ -156,7 +156,7 @@ __global__ void __launch_bounds__(256) gpi_from_psi_kernel(const float *__restri
 using namespace sfgpi;
 
 extern "C" const char *sfgpi_last_error(void) { return g_err; }
-extern "C" int sfgpi_version(void) { return 102; }
+extern "C" int sfgpi_version(void) { return 103; }
 
 extern "C" int sfgpi_keys_fill(int64_t *keys, int64_t n, void *stream) {
     if (n <= 0) return SFGPI_OK;

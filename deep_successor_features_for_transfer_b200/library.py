@@ -119,7 +119,8 @@ def _stream():
 
 
 class _PsiFunction(torch.autograd.Function):
-    """psi_j(x), j in [lo, lo+n_pol), as a function of the packed ONLINE rows (PackedSFLibrary.psi)."""
+    """psi_j(x), j in [lo, lo+n_pol), as a function of the packed ONLINE rows and, on a library built with state_grad=True, of
+    the states x (PackedSFLibrary.psi)."""
 
     @staticmethod
     def forward(ctx, online, lib, x, lo, n_pol):
@@ -141,11 +142,15 @@ class _PsiFunction(torch.autograd.Function):
             raise RuntimeError(f'the library\'s precision mode changed from {ctx.precision!r} to {lib.precision!r} between this psi '
                                'forward and its backward')
         x, acts, masks = ctx.saved_tensors
-        return lib._psi_backward(x, ctx.lo, ctx.n_pol, acts, masks, d_psi), None, None, None, None
+        grad, dx = lib._psi_backward(x, ctx.lo, ctx.n_pol, acts, masks, d_psi, want_dx=ctx.needs_input_grad[2])
+        return grad, None, dx, None, None
 
 
 class PackedSFLibrary:
-    def __init__(self, device=None, lr=None, wd=None, tsf_dim=None, capacity=4, precision='fp32', autograd=False):
+    def __init__(self, device=None, lr=None, wd=None, tsf_dim=None, capacity=4, precision='fp32', autograd=False,
+                 state_grad=False):
+        if state_grad and not autograd:
+            raise ValueError('state_grad=True needs autograd=True')
         if not torch.cuda.is_available():
             raise RuntimeError('deep_successor_features_for_transfer_b200 needs a CUDA device (sm_100a); there is no CPU path')
         _lib.lib()                                   # fail loudly right here if the native library is missing
@@ -167,6 +172,8 @@ class PackedSFLibrary:
         # autograd: the online storage is a leaf that requires grad, psi() records a differentiable forward and the packed
         # gradient [cap][row_stride] accumulates in online.grad.  weights_gen counts library-side writes of the online rows.
         self.autograd = bool(autograd)
+        # state_grad: psi() also takes states that require grad and its backward returns dL/dx (sfgpi_mlp_input_grad)
+        self.state_grad = bool(state_grad)
         self.weights_gen = 0
         self._grad_rows = set()     # rows whose gradient psi() backward has written since their optimizer's zero_grad
         self._bound_rows = set()    # ... of which the psi Linear modules' .grad are bound to their view of online.grad
@@ -525,6 +532,10 @@ class PackedSFLibrary:
 
     def forward_psi(self, x, lo=0, n_pol=None, target=False):
         """psi_j(x) for j in [lo, lo+n_pol): [B][n_pol][A][D] (get_successors / get_next_successors)."""
+        if target and self.state_grad and torch.is_grad_enabled() and isinstance(x, torch.Tensor) and x.requires_grad:
+            # a result without a backward would silently cut the states' gradient; torch would raise or differentiate
+            raise RuntimeError('the target psi nets are constants and have no gradient with respect to the states: call them under '
+                               'torch.no_grad() or pass the states .detach()ed')
         x = self._check_x(x)
         n_pol = self.n - lo if n_pol is None else n_pol
         sp = self.spec
@@ -540,15 +551,22 @@ class PackedSFLibrary:
         Under grad mode the result carries a backward that runs the precision mode's backward kernels on the dense dL/dpsi and
         accumulates dL/d(row) into online.grad ([cap][row_stride], library row layout); every psi Linear of a row that received
         a gradient then has its .grad bound to its view of that buffer.  Needs a library built with autograd=True.  The
-        backward raises if the library wrote the online rows after this forward (weights_gen).  Inputs that require grad are
-        refused: there is no input gradient.
+        backward raises if the library wrote the online rows after this forward (weights_gen).
+        States that require grad are refused unless the library was built with state_grad=True.  Then the backward also returns
+        dL/dx = sum_j dZ0_j . W0_j over the n_pol nets (one sfgpi_mlp_input_grad launch on the layer-0 gradient the backward
+        kernels leave in their scratch), and autograd carries it back through the dtype / device conversion and the
+        unsqueeze of a 1-D state, so x.grad has x's own dtype and shape.  States that do not require grad cost nothing extra.
         """
         if not self.autograd:
             raise RuntimeError('psi() needs a library built with autograd=True')
         if self._sharded:
             raise NotImplementedError('psi() does not support sharded libraries')
         if isinstance(x, torch.Tensor) and x.requires_grad:
-            raise ValueError('psi() has no gradient with respect to the states: pass x.detach()')
+            if not self.state_grad:
+                raise ValueError('psi() has no gradient with respect to the states: pass x.detach(), or build the library with '
+                                 'state_grad=True')
+            if self.spec is not None and len(self.spec.acts) < 2:
+                raise NotImplementedError('state gradients need a psi net with at least one hidden layer')
         x = self._check_x(x)
         n_pol = self.n - lo if n_pol is None else n_pol
         if not (0 <= lo and n_pol >= 1 and lo + n_pol <= self.n):
@@ -588,8 +606,9 @@ class PackedSFLibrary:
             off += n
         return out
 
-    def _psi_backward(self, x, lo, n_pol, acts, masks, d_psi):
-        """Dense-d_out backward of one psi() forward -> gradient w.r.t. the whole online storage (rows outside zero)."""
+    def _psi_backward(self, x, lo, n_pol, acts, masks, d_psi, want_dx=False):
+        """Dense-d_out backward of one psi() forward -> (gradient w.r.t. the whole online storage (rows outside zero), dL/dx
+        [B][S] when want_dx, else None)."""
         sp, B = self.spec, x.shape[0]
         d_psi = d_psi.to(torch.float32).contiguous()                 # [B][n_pol][A][D]: the psi_out layout the kernels read
         ws = self._workspace(B, n_pol, n_pol)
@@ -619,6 +638,7 @@ class PackedSFLibrary:
         b.x, b.actions, b.d_out = x.data_ptr(), None, d_psi.data_ptr()          # actions NULL: d_out is dense
         b.grad_part, b.n_split = ptr(ws['grad_part']), ws['n_split']
         _lib.call(name, C.byref(b), _stream())
+        dx = self._input_grad(ws, lo, n_pol, B) if want_dx else None     # while dZ_0 is in the workspace
         if self.online.grad is not None:
             # rows whose psi .grad a stock torch optimizer's zero_grad() set to None: start their accumulation afresh
             for i in sorted(self._bound_rows & set(range(lo, lo + n_pol))):
@@ -628,7 +648,22 @@ class PackedSFLibrary:
         grad = torch.zeros(self.online.shape, dtype=torch.float32, device=self.device)
         torch.sum(ws['grad_part'], dim=1, out=grad[lo:lo + n_pol])
         self._grad_rows.update(range(lo, lo + n_pol))
-        return grad
+        return grad, dx
+
+    def _input_grad(self, ws, lo, n_pol, B):
+        """dL/dx [B][S] = sum_j dZ0_j . W0_j from the layer-0 gradient the last backward into workspace `ws` left there."""
+        g = ws.get('input_grad')
+        if g is None:                                                # built once per workspace (dropped with the storage)
+            g = ws['input_grad'] = _lib.InputGradArgs()
+            g.net, g.precision, g.params, g.n_pol, g.B = self.spec.desc(), self._prec, ptr(self.online), n_pol, B
+            if self._stream:                                         # [parts][L-1][n_pol][B][256]: slab 0 of each part
+                g.dz0, g.dz0_part_stride = ptr(ws['dz32']), ws['dz32'][0].numel()
+            else:
+                g.dz0 = ptr(ws['dz'][0] if self.precision == 'fp32' else ws['dz16'])
+        dx = self._f(B, self.spec.dims[0])
+        g.policy_lo, g.dx = lo, dx.data_ptr()
+        _lib.call('sfgpi_mlp_input_grad', C.byref(g), _stream())
+        return dx
 
     @staticmethod
     def _grad_hook(lib):

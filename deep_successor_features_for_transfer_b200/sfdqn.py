@@ -317,6 +317,12 @@ class DeepSF:
         # autograd=True: get_successor(s) and the online psi modules record a differentiable forward under grad mode, and the
         # optimizers' step() / zero_grad() work, so the reference's eager update code runs on the packed library
         self.autograd = bool(kwargs.get('autograd', self.hyperparameters.get('autograd', False)))
+        # state_grad=True (needs autograd): those forwards also take states that require grad and pass dL/dstate back, e.g. to a
+        # learned state encoder in front of psi.  Target nets stay constants: they raise for such states under grad mode.
+        # GPI / GPI_w / greedy_action are not differentiable.
+        self.state_grad = bool(kwargs.get('state_grad', self.hyperparameters.get('state_grad', False)))
+        if self.state_grad and not self.autograd:
+            raise ValueError('state_grad=True needs autograd=True')
 
     # ---- library construction -------------------------------------------------------------------------------------
     def _hyper(self, kind, default):
@@ -324,7 +330,8 @@ class DeepSF:
 
     def _new_library(self):
         lr, wd = self._hyper('learning_rate', 1e-3), self._hyper('weight_decay', 0.0)
-        return PackedSFLibrary(self.device, lr=lr, wd=wd, tsf_dim=self._tsf_dim, precision=self.precision, autograd=self.autograd)
+        return PackedSFLibrary(self.device, lr=lr, wd=wd, tsf_dim=self._tsf_dim, precision=self.precision, autograd=self.autograd,
+                               state_grad=self.state_grad)
 
     def reset(self):
         self.n_tasks = 0
@@ -392,7 +399,8 @@ class DeepSF:
 
     # ---- GPI ----------------------------------------------------------------------------------------------------------
     def GPI_w(self, state, w):
-        """q [n_batch, n_tasks, n_actions] and the task active in GPI per state (squeezed, sfdqn.py:239)."""
+        """q [n_batch, n_tasks, n_actions] and the task active in GPI per state (squeezed, sfdqn.py:239).  Not differentiable,
+        with autograd / state_grad too: q carries no gradient to psi, w or the states."""
         w_vec = w.weight if isinstance(w, torch.nn.Module) else w
         q, _, key_task = self._library.gpi(state, w_vec)
         task = torch.squeeze(self._library.decode_keys(key_task))

@@ -347,6 +347,32 @@ typedef struct {
 int sfgpi_mlp_backward_stream(const sfgpi_backward_stream_args *args, void *stream);
 
 /*
+ * Gradient of a loss with respect to the psi MLP's INPUT states (csrc/input_grad.cu), from the layer-0 pre-activation gradient dZ_0
+ * that the backward entry points above leave in their scratch.  One state tensor feeds all n_pol nets, so the policies' terms add:
+ *   dx[b][s] = sum_{p < n_pol} sum_{k < dims[1]} dZ0[p][b][k] * W0_{policy_lo+p}[k][s]        dx [B][S] fp32, overwritten
+ * dz0 by precision (the backward's own scratch, read as it is):
+ *   SFGPI_PREC_FP32    fp32 [n_pol][B][dims[1]]   sfgpi_backward_args.dz[0]; any hidden width and S
+ *   SFGPI_PREC_BF16    bf16 [n_pol][B][256]       slab 0 of sfgpi_backward_tc_args.dz_bf16; S <= 63
+ *   SFGPI_PREC_TF32    fp32 [n_pol][B][256]       hi, slab 0 of sfgpi_backward_stream_args.dz; S <= 31
+ *   SFGPI_PREC_TF32X3  as TF32, plus lo at dz0 + dz0_part_stride floats (that scratch's part stride, (L-1)*n_pol*B*256); dZ0 = hi + lo
+ * W_0 is read from the fp32 library rows and used as the mode's forward used it: rounded to bf16 (the sfgpi_pack_bf16 value) in
+ * BF16, to tf32 (the sfgpi_pack_f32 hi value) in TF32, as stored in FP32 / TF32X3.  FFMA with fp32 accumulation; the policies are
+ * summed in a fixed order without atomics, so two calls give the same bits.  One launch; B == 0 or n_pol == 0: none.  Needs
+ * n_layers >= 2 (tensor-core modes: first hidden width 256).
+ */
+typedef struct {
+    sfgpi_net_desc net;
+    int32_t precision;              /* SFGPI_PREC_*: the mode of the backward that wrote dz0 */
+    const float *params;            /* [N][row_stride] fp32 library rows (W_0 at net.w_off[0]) */
+    int32_t policy_lo, n_pol;
+    int32_t B;
+    const void *dz0;                /* layouts above */
+    int64_t dz0_part_stride;        /* SFGPI_PREC_TF32X3: floats from the hi to the lo part; ignored otherwise */
+    float *dx;                      /* [B][S] */
+} sfgpi_input_grad_args;
+int sfgpi_mlp_input_grad(const sfgpi_input_grad_args *args, void *stream);
+
+/*
  * Learned features (phi), SURVEY 8f N3: the reward-regression head of SFDQN.pre_train (sfdqn_phi.py:850-862).
  *   phi [B][D] = output of the PhiFunction MLP (sfdqn_phi.py:90-123; run it with sfgpi_mlp_forward, n_actions = 1),
  *   e_b = w . phi_b - r_b ;  loss = mean_b e_b^2 (= mse_loss(reward_batch, fit_w(phis)))
