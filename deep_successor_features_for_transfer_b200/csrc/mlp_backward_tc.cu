@@ -439,8 +439,11 @@ mlp_dgrad_tc_kernel(const __grid_constant__ DgParams p, const __grid_constant__ 
 // ------------------------------------------------------------------------------------------------------------------------
 // wgrad
 // ------------------------------------------------------------------------------------------------------------------------
-constexpr int kWgThreads = 256;                     // 3 producer warps + 1 MMA warp + 4 epilogue warps
-constexpr int kWgStages = 3;
+// One TMA-issuing thread sustains ~27 B/cycle and issuers in different warps add up (DESIGN.md section 3): a 56 KB stage per
+// producer warp, four of them (224 KB of the 227 KB an SM has).
+constexpr int kWgThreads = 288;                     // 4 producer warps + 1 MMA warp + 4 epilogue warps
+constexpr int kWgStages = 4;
+constexpr int kWgMmaWarp = kWgStages;
 constexpr int kWgABytes = 2 * kBoxBytes;            // dZ tile: 64 b x 128 n
 constexpr int kWgBBytes = 4 * kBoxBytes;            // in tile: 64 b x 256 k
 constexpr int kWgXBytes = kBoxBytes;                // xo tile: 64 b x 64
@@ -454,12 +457,23 @@ struct WgParams {
     float *grad_part;                // [n_pol][n_split][row_stride]
 };
 
+// Store maps of dW_l (l >= 1) inside grad_part: fp32 {256 k, N_l rows, n_pol * n_split partial rows}, box {32, 128, 1},
+// 128B-swizzled.  A 128-row tile of dW_l is one contiguous range of a partial row; the map clips rows past N_l.
+struct WgStoreMaps { CUtensorMap w[SFGPI_MAX_LAYERS - 1]; };
+
+// developer aid (env SFGPI_TIMELINE): clock64 stamps of the policy-0, split-0 CTA of the first hidden layer's tile 0 --
+// [0] entry, [1] accumulator complete, [2] dW tile handed to the bulk stores, [3] stores complete, [4] exit
+static __device__ long long g_wg_tl[5];
+static __device__ int g_wg_tl_on = 0;
+
 __global__ void __launch_bounds__(kWgThreads, 1)
 mlp_wgrad_tc_kernel(const __grid_constant__ WgParams p, const __grid_constant__ CUtensorMap tmap_dz,
                     const __grid_constant__ CUtensorMap tmap_dzo, const __grid_constant__ CUtensorMap tmap_acts,
-                    const __grid_constant__ CUtensorMap tmap_xo) {
+                    const __grid_constant__ CUtensorMap tmap_xo, const __grid_constant__ WgStoreMaps smaps) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     pdl_launch_dependents(SFGPI_TR_WGRAD);
+    const bool tl = g_wg_tl_on && blockIdx.x == p.mt_out && blockIdx.y == 0;
+    if (tl && threadIdx.x == 0) g_wg_tl[0] = clock64();
     const sfgpi_net_desc &net = p.net;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t sbase = smem_u32(smem_raw);
@@ -486,7 +500,7 @@ mlp_wgrad_tc_kernel(const __grid_constant__ WgParams p, const __grid_constant__ 
         fence_mbar_init();
         tma_prefetch_desc(&tmap_dz); tma_prefetch_desc(&tmap_dzo); tma_prefetch_desc(&tmap_acts); tma_prefetch_desc(&tmap_xo);
     }
-    if (warp == 3) tmem_alloc(holder_addr, 512);
+    if (warp == kWgMmaWarp) tmem_alloc(holder_addr, 512);
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -517,7 +531,7 @@ mlp_wgrad_tc_kernel(const __grid_constant__ WgParams p, const __grid_constant__ 
                 tma_load_2d_e(st + kWgABytes + kWgBBytes, &tmap_xo, FULL(s), 0, b0, leader);
             }
         }
-    } else if (warp == 3) {
+    } else if (warp == kWgMmaWarp) {
         {
             const uint32_t leader = elect_one();
             const uint32_t idesc_main = umma_idesc_bf16_major(kTM, 256, 1u, 1u);
@@ -545,26 +559,36 @@ mlp_wgrad_tc_kernel(const __grid_constant__ WgParams p, const __grid_constant__ 
         const int quad = warp & 3;
         const int n_loc = quad * 32 + lane;
         const int n = mt * 128 + n_loc;
-        const int N_l = net.dims[l + 1], K_l = net.dims[l];
+        const int N_l = net.dims[l + 1];
+        const bool et0 = threadIdx.x == (kWgMmaWarp + 1) * 32;
         const uint32_t t_lane = tmem_base + ((uint32_t)(quad * 32) << 16);
         float *gp = p.grad_part + ((size_t)pl * p.n_split + split) * net.row_stride;
         mbar_wait(ACC_FULL, 0);
         tc_fence_after();
+        if (tl && et0) g_wg_tl[1] = clock64();
         const bool ok = n < N_l;
         if (main_mma) {
-            float *wrow = gp + net.w_off[l] + (size_t)n * K_l;              // K_l == 256
+            // The ring stages are free once the accumulator is complete: the fp32 tile goes there as eight 128B-swizzled
+            // {32 columns x 128 rows} boxes (conflict-free 16-byte stores: the lanes of a quarter-warp hit 8 different chunks),
+            // and one thread writes each box to grad_part with a bulk tensor store as soon as all rows have written it, so the
+            // stores run under the rest of the drain.  Per-row float4 stores to global memory at a 1 KB pitch touch 32 rows per
+            // warp instruction.
 #pragma unroll 1
-            for (int c0 = 0; c0 < kH; c0 += 32) {
+            for (int cb = 0; cb < kH / 32; ++cb) {
                 uint32_t v[32];
-                tmem_ld32(t_lane + c0, v);
+                tmem_ld32(t_lane + cb * 32, v);
                 tmem_wait_ld();
-                if (ok) {
+                const uint32_t box = sbase + (uint32_t)(cb * (kTM * 128));
 #pragma unroll
-                    for (int g = 0; g < 8; ++g)
-                        *reinterpret_cast<float4 *>(wrow + c0 + 4 * g) =
-                            make_float4(__uint_as_float(v[4 * g]), __uint_as_float(v[4 * g + 1]), __uint_as_float(v[4 * g + 2]),
-                                        __uint_as_float(v[4 * g + 3]));
-                }
+                for (int g = 0; g < 8; ++g)
+                    sts128(box + n_loc * 128 + ((g ^ (n_loc & 7)) << 4), v[4 * g], v[4 * g + 1], v[4 * g + 2], v[4 * g + 3]);
+                fence_proxy_async();
+                asm volatile("bar.sync 1, 128;" ::: "memory");
+                if (et0) tma_store_3d(&smaps.w[l - 1], box, cb * 32, mt * 128, pl * p.n_split + split);
+            }
+            if (et0) {
+                bulk_commit();
+                if (tl) g_wg_tl[2] = clock64();
             }
         }
         // aux columns: [0,S) = sum_b dZ[b][n] x[b][s] (dW_0 when l == 0), column S = sum_b dZ[b][n] (bias gradient)
@@ -583,15 +607,20 @@ mlp_wgrad_tc_kernel(const __grid_constant__ WgParams p, const __grid_constant__ 
             }
         }
         tc_fence_before();
+        if (main_mma && et0) {
+            bulk_wait0();                                               // the dW tile is written before the CTA retires
+            if (tl) g_wg_tl[3] = clock64();
+        }
     }
 
     tc_fence_before();
     __syncthreads();
-    if (warp == 3) {
+    if (warp == kWgMmaWarp) {
         __syncwarp();
         tc_fence_after();
         tmem_dealloc(tmem_base, 512);
     }
+    if (tl && threadIdx.x == 0) g_wg_tl[4] = clock64();
     trace_exit(SFGPI_TR_WGRAD);
 }
 
@@ -624,6 +653,23 @@ static int make_tmap_bf16(CUtensorMap *tm, const void *base, int rank, const uin
                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (cr != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed (%d)", (int)cr); return SFGPI_E_CUDA; }
+    tmap_cache_get(key, tm, true);
+    return SFGPI_OK;
+}
+
+// store map of one weight matrix W_l [rows][256] in every partial row of grad_part (see WgStoreMaps)
+static int make_tmap_wpart(CUtensorMap *tm, const float *base, int rows, int n_part, int row_stride) {
+    const uint64_t pitch = (uint64_t)row_stride * sizeof(float);
+    TmapKey key = {base, {(uint64_t)kH, (uint64_t)rows, (uint64_t)n_part}, {32, (uint32_t)kTM, 1}, 3, 1, 0, pitch};
+    if (tmap_cache_get(key, tm, false)) return SFGPI_OK;
+    EncodeTiledFn encode = get_encode_fn();
+    if (!encode) { set_error("cuTensorMapEncodeTiled entry point not found"); return SFGPI_E_CUDA; }
+    const cuuint64_t gdim[3] = {(cuuint64_t)kH, (cuuint64_t)rows, (cuuint64_t)n_part}, gstride[2] = {kH * sizeof(float), pitch};
+    const cuuint32_t bx[3] = {32, (cuuint32_t)kTM, 1}, estride[3] = {1, 1, 1};
+    CUresult cr = encode(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float *>(base), gdim, gstride, bx, estride,
+                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (cr != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed for grad_part (%d)", (int)cr); return SFGPI_E_CUDA; }
     tmap_cache_get(key, tm, true);
     return SFGPI_OK;
 }
@@ -769,10 +815,28 @@ extern "C" int sfgpi_mlp_backward_tc(const sfgpi_backward_tc_args *args, void *s
         if ((rc = make_tmap_bf16(&tm_acts, a.acts_bf16, 3, d3, box3))) return rc;
         if ((rc = make_tmap_bf16(&tm_xo, a.xo_bf16, 2, dx, box2))) return rc;
     }
+    WgStoreMaps smaps;
+    memset(&smaps, 0, sizeof(smaps));
+    for (int l = 1; l < L; ++l)
+        if ((rc = make_tmap_wpart(&smaps.w[l - 1], a.grad_part + net.w_off[l], net.dims[l + 1], a.n_pol * a.n_split, net.row_stride))) return rc;
     const int wg_smem = kWgStages * kWgStageBytes + 256;
     static bool cfg2 = false;
     if (!cfg2) { cudaFuncSetAttribute(mlp_wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, wg_smem); cfg2 = true; }
+    if (dg_tl) {
+        const int on = 1;
+        long long z[5] = {0};
+        cudaMemcpyToSymbol(g_wg_tl_on, &on, sizeof(on));
+        cudaMemcpyToSymbol(g_wg_tl, z, sizeof(z));
+    }
     dim3 grid(wp.items_per_policy * a.n_split, a.n_pol);
-    launch_pdl(mlp_wgrad_tc_kernel, grid, dim3(kWgThreads), wg_smem, st, wp, tm_dz, tm_dzo, tm_acts, tm_xo);
-    return check_launch("sfgpi_mlp_backward_tc(wgrad)");
+    launch_pdl(mlp_wgrad_tc_kernel, grid, dim3(kWgThreads), wg_smem, st, wp, tm_dz, tm_dzo, tm_acts, tm_xo, smaps);
+    rc = check_launch("sfgpi_mlp_backward_tc(wgrad)");
+    if (rc == SFGPI_OK && dg_tl) {                               // developer aid: one hidden-layer CTA's epilogue (cycles)
+        long long h[5];
+        cudaStreamSynchronize(st);
+        cudaMemcpyFromSymbol(h, g_wg_tl, sizeof(h));
+        fprintf(stderr, "[sfgpi wgrad timeline] grid=%dx%d; accumulator %lld, epilogue %lld (tile handed to TMA %lld), exit %lld\n",
+                grid.x, grid.y, h[1] - h[0], h[3] - h[1], h[2] - h[1], h[4] - h[0]);
+    }
+    return rc;
 }

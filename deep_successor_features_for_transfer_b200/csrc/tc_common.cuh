@@ -276,15 +276,17 @@ static inline EncodeTiledFn get_encode_fn() {
 // Host-side cache of encoded tensor maps (per translation unit).  A train step needs ~15 maps whose arguments never change from
 // one step to the next; cuTensorMapEncodeTiled costs ~0.5-1 us each and the forward's nine sit on the host's critical path
 // between the prologue launch and the forward launch (4.7 us hand-over in an isolated step, profiles/r02_forward_chain.md).
-// Key = every argument of the encode call; 64 entries, round-robin replacement.
+// Key = every argument of the encode call; 64 entries, round-robin replacement.  outer_stride: byte stride of the outermost
+// dimension when it is not the packed one (0 = packed).
 struct TmapKey {
     const void *base;
     uint64_t dims[3];
     uint32_t box[3];
     int rank, dtype, swizzle;
+    uint64_t outer_stride;
     bool operator==(const TmapKey &o) const {
         return base == o.base && rank == o.rank && dtype == o.dtype && swizzle == o.swizzle && dims[0] == o.dims[0] && dims[1] == o.dims[1] &&
-               dims[2] == o.dims[2] && box[0] == o.box[0] && box[1] == o.box[1] && box[2] == o.box[2];
+               dims[2] == o.dims[2] && box[0] == o.box[0] && box[1] == o.box[1] && box[2] == o.box[2] && outer_stride == o.outer_stride;
     }
 };
 static inline bool tmap_cache_get(const TmapKey &k, CUtensorMap *out, bool store) {
