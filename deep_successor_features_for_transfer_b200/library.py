@@ -462,45 +462,62 @@ class PackedSFLibrary:
     def _f(self, *shape):
         return torch.empty(*shape, dtype=torch.float32, device=self.device)
 
-    def _workspace(self, B, n_pol, n_keys):
-        key = (B, n_pol, n_keys)
+    def _hidden_storage(self, n_pol, B, new, precision=None):
+        """
+        Storage for hidden layers 0..L-2 of n_pol nets at batch B in mode `precision` (default: the library's) -> (values,
+        ReLU mask words).  Saved activations and dZ have these shapes in every mode.
+          fp32:          one flat fp32 buffer holding every layer's [n_pol][B][dims[l+1]] (views: _fp32_acts); masks None
+          bf16:          bf16 [L-1][n_pol][B][256]
+          tf32 / tf32x3: fp32 [parts][L-1][n_pol][B][256] (hi (, lo)), row-major, written by TMA and read back MN-major by wgrad
+        The tensor-core modes' masks are int32 [L-1][n_pol][B][8].  new: torch.empty or torch.zeros.
+        """
+        sp, L, dev = self.spec, len(self.spec.acts), self.device
+        precision = precision or self.precision
+        if precision == 'fp32':
+            return new(n_pol * B * sum(sp.dims[1:L]), dtype=torch.float32, device=dev), None
+        if precision == 'bf16':
+            values = new(L - 1, n_pol, B, 256, dtype=torch.bfloat16, device=dev)
+        else:
+            values = new(2 if precision == 'tf32x3' else 1, L - 1, n_pol, B, 256, dtype=torch.float32, device=dev)
+        return values, new(L - 1, n_pol, B, 8, dtype=torch.int32, device=dev)
+
+    def _fp32_scratch(self, n_pol, B):
+        """Scratch of the fp32 backward kernels for n_pol nets at batch B, whatever the library's mode (the G4 step runs them
+        in every mode): saved activations, dZ, the split-K count and the weight-gradient partials [n_pol][n_split][row_stride]."""
+        sp, L = self.spec, len(self.spec.acts)
+        acts, masks = self._hidden_storage(n_pol, B, torch.zeros, 'fp32')
+        tiles = sum(((sp.dims[l + 1] + 63) // 64) * ((sp.dims[l] + 255) // 256) for l in range(L))
+        n_split = max(1, min((B + 127) // 128, -(-296 // (tiles * n_pol))))
+        return dict(acts=acts, masks=masks, dz=torch.zeros_like(acts), n_split=n_split,
+                    grad_part=torch.zeros(n_pol, n_split, sp.row_stride, dtype=torch.float32, device=self.device))
+
+    def _workspace(self, B, n_pol):
+        """Scratch of the train step, psi_gradients and the psi() backward for n_pol nets at batch B: the backward's (acts,
+        masks, dz, in the tensor-core modes dzo / xo, grad_part, n_split) and the TD step's buffers."""
+        key = (B, n_pol)
         ws = self._ws.get(key)
         if ws is None:
             sp = self.spec
             L, D = len(sp.acts), sp.n_features
-            ws = dict(cur_sel=self._f(n_pol, B, D), next_sel=self._f(n_pol, B, D), d_out=self._f(n_pol, B, D),
-                      keys=torch.empty(n_keys, B, dtype=torch.int64, device=self.device))
+            if self.precision == 'fp32':
+                ws = self._fp32_scratch(n_pol, B)
+            else:
+                # tensor-core backward: row-major activations / dZ (MN-major UMMA operands), split-K over the batch in one
+                # wave of CTAs
+                acts, masks = self._hidden_storage(n_pol, B, torch.zeros)
+                lib, desc = _lib.lib(), sp.desc()
+                adp = (lib.sfgpi_f32_out_pad if self._stream else lib.sfgpi_bwd_tc_out_pad)(C.byref(desc))
+                lead = (self._parts,) if self._stream else ()
+                items = (sp.dims[-1] + 127) // 128 + 2 * (L - 1)
+                n_split = lib.sfgpi_bwd_tc_splits(B, max(1, 148 // (items * n_pol)))
+                ws = dict(acts=acts, masks=masks, dz=torch.zeros_like(acts), dzo=acts.new_zeros(*lead, n_pol, B, adp),
+                          xo=acts.new_zeros(*lead, B, 32 if self._stream else 64), n_split=n_split,
+                          grad_part=torch.zeros(n_pol, n_split, sp.row_stride, dtype=torch.float32, device=self.device))
+            ws.update(cur_sel=self._f(n_pol, B, D), next_sel=self._f(n_pol, B, D), d_out=self._f(n_pol, B, D),
+                      keys=torch.empty(n_pol, B, dtype=torch.int64, device=self.device))
             nblk = _lib.lib().sfgpi_td_partials(B)        # one TD partial per 8-CTA cluster (256 transitions)
             ws['nblk'] = nblk
             ws['loss_part'] = self._f(n_pol, nblk, 2)
-            if self._stream:
-                # tf32 modes: fp32 hi (/ lo) activations and dZ, row-major, written by TMA and read back MN-major by wgrad
-                desc = sp.desc()
-                z = lambda *shape: torch.zeros(*shape, dtype=torch.float32, device=self.device)
-                adp = _lib.lib().sfgpi_f32_out_pad(C.byref(desc))
-                P_ = self._parts
-                ws['acts32'], ws['dz32'] = z(P_, L - 1, n_pol, B, 256), z(P_, L - 1, n_pol, B, 256)
-                ws['dzo32'], ws['xo32'] = z(P_, n_pol, B, adp), z(P_, B, 32)
-                ws['masks'] = torch.zeros(L - 1, n_pol, B, 8, dtype=torch.int32, device=self.device)
-                items = (sp.dims[-1] + 127) // 128 + 2 * (L - 1)
-                n_split = _lib.lib().sfgpi_bwd_tc_splits(B, max(1, 148 // (items * n_pol)))
-            elif self.precision == 'fp32':
-                ws['acts'] = [self._f(n_pol, B, sp.dims[l + 1]) for l in range(L - 1)]
-                ws['dz'] = [self._f(n_pol, B, sp.dims[l + 1]) for l in range(L - 1)]
-                tiles = sum(((sp.dims[l + 1] + 63) // 64) * ((sp.dims[l] + 255) // 256) for l in range(L))
-                n_split = max(1, min((B + 127) // 128, -(-296 // (tiles * n_pol))))
-            else:
-                # tensor-core backward: bf16 row-major activations / dZ (MN-major UMMA operands), split-K over the batch
-                desc = sp.desc()
-                bf = lambda *shape: torch.zeros(*shape, dtype=torch.bfloat16, device=self.device)
-                adp = _lib.lib().sfgpi_bwd_tc_out_pad(C.byref(desc))
-                ws['acts16'], ws['dz16'] = bf(L - 1, n_pol, B, 256), bf(L - 1, n_pol, B, 256)
-                ws['dzo16'], ws['xo16'] = bf(n_pol, B, adp), bf(B, 64)
-                ws['masks'] = torch.zeros(L - 1, n_pol, B, 8, dtype=torch.int32, device=self.device)   # ReLU sign bits
-                items = (sp.dims[-1] + 127) // 128 + 2 * (L - 1)
-                n_split = _lib.lib().sfgpi_bwd_tc_splits(B, max(1, 148 // (items * n_pol)))      # one wave of CTAs
-            ws['n_split'] = n_split
-            ws['grad_part'] = torch.zeros(n_pol, n_split, sp.row_stride, dtype=torch.float32, device=self.device)
             if self.G is not None:
                 S = sp.dims[0]
                 ws['aux_len'] = D + self.g.shape[1] + D * self.G + D
@@ -580,20 +597,11 @@ class PackedSFLibrary:
         torch.empty: the forward kernels store every activation the backward reads (every row < B, all 256 columns of the
         tensor-core layouts, the mask words of every ReLU layer; masks of other layers are never read)."""
         sp, B = self.spec, x.shape[0]
-        L = len(sp.acts)
         out = self._f(B, n_pol, sp.n_actions, sp.n_features)
         a = self._fwd_args(self.online, lo, n_pol, x)
         a.psi_out = ptr(out)
-        masks = None
-        if self.precision == 'fp32':
-            acts = self._f(n_pol * B * sum(sp.dims[1:L]))
-            for l, t in enumerate(self._fp32_acts(acts, n_pol, B)):
-                a.acts_out[l] = t.data_ptr()
-        else:
-            shape = (self._parts, L - 1, n_pol, B, 256) if self._stream else (L - 1, n_pol, B, 256)
-            acts = torch.empty(*shape, dtype=torch.float32 if self._stream else torch.bfloat16, device=self.device)
-            masks = torch.empty(L - 1, n_pol, B, 8, dtype=torch.int32, device=self.device)
-            a.acts_bf16_out, a.relu_mask_out = acts.data_ptr(), masks.data_ptr()
+        acts, masks = self._hidden_storage(n_pol, B, torch.empty)
+        self._save_acts(a, acts, masks)
         self._forward(a, 'online')
         return out, acts, masks
 
@@ -606,38 +614,63 @@ class PackedSFLibrary:
             off += n
         return out
 
+    def _save_acts(self, a, acts, masks):
+        """Point forward args `a` at the storage (_hidden_storage) for the activations it saves: per-layer fp32 views when
+        masks is None, else the tensor-core layout and its ReLU mask words."""
+        if masks is None:
+            for l, t in enumerate(self._fp32_acts(acts, a.n_pol, a.B)):
+                a.acts_out[l] = t.data_ptr()
+        else:
+            a.acts_bf16_out, a.relu_mask_out = acts.data_ptr(), masks.data_ptr()
+
+    def _fp32_backward(self, scratch, lo, n_pol, B, acts=None):
+        """BackwardArgs of the fp32 kernels over `scratch` (_fp32_scratch) for this library's nets [lo, lo+n_pol), whatever
+        its mode; acts: saved activations outside the scratch."""
+        b = _lib.BackwardArgs()
+        b.net, b.params, b.policy_lo, b.n_pol, b.B = self.spec.desc(), ptr(self.online), lo, n_pol, B
+        acts = self._fp32_acts(scratch['acts'] if acts is None else acts, n_pol, B)
+        for l, (h, dz) in enumerate(zip(acts, self._fp32_acts(scratch['dz'], n_pol, B))):
+            b.acts[l], b.dz[l] = h.data_ptr(), dz.data_ptr()
+        b.grad_part, b.n_split = ptr(scratch['grad_part']), scratch['n_split']
+        return b
+
+    def _backward_args(self, ws, lo, n_pol, B, acts=None, masks=None):
+        """
+        The mode's backward argument block for nets [lo, lo+n_pol) at batch B over workspace `ws` -> (args, C entry point,
+        sfgpi_run op).  acts / masks: the saved activations of a forward outside the workspace (psi()), else ws's.  The caller
+        sets x, actions (NULL: d_out is a dense dL/dpsi) and d_out; the train step also xo_ready / expand_td.
+        """
+        if self.precision == 'fp32':
+            return self._fp32_backward(ws, lo, n_pol, B, acts), 'sfgpi_mlp_backward', 'BACKWARD'
+        if acts is None:
+            acts, masks = ws['acts'], ws['masks']
+        if self._stream:
+            b = _lib.BackwardStreamArgs()
+            sh_t, wo_t = self._shadow_t()
+            b.precision, b.shadow_t, b.wout_t = self._prec, ptr(sh_t), ptr(wo_t)
+            b.acts, b.dz, b.dzo, b.xo = ptr(acts), ptr(ws['dz']), ptr(ws['dzo']), ptr(ws['xo'])
+            entry, op = 'sfgpi_mlp_backward_stream', 'BACKWARD_STREAM'
+        else:
+            b = _lib.BackwardTcArgs()
+            b.params_bf16 = ptr(self._shadow_for('online'))
+            b.acts_bf16, b.dz_bf16, b.dzo_bf16, b.xo_bf16 = ptr(acts), ptr(ws['dz']), ptr(ws['dzo']), ptr(ws['xo'])
+            entry, op = 'sfgpi_mlp_backward_tc', 'BACKWARD_TC'
+        b.net, b.n_policies_total, b.relu_masks = self.spec.desc(), self.cap, ptr(masks)
+        b.policy_lo, b.n_pol, b.B = lo, n_pol, B
+        b.grad_part, b.n_split = ptr(ws['grad_part']), ws['n_split']
+        return b, entry, op
+
     def _psi_backward(self, x, lo, n_pol, acts, masks, d_psi, want_dx=False):
         """Dense-d_out backward of one psi() forward -> (gradient w.r.t. the whole online storage (rows outside zero), dL/dx
         [B][S] when want_dx, else None)."""
-        sp, B = self.spec, x.shape[0]
+        B = x.shape[0]
         d_psi = d_psi.to(torch.float32).contiguous()                 # [B][n_pol][A][D]: the psi_out layout the kernels read
-        ws = self._workspace(B, n_pol, n_pol)
-        if self._stream:
+        ws = self._workspace(B, n_pol)
+        if self.precision != 'fp32':                      # the backward's operands (tf32: transposed)
             self._pack('online', lo, n_pol, transposed=True)
-            b = _lib.BackwardStreamArgs()
-            sh_t, wo_t = self._shadow_t()
-            b.net, b.precision, b.shadow_t, b.wout_t, b.n_policies_total = sp.desc(), self._prec, ptr(sh_t), ptr(wo_t), self.cap
-            b.acts, b.dz, b.dzo, b.xo = ptr(acts), ptr(ws['dz32']), ptr(ws['dzo32']), ptr(ws['xo32'])
-            b.relu_masks = ptr(masks)
-            name = 'sfgpi_mlp_backward_stream'
-        elif self.precision != 'fp32':
-            self._pack('online', lo, n_pol)
-            b = _lib.BackwardTcArgs()
-            b.net, b.params_bf16, b.n_policies_total = sp.desc(), ptr(self._shadow_for('online')), self.cap
-            b.acts_bf16, b.dz_bf16, b.dzo_bf16, b.xo_bf16 = ptr(acts), ptr(ws['dz16']), ptr(ws['dzo16']), ptr(ws['xo16'])
-            b.relu_masks = ptr(masks)
-            name = 'sfgpi_mlp_backward_tc'
-        else:
-            b = _lib.BackwardArgs()
-            b.net, b.params = sp.desc(), ptr(self.online)
-            for l, t in enumerate(self._fp32_acts(acts, n_pol, B)):
-                b.acts[l] = t.data_ptr()
-                b.dz[l] = ws['dz'][l].data_ptr()
-            name = 'sfgpi_mlp_backward'
-        b.policy_lo, b.n_pol, b.B = lo, n_pol, B
+        b, entry, _ = self._backward_args(ws, lo, n_pol, B, acts, masks)
         b.x, b.actions, b.d_out = x.data_ptr(), None, d_psi.data_ptr()          # actions NULL: d_out is dense
-        b.grad_part, b.n_split = ptr(ws['grad_part']), ws['n_split']
-        _lib.call(name, C.byref(b), _stream())
+        _lib.call(entry, C.byref(b), _stream())
         dx = self._input_grad(ws, lo, n_pol, B) if want_dx else None     # while dZ_0 is in the workspace
         if self.online.grad is not None:
             # rows whose psi .grad a stock torch optimizer's zero_grad() set to None: start their accumulation afresh
@@ -656,10 +689,9 @@ class PackedSFLibrary:
         if g is None:                                                # built once per workspace (dropped with the storage)
             g = ws['input_grad'] = _lib.InputGradArgs()
             g.net, g.precision, g.params, g.n_pol, g.B = self.spec.desc(), self._prec, ptr(self.online), n_pol, B
+            g.dz0 = ptr(ws['dz'])                                    # layer 0 (of part 0) starts every mode's layout
             if self._stream:                                         # [parts][L-1][n_pol][B][256]: slab 0 of each part
-                g.dz0, g.dz0_part_stride = ptr(ws['dz32']), ws['dz32'][0].numel()
-            else:
-                g.dz0 = ptr(ws['dz'][0] if self.precision == 'fp32' else ws['dz16'])
+                g.dz0_part_stride = ws['dz'][0].numel()
         dx = self._f(B, self.spec.dims[0])
         g.policy_lo, g.dx = lo, dx.data_ptr()
         _lib.call('sfgpi_mlp_input_grad', C.byref(g), _stream())
@@ -756,12 +788,12 @@ class PackedSFLibrary:
     def _build_plan(self, B, policy, use_gpi, variant, beta):
         """Pre-builds every C-ABI argument block of one train step; only the six input pointers change per call."""
         sp = self.spec
-        D, A, S, L = sp.n_features, sp.n_actions, sp.dims[0], len(sp.acts)
+        D, A, S = sp.n_features, sp.n_actions, sp.dims[0]
         ensemble = policy == 'all'
         lo, n_pol = (0, self.n) if ensemble else (int(policy), 1)
         if not (0 <= lo < self.n):
             raise IndexError('policy index out of range')
-        ws = self._workspace(B, n_pol, n_pol)
+        ws = self._workspace(B, n_pol)
         keys = ws['keys']
         P = lambda tns, i=lo: C.c_void_p(tns[i].data_ptr())
 
@@ -769,13 +801,7 @@ class PackedSFLibrary:
         a1 = self._fwd_args(self.online, lo, n_pol, None, B)
         tc = self.precision != 'fp32'
         st_mode = self._stream
-        if st_mode:
-            a1.acts_bf16_out, a1.relu_mask_out = ws['acts32'].data_ptr(), ws['masks'].data_ptr()
-        elif tc:
-            a1.acts_bf16_out, a1.relu_mask_out = ws['acts16'].data_ptr(), ws['masks'].data_ptr()
-        else:
-            for l in range(L - 1):
-                a1.acts_out[l] = ws['acts'][l].data_ptr()
+        self._save_acts(a1, ws['acts'], ws['masks'])
         a1.sel_out = ptr(ws['cur_sel'])
         # (2) next actions: GPI over the whole library (or own psi) with w_i            sfdqn.py:314-322
         #     sharded: this rank scores its local policies for ALL n_total reward vectors (gathered into w_all); the
@@ -818,8 +844,7 @@ class PackedSFLibrary:
         if tc:
             # tensor-core mode: the three forwards share one launch, so the target nets cannot wait for a*; they emit the full
             # psi^-(s') [B][n_pol][A*D] and the TD kernel gathers row a* by the (all-reduced) GPI key.
-            ws['next_psi'] = ws.get('next_psi', None)
-            if ws['next_psi'] is None:
+            if 'next_psi' not in ws:
                 ws['next_psi'] = self._f(B, n_pol, A * D)
             a3.psi_out = ptr(ws['next_psi'])
         else:
@@ -838,29 +863,10 @@ class PackedSFLibrary:
         if variant == 2:
             t.tsf_part = ptr(ws['tsf_part'])
         # (5) backward through psi: dgrad chain + split-K wgrad
-        if st_mode:
-            b = _lib.BackwardStreamArgs()
-            sh_t, wo_t = self._shadow_t()
-            b.net, b.precision, b.shadow_t, b.wout_t, b.n_policies_total = sp.desc(), self._prec, ptr(sh_t), ptr(wo_t), self.cap
-            b.policy_lo, b.n_pol, b.B, b.d_out = lo, n_pol, B, ptr(ws['d_out'])
-            b.acts, b.dz, b.dzo, b.xo = (ptr(ws[k]) for k in ('acts32', 'dz32', 'dzo32', 'xo32'))
-            b.relu_masks = ptr(ws['masks'])
-        elif tc:
-            b = _lib.BackwardTcArgs()
-            b.net, b.params_bf16, b.n_policies_total = sp.desc(), ptr(self._shadow_for('online')), self.cap
-            b.policy_lo, b.n_pol, b.B, b.d_out = lo, n_pol, B, ptr(ws['d_out'])
-            b.acts_bf16, b.dz_bf16, b.dzo_bf16, b.xo_bf16 = (ptr(ws[k]) for k in ('acts16', 'dz16', 'dzo16', 'xo16'))
-            b.relu_masks = ptr(ws['masks'])
-            if variant == 2:
-                t.defer_expand, b.expand_td = 1, C.addressof(t)        # TSF expand rides in the dgrad launch (idle SMs)
-        else:
-            b = _lib.BackwardArgs()
-            b.net, b.params, b.policy_lo, b.n_pol = sp.desc(), ptr(self.online), lo, n_pol
-            b.B, b.d_out = B, ptr(ws['d_out'])
-            for l in range(L - 1):
-                b.acts[l] = ws['acts'][l].data_ptr()
-                b.dz[l] = ws['dz'][l].data_ptr()
-        b.grad_part, b.n_split = ptr(ws['grad_part']), ws['n_split']
+        b, _, b_op = self._backward_args(ws, lo, n_pol, B)
+        b.d_out = ptr(ws['d_out'])
+        if variant == 2 and b_op == 'BACKWARD_TC':
+            t.defer_expand, b.expand_td = 1, C.addressof(t)            # TSF expand rides in the dgrad launch (idle SMs)
         # (6) Adam over (psi | w | g | h) for all stepped optimizers, + loss reduction    sfdqn.py:362, tsfdqn.py:700
         ad = _lib.AdamArgs()
         ad.n_pol, ad.step = n_pol, C.c_void_p(self.step[lo:].data_ptr())
@@ -894,7 +900,7 @@ class PackedSFLibrary:
         ad.l1_scale, ad.l2_scale = 1.0 / (B * A * D), 1.0 / B
         ad.beta_loss = (float(beta) if variant == 2 else 1.0) if variant >= 1 else 0.0
         ad.sequential_shared = 1
-        return dict(ws=ws, a1=a1, a2=a2, a3=a3, t=t, b=b, ad=ad, n_pol=n_pol, lo=lo, tc=tc, st=st_mode, B=B, ring=0, keys=keys, w_all=w_all, sharded=sharded,
+        return dict(ws=ws, a1=a1, a2=a2, a3=a3, t=t, b=b, b_op=b_op, ad=ad, n_pol=n_pol, lo=lo, tc=tc, st=st_mode, B=B, ring=0, keys=keys, w_all=w_all, sharded=sharded,
                     peer=peer, variant=variant,
                     losses=torch.zeros(64, n_pol, 3, dtype=torch.float32, device=self.device))
 
@@ -987,17 +993,7 @@ class PackedSFLibrary:
                 ad.losses_host = host_losses.data_ptr()
             else:
                 d2h.op, d2h.p[0], d2h.p[1], d2h.i[0] = _lib.OP['D2H'], host_losses.data_ptr(), losses.data_ptr(), plan['n_pol'] * 12
-        # Adam bias corrections are double-buffered: this launch reads the current buffer of its optimizers and writes the next
-        # step's corrections into the other one (no finishing launch).  Optimizers stepped together must be in phase.
-        lo_, n_ = plan['lo'], plan['n_pol']
-        par = self._adam_par[lo_:lo_ + n_]
-        if len(set(par)) > 1:                                 # out of phase (single-policy and all-policy steps were mixed)
-            _lib.call('sfgpi_adam_refresh', self.step[lo_:].data_ptr(), self.adam_consts[lo_:].data_ptr(),
-                      self.adam_consts2[lo_:].data_ptr(), n_, 0.9, 0.999, _stream())
-            par = [0] * n_
-        cur, nxt = (self.adam_consts, self.adam_consts2) if par[0] == 0 else (self.adam_consts2, self.adam_consts)
-        ad.consts, ad.consts_next = cur[lo_:].data_ptr(), nxt[lo_:].data_ptr()
-        self._adam_par[lo_:lo_ + n_] = [par[0] ^ 1] * n_
+        ad.consts, ad.consts_next = self._adam_consts(plan['lo'], plan['n_pol'])
         peer = plan.get('peer')
         if peer is not None:
             # peer-memory exchange: epoch numbers (identical on every rank) pick the arena halves this step writes / pulls
@@ -1056,6 +1052,22 @@ class PackedSFLibrary:
             dist.all_reduce(delta, op=dist.ReduceOp.SUM, group=self.shard.group)
             self.h.copy_(h0 + delta)
         return losses
+
+    def _adam_consts(self, lo, n):
+        """
+        Adam bias corrections of optimizers [lo, lo+n) for one Adam launch -> (consts, consts_next) pointers.  They are double-
+        buffered: the launch reads the current buffer of its optimizers and writes the next step's corrections into the other
+        one (no finishing launch).  Optimizers stepped together must be in phase: when they are not (single-policy and
+        all-policy steps were mixed), both buffers are refreshed from the step counters first.  Flips their parity.
+        """
+        par = self._adam_par[lo:lo + n]
+        if len(set(par)) > 1:
+            _lib.call('sfgpi_adam_refresh', self.step[lo:].data_ptr(), self.adam_consts[lo:].data_ptr(),
+                      self.adam_consts2[lo:].data_ptr(), n, 0.9, 0.999, _stream())
+            par = [0] * n
+        cur, nxt = (self.adam_consts, self.adam_consts2) if par[0] == 0 else (self.adam_consts2, self.adam_consts)
+        self._adam_par[lo:lo + n] = [par[0] ^ 1] * n
+        return cur[lo:].data_ptr(), nxt[lo:].data_ptr()
 
     def _exchange(self, xc, with_h):
         """
@@ -1137,7 +1149,7 @@ class PackedSFLibrary:
             pr.fold_params, pr.fold_lo, pr.fold_n = self.online.data_ptr(), a2.policy_lo, a2.n_pol
             pr.w, pr.n_w, pr.w_diag = a2.w, a2.n_w, a2.w_diag
             pr.wq, pr.bq = plan['wq'].data_ptr(), plan['bq'].data_ptr()
-            pr.B, pr.xo_bf16 = B, ws['xo16'].data_ptr()       # pr.x = this step's states, patched per step
+            pr.B, pr.xo_bf16 = B, ws['xo'].data_ptr()         # pr.x = this step's states, patched per step
             b.xo_ready = 1
             if t.variant == 2:                                # M = Wh Wg, c once per policy here, not once per CTA of the TD kernel
                 if ws.get('tsf_mc') is None:
@@ -1185,7 +1197,7 @@ class PackedSFLibrary:
             cmd(seg1, 'NOP')
             cmd(seg2, 'FORWARD', (C.addressof(a3),))
         cmd(seg2, 'TD', (C.addressof(t),))
-        cmd(seg2, 'BACKWARD_STREAM' if st_mode else ('BACKWARD_TC' if plan['tc'] else 'BACKWARD'), (C.addressof(b),))
+        cmd(seg2, plan['b_op'], (C.addressof(b),))
         cmd(seg2, 'ADAM', (C.addressof(ad),))
         cmd(seg2, 'NOP', (0, 0), (0, 0, 0, 777))              # slot of the optional D2H read-back of the losses (host_losses)
         if peer is not None:
@@ -1256,49 +1268,21 @@ class PackedSFLibrary:
         """
         x = self._check_x(states)
         n_pol = self.n - lo if n_pol is None else n_pol
-        B, sp = x.shape[0], self.spec
-        L, D = len(sp.acts), sp.n_features
+        B, D = x.shape[0], self.spec.n_features
         actions = torch.as_tensor(actions).to(device=self.device, dtype=torch.int64).reshape(-1).contiguous()
         d_out = torch.as_tensor(d_out).to(device=self.device, dtype=torch.float32).contiguous()
         if d_out.shape != (n_pol, B, D) or actions.numel() != B:
             raise ValueError('d_out must be [n_pol, B, D] and actions [B]')
-        ws = self._workspace(B, n_pol, n_pol)
-        st = _stream()
+        ws = self._workspace(B, n_pol)
+        if self.precision != 'fp32':                      # the forward's operands and the backward's (tf32: transposed)
+            self._pack('online', lo, n_pol, transposed=True)
         a1 = self._fwd_args(self.online, lo, n_pol, x)
         a1.sel_actions, a1.sel_out = actions.data_ptr(), ptr(ws['cur_sel'])
-        if self._stream:
-            self._pack('online', lo, n_pol, transposed=True)
-            a1.acts_bf16_out, a1.relu_mask_out = ws['acts32'].data_ptr(), ws['masks'].data_ptr()
-            self._forward(a1, 'online', fresh=True)
-            b = _lib.BackwardStreamArgs()
-            sh_t, wo_t = self._shadow_t()
-            b.net, b.precision, b.shadow_t, b.wout_t, b.n_policies_total = sp.desc(), self._prec, ptr(sh_t), ptr(wo_t), self.cap
-            b.acts, b.dz, b.dzo, b.xo = (ptr(ws[k]) for k in ('acts32', 'dz32', 'dzo32', 'xo32'))
-            b.relu_masks = ptr(ws['masks'])
-            name = 'sfgpi_mlp_backward_stream'
-        elif self.precision != 'fp32':
-            self._pack('online', lo, n_pol)
-            a1.acts_bf16_out, a1.relu_mask_out = ws['acts16'].data_ptr(), ws['masks'].data_ptr()
-            self._forward(a1, 'online', fresh=True)
-            b = _lib.BackwardTcArgs()
-            b.net, b.params_bf16, b.n_policies_total = sp.desc(), ptr(self._shadow_for('online')), self.cap
-            b.acts_bf16, b.dz_bf16, b.dzo_bf16, b.xo_bf16 = (ptr(ws[k]) for k in ('acts16', 'dz16', 'dzo16', 'xo16'))
-            b.relu_masks = ptr(ws['masks'])
-            name = 'sfgpi_mlp_backward_tc'
-        else:
-            for l in range(L - 1):
-                a1.acts_out[l] = ws['acts'][l].data_ptr()
-            self._forward(a1, 'online')
-            b = _lib.BackwardArgs()
-            b.net, b.params = sp.desc(), ptr(self.online)
-            for l in range(L - 1):
-                b.acts[l] = ws['acts'][l].data_ptr()
-                b.dz[l] = ws['dz'][l].data_ptr()
-            name = 'sfgpi_mlp_backward'
-        b.policy_lo, b.n_pol, b.B = lo, n_pol, B
+        self._save_acts(a1, ws['acts'], ws['masks'])
+        self._forward(a1, 'online', fresh=True)
+        b, entry, _ = self._backward_args(ws, lo, n_pol, B)
         b.x, b.actions, b.d_out = x.data_ptr(), actions.data_ptr(), d_out.data_ptr()
-        b.grad_part, b.n_split = ptr(ws['grad_part']), ws['n_split']
-        _lib.call(name, C.byref(b), st)
+        _lib.call(entry, C.byref(b), _stream())
         return ws['grad_part'].sum(dim=1)
 
     def train_step_g4(self, transitions, policy, phi_lib, w_bias, coef, use_gpi=True):
@@ -1312,7 +1296,7 @@ class PackedSFLibrary:
         """
         states, actions, rs, _, next_states, gammas = transitions
         sp = self.spec
-        S, D, A, L = sp.dims[0], sp.n_features, sp.n_actions, len(sp.acts)
+        S, D, A = sp.dims[0], sp.n_features, sp.n_actions
         f32 = lambda t: self._as_input(t, torch.float32).to(self.device)
         states, next_states, rs, gammas = f32(states), f32(next_states), f32(rs).reshape(-1), f32(gammas).reshape(-1)
         actions = self._as_input(actions, torch.int64).to(self.device).reshape(-1)
@@ -1330,23 +1314,15 @@ class PackedSFLibrary:
         ws = self._ws.get(('g4', B))
         if ws is None:
             z = lambda *shape: torch.zeros(*shape, dtype=torch.float32, device=self.device)
-            Lp = len(psp.acts)
-
-            def bwd_ws(spec, nl):
-                tiles = sum(((spec.dims[l + 1] + 63) // 64) * ((spec.dims[l] + 255) // 256) for l in range(nl))
-                n_split = max(1, min((B + 127) // 128, -(-296 // tiles)))
-                return dict(acts=[z(1, B, spec.dims[l + 1]) for l in range(nl - 1)], dz=[z(1, B, spec.dims[l + 1]) for l in range(nl - 1)],
-                            n_split=n_split, grad=z(1, n_split, spec.row_stride))
-            ws = self._ws[('g4', B)] = dict(psi=bwd_ws(sp, L), phi=bwd_ws(psp, Lp), cur=z(1, B, D), nxt=z(1, B, D), phi_out=z(B, D),
-                                            d_psi=z(1, B, D), d_phi=z(1, B, D), small=z(D + 2), losses=z(64, 4), ring=0,
-                                            keys=torch.empty(1, B, dtype=torch.int64, device=self.device),
+            ws = self._ws[('g4', B)] = dict(psi=self._fp32_scratch(1, B), phi=phi_lib._fp32_scratch(1, B), cur=z(1, B, D),
+                                            nxt=z(1, B, D), phi_out=z(B, D), d_psi=z(1, B, D), d_phi=z(1, B, D), small=z(D + 2),
+                                            losses=z(64, 4), ring=0, keys=torch.empty(1, B, dtype=torch.int64, device=self.device),
                                             zeros=torch.zeros(B, dtype=torch.int64, device=self.device))
         # (1) phi = phi_theta(cat[s, a, s'])                                              deep_phi.py:110-111
         x_phi = torch.cat([states, actions.reshape(B, 1).to(torch.float32), next_states], dim=1).contiguous()
         ap = phi_lib._fwd_args(phi_lib.online, 0, 1, x_phi)
         ap.psi_out = ptr(ws['phi_out'])
-        for l in range(len(psp.acts) - 1):
-            ap.acts_out[l] = ws['phi']['acts'][l].data_ptr()
+        phi_lib._save_acts(ap, ws['phi']['acts'], ws['phi']['masks'])
         _lib.call('sfgpi_mlp_forward', C.byref(ap), st)
         # (2) next actions: GPI over the library under fit_w[i] (the bias shifts every q equally), or the policy's own psi  :113-123
         keys = ws['keys']
@@ -1357,8 +1333,7 @@ class PackedSFLibrary:
         _lib.call('sfgpi_mlp_forward', C.byref(a2), st)
         # (3) online psi_i(s): saves activations, gathers psi(s)[a];  (4) target psi^-_i(s')[a*]                      :130-136
         a1 = self._fwd_args(self.online, i, 1, states)
-        for l in range(L - 1):
-            a1.acts_out[l] = ws['psi']['acts'][l].data_ptr()
+        self._save_acts(a1, ws['psi']['acts'], ws['psi']['masks'])
         a1.sel_actions, a1.sel_out = actions.data_ptr(), ptr(ws['cur'])
         _lib.call('sfgpi_mlp_forward', C.byref(a1), st)
         a3 = self._fwd_args(self.target, i, 1, next_states)
@@ -1374,15 +1349,10 @@ class PackedSFLibrary:
         g.d_psi, g.d_phi, g.grad_small, g.losses = ptr(ws['d_psi']), ptr(ws['d_phi']), ptr(ws['small']), ptr(losses)
         _lib.call('sfgpi_g4_head', C.byref(g), st)
         # (6) backward through psi_i and through phi_theta
-        for lib_, spec, w_, x_, acts_, d_, pol in ((self, sp, ws['psi'], states, actions, ws['d_psi'], i),
-                                                   (phi_lib, psp, ws['phi'], x_phi, ws['zeros'], ws['d_phi'], 0)):
-            b = _lib.BackwardArgs()
-            b.net, b.params, b.policy_lo, b.n_pol, b.B = spec.desc(), ptr(lib_.online), pol, 1, B
+        for lib_, w_, x_, acts_, d_, pol in ((self, ws['psi'], states, actions, ws['d_psi'], i),
+                                             (phi_lib, ws['phi'], x_phi, ws['zeros'], ws['d_phi'], 0)):
+            b = lib_._fp32_backward(w_, pol, 1, B)
             b.x, b.actions, b.d_out = x_.data_ptr(), acts_.data_ptr(), d_.data_ptr()
-            for l in range(len(spec.acts) - 1):
-                b.acts[l] = w_['acts'][l].data_ptr()
-                b.dz[l] = w_['dz'][l].data_ptr()
-            b.grad_part, b.n_split = ptr(w_['grad']), w_['n_split']
             _lib.call('sfgpi_mlp_backward', C.byref(b), st)
         # (7) one fresh Adam over the four groups (lr 1e-3 each, :159-172), coefficient clamped (:212-215)
         ad = _lib.AdamArgs()
@@ -1396,8 +1366,8 @@ class PackedSFLibrary:
             s_.len, s_.lr, s_.weight_decay = length, 1e-3, 0.0
             if clamp is not None:
                 s_.clamp_min, s_.clamp_max = clamp
-        seg(0, self.online[i].data_ptr(), sp.row_stride, ws['psi']['grad'].data_ptr(), ws['psi']['n_split'], sp.row_stride)
-        seg(1, phi_lib.online[0].data_ptr(), psp.row_stride, ws['phi']['grad'].data_ptr(), ws['phi']['n_split'], psp.row_stride)
+        seg(0, self.online[i].data_ptr(), sp.row_stride, ws['psi']['grad_part'].data_ptr(), ws['psi']['n_split'], sp.row_stride)
+        seg(1, phi_lib.online[0].data_ptr(), psp.row_stride, ws['phi']['grad_part'].data_ptr(), ws['phi']['n_split'], psp.row_stride)
         seg(2, self.w[i].data_ptr(), D, ws['small'].data_ptr(), 1, D + 2)
         seg(3, w_bias.data_ptr(), 1, ws['small'].data_ptr() + 4 * D, 1, D + 2)
         seg(4, coef.data_ptr(), 1, ws['small'].data_ptr() + 4 * (D + 1), 1, D + 2, clamp=(1e-2, 1e6))

@@ -291,11 +291,8 @@ class PackedAdamView:
             s.len, s.lr, s.weight_decay = length, L.lr[kind], L.wd[kind]
         ad.n_seg = len(segs)
         # bias corrections: the same double-buffered pair the fused step reads and advances (library.train_step)
-        par = L._adam_par[i]
-        cur, nxt = (L.adam_consts, L.adam_consts2) if par == 0 else (L.adam_consts2, L.adam_consts)
-        ad.consts, ad.consts_next = cur[i:].data_ptr(), nxt[i:].data_ptr()
+        ad.consts, ad.consts_next = L._adam_consts(i, 1)
         _lib.call('sfgpi_adam_step', C.byref(ad), _stream())
-        L._adam_par[i] = par ^ 1
         L.weights_gen += 1
 
 

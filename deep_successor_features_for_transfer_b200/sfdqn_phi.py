@@ -18,7 +18,6 @@ import random
 import torch
 
 from . import _lib
-from ._lib import ptr
 from .library import PackedSFLibrary, _stream
 from .sfdqn import DeepSF, ReplayBuffer, _device
 
@@ -97,23 +96,17 @@ class PhiFunction:
         if plan is not None:
             return plan
         lib, sp, dev = self._library, self._library.spec, self.device
-        L, D = len(sp.acts), self.D
-        ws = lib._workspace(B, 1, 1)
+        D = self.D
+        ws = lib._workspace(B, 1)
         nblk = _lib.lib().sfgpi_phi_head_partials(B)
         f = lambda *shape: torch.zeros(*shape, dtype=torch.float32, device=dev)
         buf = dict(x=f(B, self.in_dim), r=f(B), phi=f(B, D), d_out=f(1, B, D), dw=f(nblk, D), lp=f(nblk, 2),
                    zeros=torch.zeros(B, dtype=torch.int64, device=dev), losses=f(64, 1, 3), ring=0)
         a = lib._fwd_args(lib.online, 0, 1, buf['x'])
         a.psi_out = buf['phi'].data_ptr()
-        for l in range(L - 1):
-            a.acts_out[l] = ws['acts'][l].data_ptr()
-        b = _lib.BackwardArgs()
-        b.net, b.params, b.policy_lo, b.n_pol, b.B = sp.desc(), ptr(lib.online), 0, 1, B
+        lib._save_acts(a, ws['acts'], ws['masks'])
+        b, _, _ = lib._backward_args(ws, 0, 1, B)
         b.x, b.actions, b.d_out = buf['x'].data_ptr(), buf['zeros'].data_ptr(), buf['d_out'].data_ptr()
-        for l in range(L - 1):
-            b.acts[l] = ws['acts'][l].data_ptr()
-            b.dz[l] = ws['dz'][l].data_ptr()
-        b.grad_part, b.n_split = ptr(ws['grad_part']), ws['n_split']
 
         def adam(param, m, v, length, grad, n_part, part_stride, lr, step, consts):
             ad = _lib.AdamArgs()

@@ -133,7 +133,7 @@ def main():
                 xr.grad = None
                 lib.psi(xr, 0, N).backward(d_psi)
             without, with_ = timed_pair(lambda: lib.psi(x, 0, N).backward(d_psi), with_dx, args.iters, args.reps)
-            ws = lib._workspace(B, N, N)                          # holds the last backward's dZ0
+            ws = lib._workspace(B, N)                          # holds the last backward's dZ0
             dx = lib._input_grad(ws, 0, N, B)
             assert torch.equal(dx, xr.grad)
             g = ws['input_grad']                                  # the launch _input_grad makes, without its Python around it

@@ -19,7 +19,7 @@ for precision in sys.argv[1:] or ['tf32x3']:
         d_out = torch.randn(n_pol, B, D, generator=gen) * 1e-4
         ref = tt.torch_psi_grads(o, lo, n_pol, x, actions, d_out)
         got = lib.psi_gradients(x.cuda(), actions.cuda(), d_out.cuda(), lo, n_pol).cpu()
-        ws = lib._workspace(B, n_pol, n_pol)
+        ws = lib._workspace(B, n_pol)
         errs = []
         for p in range(n_pol):
             for l, ((W, b), (gW, gb)) in enumerate(zip(lib.spec.views(got[p]), ref[p])):

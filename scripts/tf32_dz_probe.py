@@ -17,10 +17,10 @@ x, actions = tr[0], tr[1]
 lo, n_pol = 1, N - 1
 d_out = torch.randn(n_pol, B, D, generator=gen) * 1e-4
 got = lib.psi_gradients(x.cuda(), actions.cuda(), d_out.cuda(), lo, n_pol).cpu()
-ws = lib._workspace(B, n_pol, n_pol)
-acts = ws['acts32'].sum(0).cpu()      # [L-1][n_pol][B][256]
-dz = ws['dz32'].sum(0).cpu()
-dzo = ws['dzo32'].sum(0).cpu()
+ws = lib._workspace(B, n_pol)
+acts = ws['acts'].sum(0).cpu()      # [L-1][n_pol][B][256]
+dz = ws['dz'].sum(0).cpu()
+dzo = ws['dzo'].sum(0).cpu()
 for p in range(n_pol):
     layers = o.psi[lo + p]
     hs, zs = [], []

@@ -36,7 +36,7 @@ def _rel(a, b):
     (4, 9, 12, ('relu', 'relu'), 32),     # one partial tile per policy (both launches one tile per CTA)
     (4, 2, 20, ('tanh', 'tanh'), 4096),   # tanh CartPole net: the epilogue reads the saved activations
 ])
-def test_one_tile_and_paired_dgrad_agree(S, A, D, acts, B, dense):
+def test_one_tile_and_paired_backward_agree(S, A, D, acts, B, dense):
     small, large = _lib(S, A, D, acts, 4, seed=5), _lib(S, A, D, acts, 8, seed=5)
     gen = torch.Generator().manual_seed(9)
     x, actions = (v.cuda() for v in synthetic_transitions(B, S, A, D, gen)[:2])
@@ -56,9 +56,9 @@ def test_one_tile_and_paired_dgrad_agree(S, A, D, acts, B, dense):
         else:
             grads.append(lib.psi_gradients(x, actions, d8[:n_pol], 0, n_pol))
         torch.cuda.synchronize()
-        ws.append(lib._ws[(B, n_pol, n_pol)])
-    assert torch.equal(ws[0]['dzo16'], ws[1]['dzo16'][:4])
-    assert torch.equal(ws[0]['dz16'], ws[1]['dz16'][:, :4])
+        ws.append(lib._ws[(B, n_pol)])
+    assert torch.equal(ws[0]['dzo'], ws[1]['dzo'][:4])
+    assert torch.equal(ws[0]['dz'], ws[1]['dz'][:, :4])
     got, ref = grads[0][:4], grads[1][:4]
     if ws[0]['n_split'] == ws[1]['n_split']:
         assert torch.equal(got, ref)
