@@ -127,7 +127,7 @@ class Cmd(C.Structure):
 OP = dict(H2D=1, D2H=2, D2D=3, KEYS_FILL=4, PACK_BF16=5, FOLD_GPI=6, FORWARD=7, FORWARD_TC_JOBS=8, TD=9, BACKWARD=10,
           BACKWARD_TC=11, ADAM=12, EVENT=13, PEER_KEYS=14, SHARD_PACK=15, PEER_UNPACK=16, STEP_PREP=17, PACK_F32=19,
           FOLD_GPI_F32=20, FORWARD_STREAM=21, BACKWARD_STREAM=22, KEYS_DECODE=23)
-OP_LAUNCHES = {13: 0, 0: 0, 1: 0, 2: 0, 3: 0, 4: 1, 5: 1, 6: 1, 7: 1, 8: 1, 9: 1, 10: 2, 11: 3, 12: 2, 14: 1, 15: 1, 16: 1, 17: 1,
+OP_LAUNCHES = {13: 0, 0: 0, 1: 0, 2: 0, 3: 0, 4: 1, 5: 1, 6: 1, 7: 1, 8: 1, 9: 1, 10: 2, 11: 3, 12: 1, 14: 1, 15: 1, 16: 1, 17: 1,
                19: 1, 20: 1, 21: 1, 22: 3, 23: 1}
 MAX_PEERS = 16
 PEER_CHANNELS = 4
@@ -159,7 +159,7 @@ class AdamArgs(C.Structure):
     _fields_ = [('n_seg', C.c_int32), ('n_pol', C.c_int32), ('seg', AdamSegment * MAX_SEGMENTS), ('step', C.c_void_p),
                 ('beta1', C.c_double), ('beta2', C.c_double), ('eps', C.c_double), ('loss_part', C.c_void_p),
                 ('n_loss_part', C.c_int32), ('l1_scale', C.c_float), ('l2_scale', C.c_float), ('beta_loss', C.c_float),
-                ('losses', C.c_void_p), ('sequential_shared', C.c_int32), ('consts', C.c_void_p), ('consts_next', C.c_void_p),
+                ('losses', C.c_void_p), ('consts', C.c_void_p), ('consts_next', C.c_void_p),
                 ('fresh', C.c_int32), ('losses_host', C.c_void_p)]
 
 
@@ -237,7 +237,7 @@ SYMBOLS = {
 _lib = None
 launch_count = 0          # kernels launched through the C ABI (bench.py reports it as gpu_launches)
 LAUNCHES_PER_CALL = {'sfgpi_pack_bf16': 1, 'sfgpi_fold_gpi': 1, 'sfgpi_mlp_forward_tc': 1, 'sfgpi_mlp_forward': 1, 'sfgpi_keys_fill': 1, 'sfgpi_keys_decode': 1, 'sfgpi_gpi_from_psi': 1,
-                     'sfgpi_td_step': 2, 'sfgpi_mlp_backward': 2, 'sfgpi_mlp_backward_tc': 3, 'sfgpi_adam_step': 2,
+                     'sfgpi_td_step': 2, 'sfgpi_mlp_backward': 2, 'sfgpi_mlp_backward_tc': 3, 'sfgpi_adam_step': 1,
                      'sfgpi_step_prep': 1, 'sfgpi_mlp_backward_stream': 3,
     'sfgpi_peer_alloc': 0, 'sfgpi_peer_open': 0, 'sfgpi_peer_close': 0, 'sfgpi_peer_free': 0}
 

@@ -13,27 +13,25 @@ struct AdamConsts { float b2, one_m_b1, one_m_b2, eps; };
 
 __device__ __forceinline__ void adam_elem(float &p, float &m, float &v, float g, float step_size, float sqrt_bc2, float wd,
                                           const AdamConsts &k) {
+    // every multiply-add is explicit, so each inlined copy rounds alike: left to the compiler, the v update was contracted
+    // differently in the 128-bit and the scalar copy
     if (wd != 0.0f) g = fmaf(wd, p, g);
-    m = m + k.one_m_b1 * (g - m);                          // lerp_, weight < 0.5 branch
-    v = v * k.b2 + k.one_m_b2 * g * g;                     // mul_ then addcmul_
+    m = fmaf(k.one_m_b1, g - m, m);                        // lerp_, weight < 0.5 branch
+    v = fmaf(v, k.b2, __fmul_rn(__fmul_rn(k.one_m_b2, g), g));     // mul_ then addcmul_
     const float denom = __fdiv_rn(sqrtf(v), sqrt_bc2) + k.eps;
     p = p - __fdiv_rn(step_size * m, denom);               // addcdiv_(value = -step_size): self + value*t1/t2
 }
 
-// bias corrections of optimizer q for its NEXT step: {1 - beta1^t, sqrt(1 - beta2^t)} in double, as torch computes them on
-// the host.  Read from a.consts when the caller maintains it (adam_finish_kernel refreshes it after every step, so no
-// double-precision pow sits on the critical path of the step), else computed here.
+// bias corrections of optimizer q for this step: {1 - beta1^t, sqrt(1 - beta2^t)} in double, as torch computes them on the
+// host.  Read from a.consts, which the previous launch wrote (as its consts_next), so no double-precision pow sits on the
+// critical path of the step.
 __device__ __forceinline__ void bias_corrections(const sfgpi_adam_args &a, int q, double &bc1, float &sqrt_bc2) {
     if (a.fresh) {                                           // first step of a brand-new optimizer: t = 1
         bc1 = 1.0 - a.beta1;
         sqrt_bc2 = (float)sqrt(1.0 - a.beta2);
-    } else if (a.consts != nullptr) {
+    } else {
         bc1 = a.consts[2 * q];
         sqrt_bc2 = (float)a.consts[2 * q + 1];
-    } else {
-        const double t = (double)(a.step[q] + 1);
-        bc1 = 1.0 - pow(a.beta1, t);
-        sqrt_bc2 = (float)sqrt(1.0 - pow(a.beta2, t));
     }
 }
 
@@ -69,176 +67,67 @@ __device__ __forceinline__ float4 sum_partials4(const float4 *__restrict__ gp, i
                        (g0.w + g1.w) + (g2.w + g3.w));
 }
 
-// step += 1 and, when the caller keeps them, the bias corrections of the step after that
-__device__ __forceinline__ void adam_finish_one(int32_t *step, double *consts, int i, double beta1, double beta2) {
-    const int s = step[i] + 1;
-    step[i] = s;
-    if (consts != nullptr) {
-        const double t = (double)(s + 1);
-        consts[2 * i] = 1.0 - pow(beta1, t);
-        consts[2 * i + 1] = sqrt(1.0 - pow(beta2, t));
+// N consecutive floats (N = 4: one 128-bit access) <-> registers
+template <int N> __device__ __forceinline__ void load_n(float (&r)[N], const float *src) {
+    if constexpr (N == 4) {
+        const float4 t = *reinterpret_cast<const float4 *>(src);
+        r[0] = t.x; r[1] = t.y; r[2] = t.z; r[3] = t.w;
+    } else {
+        r[0] = *src;
     }
 }
-
-__global__ void __launch_bounds__(kAdamThreads) adam_kernel(const __grid_constant__ sfgpi_adam_args a, int blocks_per_pol) {
-    __shared__ float sqrt_bc2_s, step_size_s[SFGPI_MAX_SEGMENTS];
-    pdl_launch_dependents(SFGPI_TR_ADAM);
-    pdl_wait(SFGPI_TR_ADAM);
-    const int p = blockIdx.y;                               // optimizer (policy slot)
-    // ---- losses (block 0 of each optimizer): fixed-order sum of the TD kernel's per-CTA partials ----
-    if (blockIdx.x == 0 && a.loss_part != nullptr && threadIdx.x < 32) {
-        float s1 = 0.0f, s2 = 0.0f;
-        const float *lp = a.loss_part + (size_t)p * a.n_loss_part * 2;
-        for (int i = threadIdx.x; i < a.n_loss_part; i += 32) { s1 += lp[2 * i]; s2 += lp[2 * i + 1]; }
-        s1 = warp_sum(s1); s2 = warp_sum(s2);
-        if (threadIdx.x == 0) {
-            const float l1 = s1 * a.l1_scale, l2 = s2 * a.l2_scale;
-            a.losses[p * 3 + 0] = l1 + a.beta_loss * l2;
-            a.losses[p * 3 + 1] = l1;
-            a.losses[p * 3 + 2] = l2;
-            if (a.losses_host != nullptr) {                  // the step's result, straight into pinned host memory
-                a.losses_host[p * 3 + 0] = l1 + a.beta_loss * l2;
-                a.losses_host[p * 3 + 1] = l1;
-                a.losses_host[p * 3 + 2] = l2;
-            }
-        }
-    }
-    if (threadIdx.x == 0) {
-        double bc1;
-        float sb2;
-        bias_corrections(a, p, bc1, sb2);
-        sqrt_bc2_s = sb2;
-        for (int s = 0; s < a.n_seg; ++s) step_size_s[s] = (float)((double)a.seg[s].lr / bc1);
-    }
-    __syncthreads();
-    const float sqrt_bc2 = sqrt_bc2_s;
-    const AdamConsts kc = {(float)a.beta2, (float)(1.0 - a.beta1), (float)(1.0 - a.beta2), (float)a.eps};
-
-    for (int s = 0; s < a.n_seg; ++s) {
-        const sfgpi_adam_segment &sg = a.seg[s];
-        const bool shared = (sg.param_stride == 0 && a.n_pol > 1);
-        const float step_size = step_size_s[s];
-        if (!shared) {
-            const float *gp0 = sg.grad_part + (size_t)p * sg.grad_pol_stride;
-            float *pp0 = sg.param + (size_t)p * sg.param_stride;
-            float *pm0 = sg.m + (size_t)p * sg.m_stride;
-            float *pv0 = sg.v + (size_t)p * sg.v_stride;
-            const bool vec = ((sg.len | sg.grad_part_stride) & 3) == 0 &&
-                             ((reinterpret_cast<uintptr_t>(gp0) | reinterpret_cast<uintptr_t>(pp0) |
-                               reinterpret_cast<uintptr_t>(pm0) | reinterpret_cast<uintptr_t>(pv0)) & 15) == 0;
-            const bool clamp = sg.clamp_min < sg.clamp_max;
-            if (a.fresh || clamp) {                           // first-step / clamped segments (G4, target-task adaptation): scalar path
-                for (int i = blockIdx.x * kAdamThreads + threadIdx.x; i < sg.len; i += blocks_per_pol * kAdamThreads) {
-                    const float g = sum_partials(gp0 + i, sg.n_part, (size_t)sg.grad_part_stride);
-                    float pw = pp0[i], m = a.fresh ? 0.0f : pm0[i], v = a.fresh ? 0.0f : pv0[i];
-                    adam_elem(pw, m, v, g, step_size, sqrt_bc2, sg.weight_decay, kc);
-                    if (clamp) pw = fminf(fmaxf(pw, sg.clamp_min), sg.clamp_max);
-                    pp0[i] = pw;
-                    if (!a.fresh) { pm0[i] = m; pv0[i] = v; }
-                }
-            } else if (vec) {                                 // 128-bit path: 4 parameters per thread per trip
-                const int n4 = sg.len >> 2;
-                for (int i = blockIdx.x * kAdamThreads + threadIdx.x; i < n4; i += blocks_per_pol * kAdamThreads) {
-                    float4 g = sum_partials4(reinterpret_cast<const float4 *>(gp0) + i, sg.n_part, (size_t)(sg.grad_part_stride >> 2));
-                    float4 pw = reinterpret_cast<float4 *>(pp0)[i], m = reinterpret_cast<float4 *>(pm0)[i],
-                           v = reinterpret_cast<float4 *>(pv0)[i];
-                    adam_elem(pw.x, m.x, v.x, g.x, step_size, sqrt_bc2, sg.weight_decay, kc);
-                    adam_elem(pw.y, m.y, v.y, g.y, step_size, sqrt_bc2, sg.weight_decay, kc);
-                    adam_elem(pw.z, m.z, v.z, g.z, step_size, sqrt_bc2, sg.weight_decay, kc);
-                    adam_elem(pw.w, m.w, v.w, g.w, step_size, sqrt_bc2, sg.weight_decay, kc);
-                    reinterpret_cast<float4 *>(pp0)[i] = pw;
-                    reinterpret_cast<float4 *>(pm0)[i] = m;
-                    reinterpret_cast<float4 *>(pv0)[i] = v;
-                }
-            } else {
-                for (int i = blockIdx.x * kAdamThreads + threadIdx.x; i < sg.len; i += blocks_per_pol * kAdamThreads) {
-                    const float g = sum_partials(gp0 + i, sg.n_part, (size_t)sg.grad_part_stride);
-                    float pw = pp0[i], m = pm0[i], v = pv0[i];
-                    adam_elem(pw, m, v, g, step_size, sqrt_bc2, sg.weight_decay, kc);
-                    pp0[i] = pw; pm0[i] = m; pv0[i] = v;
-                }
-            }
-        } else {
-            // shared tensor (TSF's h) stepped by every optimizer from the SAME pre-step value (frozen-snapshot ensemble semantics,
-            // see DESIGN.md); each optimizer has its own moments and step.  One WARP per element, lane = optimizer: the per-optimizer
-            // work (partial sums, moments, delta) runs in parallel and the deltas are summed by a fixed butterfly.  Every block of
-            // the grid takes part.
-            const int lane = threadIdx.x & 31;
-            const int warps_total = gridDim.x * gridDim.y * (kAdamThreads / 32);
-            const int wg = (blockIdx.y * gridDim.x + blockIdx.x) * (kAdamThreads / 32) + (threadIdx.x >> 5);
-            for (int i = wg; i < sg.len; i += warps_total) {
-                const float p0 = sg.param[i];
-                float dsum = 0.0f;
-                for (int q0 = 0; q0 < a.n_pol; q0 += 32) {
-                    const int q = q0 + lane;
-                    float delta = 0.0f;
-                    if (q < a.n_pol) {
-                        double qbc1;
-                        float qsb2;
-                        bias_corrections(a, q, qbc1, qsb2);
-                        const float g = sum_partials(sg.grad_part + (size_t)q * sg.grad_pol_stride + i, sg.n_part,
-                                                     (size_t)sg.grad_part_stride);
-                        float *pm = sg.m + (size_t)q * sg.m_stride + i;
-                        float *pv = sg.v + (size_t)q * sg.v_stride + i;
-                        float pw = p0, m = *pm, v = *pv;
-                        adam_elem(pw, m, v, g, (float)((double)sg.lr / qbc1), qsb2, sg.weight_decay, kc);
-                        *pm = m; *pv = v;
-                        delta = pw - p0;
-                    }
-                    dsum += warp_sum(delta);
-                }
-                __syncwarp();
-                if (lane == 0) sg.param[i] = p0 + dsum;
-            }
-        }
-    }
-    // fused finish (consts_next given): optimizer p's first CTA advances the step counter and derives the NEXT step's bias
-    // corrections into the other buffer.  Nothing in this launch reads `step` or `consts_next`, so there is no ordering to
-    // enforce -- unlike a last-CTA tail, this adds no serial work after the update itself.
-    if (a.consts_next != nullptr && !a.fresh && blockIdx.x == 0 && threadIdx.x == 0) {
-        const int s_new = a.step[p] + 1;
-        a.step[p] = s_new;
-        const double t = (double)(s_new + 1);
-        a.consts_next[2 * p] = 1.0 - pow(a.beta1, t);
-        a.consts_next[2 * p + 1] = sqrt(1.0 - pow(a.beta2, t));
-    }
-    trace_exit(SFGPI_TR_ADAM);
+template <int N> __device__ __forceinline__ void store_n(float *dst, const float (&r)[N]) {
+    if constexpr (N == 4) *reinterpret_cast<float4 *>(dst) = make_float4(r[0], r[1], r[2], r[3]);
+    else *dst = r[0];
 }
 
-__global__ void adam_refresh_kernel(const int32_t *step, double *ca, double *cb, int n, double beta1, double beta2) {
-    pdl_launch_dependents();
-    pdl_wait();
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) {
-        const double t = (double)(step[i] + 1);
-        const double c0 = 1.0 - pow(beta1, t), c1 = sqrt(1.0 - pow(beta2, t));
-        ca[2 * i] = c0; ca[2 * i + 1] = c1;
-        cb[2 * i] = c0; cb[2 * i + 1] = c1;
+// item i of a per-optimizer segment: parameters [N*i, N*i + N) of optimizer p.  Every load (bias corrections, p, m, v,
+// partials) is issued before the first use and the step size (a double division, as on the host) is computed while they are
+// in flight.  Per element the arithmetic is the same for N = 4 and N = 1, so the kind of range does not change a bit.
+template <int N>
+__device__ __forceinline__ void adam_item(const sfgpi_adam_args &a, const sfgpi_adam_segment &sg, int p, int i, const AdamConsts &kc) {
+    double bc1;
+    float sqrt_bc2;
+    bias_corrections(a, p, bc1, sqrt_bc2);
+    const size_t e0 = (size_t)i * N;
+    const float *gp = sg.grad_part + (size_t)p * sg.grad_pol_stride + e0;
+    float *pp = sg.param + (size_t)p * sg.param_stride + e0;
+    float *pm = a.fresh ? nullptr : sg.m + (size_t)p * sg.m_stride + e0;       // fresh: moments start at 0 and are not stored
+    float *pv = a.fresh ? nullptr : sg.v + (size_t)p * sg.v_stride + e0;
+    float w[N], m[N] = {}, v[N] = {}, g[N];
+    load_n(w, pp);
+    if (!a.fresh) { load_n(m, pm); load_n(v, pv); }
+    if constexpr (N == 4) {
+        const float4 g4 = sum_partials4(reinterpret_cast<const float4 *>(gp), sg.n_part, (size_t)(sg.grad_part_stride >> 2));
+        g[0] = g4.x; g[1] = g4.y; g[2] = g4.z; g[3] = g4.w;
+    } else {
+        g[0] = sum_partials(gp, sg.n_part, (size_t)sg.grad_part_stride);
     }
+    const float step_size = (float)((double)sg.lr / bc1);
+#pragma unroll
+    for (int e = 0; e < N; ++e) adam_elem(w[e], m[e], v[e], g[e], step_size, sqrt_bc2, sg.weight_decay, kc);
+    if (sg.clamp_min < sg.clamp_max) {                       // (the G4 loss coefficient)
+#pragma unroll
+        for (int e = 0; e < N; ++e) w[e] = fminf(fmaxf(w[e], sg.clamp_min), sg.clamp_max);
+    }
+    store_n(pp, w);
+    if (!a.fresh) { store_n(pm, m); store_n(pv, v); }
 }
 
-__global__ void adam_finish_kernel(int32_t *step, double *consts, int n, double beta1, double beta2) {
-    pdl_launch_dependents();
-    pdl_wait();
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) adam_finish_one(step, consts, i, beta1, beta2);
-}
-
-// ---- flattened fast path -----------------------------------------------------------------------------------------------------
-// adam_kernel above walks the segments one after the other and starts with a one-thread prologue (bias corrections in double,
-// __syncthreads): with ~1 trip per thread that is a chain of 5-6 dependent memory round trips (prologue, psi, w, g, shared h)
-// on a kernel that moves 31 MB -- 16.5 us for 4.8 us of HBM time (profiles/r01_step_kernels_full_v2.md).  Here every segment
-// has its own block range of ONE grid, every thread owns exactly one 128-bit item and issues all of its loads (bias
-// corrections, partials, p, m, v) before the first use, and the step size (lr / (1 - beta1^t), a double division as on the
-// host) is computed by each thread while those loads are in flight.  Same arithmetic and summation order per element as
-// adam_kernel: bit-identical results.  Taken when every per-optimizer segment is 128-bit aligned and neither fresh nor clamped.
-struct AdamFlat {
+// Block layout of one launch, per grid row (= optimizer): every per-optimizer segment owns a block range, 128-bit (4
+// parameters per thread) or scalar (1 per thread) as its lengths, strides and pointers allow; then the blocks that step the
+// shared segments; then one last block.  A segment-by-segment loop behind a one-thread prologue was a chain of 5-6 dependent
+// memory round trips (17.0 -> 8.6 us, DESIGN.md).
+struct AdamGrid {
     int blk_end[SFGPI_MAX_SEGMENTS];   // exclusive prefix ends of the per-optimizer segments' block ranges (shared segments: empty)
+    int vec_mask;                      // bit s: segment s's range is 128-bit
     int n_own;                         // blocks of per-optimizer segments
     int n_shared;                      // blocks (per grid row) that step the shared segments, warp per element
 };
 
-__global__ void __launch_bounds__(kAdamThreads) adam_flat_kernel(const __grid_constant__ sfgpi_adam_args a, const __grid_constant__ AdamFlat f) {
+// At most 64 registers (4 blocks per SM): with more freedom ptxas spills more, not less, around the slow-path calls of the
+// correctly rounded divisions.
+__global__ void __launch_bounds__(kAdamThreads, 4) adam_step_kernel(const __grid_constant__ sfgpi_adam_args a, const __grid_constant__ AdamGrid f) {
     pdl_launch_dependents(SFGPI_TR_ADAM);
     pdl_wait(SFGPI_TR_ADAM);
     const int p = blockIdx.y;                               // optimizer (policy slot)
@@ -249,25 +138,15 @@ __global__ void __launch_bounds__(kAdamThreads) adam_flat_kernel(const __grid_co
         while (bid >= f.blk_end[s]) ++s;
         const sfgpi_adam_segment &sg = a.seg[s];
         const int i = (bid - (s ? f.blk_end[s - 1] : 0)) * kAdamThreads + threadIdx.x;
-        if (i < (sg.len >> 2)) {
-            const double bc1 = a.consts[2 * p];
-            const float sqrt_bc2 = (float)a.consts[2 * p + 1];
-            const float4 *gp = reinterpret_cast<const float4 *>(sg.grad_part + (size_t)p * sg.grad_pol_stride) + i;
-            float4 *pp = reinterpret_cast<float4 *>(sg.param + (size_t)p * sg.param_stride) + i;
-            float4 *pm = reinterpret_cast<float4 *>(sg.m + (size_t)p * sg.m_stride) + i;
-            float4 *pv = reinterpret_cast<float4 *>(sg.v + (size_t)p * sg.v_stride) + i;
-            float4 pw = *pp, m = *pm, v = *pv;
-            const float4 g = sum_partials4(gp, sg.n_part, (size_t)(sg.grad_part_stride >> 2));
-            const float step_size = (float)((double)sg.lr / bc1);
-            adam_elem(pw.x, m.x, v.x, g.x, step_size, sqrt_bc2, sg.weight_decay, kc);
-            adam_elem(pw.y, m.y, v.y, g.y, step_size, sqrt_bc2, sg.weight_decay, kc);
-            adam_elem(pw.z, m.z, v.z, g.z, step_size, sqrt_bc2, sg.weight_decay, kc);
-            adam_elem(pw.w, m.w, v.w, g.w, step_size, sqrt_bc2, sg.weight_decay, kc);
-            *pp = pw; *pm = m; *pv = v;
+        if ((f.vec_mask >> s) & 1) {
+            if (i < (sg.len >> 2)) adam_item<4>(a, sg, p, i, kc);
+        } else if (i < sg.len) {
+            adam_item<1>(a, sg, p, i, kc);
         }
     } else if (bid < f.n_own + f.n_shared) {
-        // shared tensors (TSF's h): every optimizer steps them from the SAME pre-step value, each with its own moments; one warp
-        // per element, lane = optimizer, deltas summed by a fixed butterfly (as in adam_kernel)
+        // shared tensors (TSF's h): every optimizer steps them from the SAME pre-step value, each with its own moments and
+        // bias corrections (frozen-snapshot ensemble semantics, DESIGN.md); one warp per element, lane = optimizer, deltas
+        // summed by a fixed butterfly
         const int lane = threadIdx.x & 31;
         const int warps_total = f.n_shared * gridDim.y * (kAdamThreads / 32);
         const int wg = (blockIdx.y * f.n_shared + (bid - f.n_own)) * (kAdamThreads / 32) + (threadIdx.x >> 5);
@@ -281,8 +160,9 @@ __global__ void __launch_bounds__(kAdamThreads) adam_flat_kernel(const __grid_co
                     const int q = q0 + lane;
                     float delta = 0.0f;
                     if (q < a.n_pol) {
-                        const double qbc1 = a.consts[2 * q];
-                        const float qsb2 = (float)a.consts[2 * q + 1];
+                        double qbc1;
+                        float qsb2;
+                        bias_corrections(a, q, qbc1, qsb2);
                         float *pm = sg.m + (size_t)q * sg.m_stride + i;
                         float *pv = sg.v + (size_t)q * sg.v_stride + i;
                         float pw = p0, m = *pm, v = *pv;
@@ -317,7 +197,7 @@ __global__ void __launch_bounds__(kAdamThreads) adam_flat_kernel(const __grid_co
                 }
             }
         }
-        if (threadIdx.x == 32) {
+        if (!a.fresh && threadIdx.x == 32) {
             const int s_new = a.step[p] + 1;
             a.step[p] = s_new;
             const double t = (double)(s_new + 1);
@@ -328,78 +208,66 @@ __global__ void __launch_bounds__(kAdamThreads) adam_flat_kernel(const __grid_co
     trace_exit(SFGPI_TR_ADAM);
 }
 
+__global__ void adam_refresh_kernel(const int32_t *step, double *ca, double *cb, int n, double beta1, double beta2) {
+    pdl_launch_dependents();
+    pdl_wait();
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) {
+        const double t = (double)(step[i] + 1);
+        const double c0 = 1.0 - pow(beta1, t), c1 = sqrt(1.0 - pow(beta2, t));
+        ca[2 * i] = c0; ca[2 * i + 1] = c1;
+        cb[2 * i] = c0; cb[2 * i + 1] = c1;
+    }
+}
+
 }  // namespace sfgpi
 
 using namespace sfgpi;
 
 extern "C" int sfgpi_adam_step(const sfgpi_adam_args *args, void *stream) {
-    trace_bind();
-    sfgpi_adam_args a_host = *args;
-    if (a_host.losses_host != nullptr) {                     // the kernel needs the device-visible address of the pinned buffer
+    sfgpi_adam_args a = *args;
+    if (a.n_seg < 1 || a.n_seg > SFGPI_MAX_SEGMENTS || a.n_pol < 1) { set_error("sfgpi_adam_step: invalid arguments"); return SFGPI_E_INVALID; }
+    if (!a.fresh) {
+        const char *missing = !a.step ? "step" : !a.consts ? "consts" : !a.consts_next ? "consts_next" : nullptr;
+        if (missing) { set_error("sfgpi_adam_step: a non-fresh step needs %s", missing); return SFGPI_E_INVALID; }
+        if (a.consts_next == a.consts) { set_error("sfgpi_adam_step: consts_next must be a buffer distinct from consts"); return SFGPI_E_INVALID; }
+    }
+    AdamGrid f = {};
+    int nb = 0, shared_len = 0;
+    for (int s = 0; s < a.n_seg; ++s) {
+        const sfgpi_adam_segment &sg = a.seg[s];
+        if (sg.len < 0 || sg.n_part < 1) { set_error("sfgpi_adam_step: bad segment %d", s); return SFGPI_E_INVALID; }
+        if (sg.param_stride == 0 && a.n_pol > 1) {
+            if (a.fresh) { set_error("sfgpi_adam_step: fresh optimizers cannot share a tensor"); return SFGPI_E_INVALID; }
+            shared_len = sg.len > shared_len ? sg.len : shared_len;
+        } else {
+            const bool vec = ((sg.len | sg.grad_part_stride | sg.grad_pol_stride | sg.param_stride | sg.m_stride | sg.v_stride) & 3) == 0 &&
+                             ((reinterpret_cast<uintptr_t>(sg.grad_part) | reinterpret_cast<uintptr_t>(sg.param) |
+                               reinterpret_cast<uintptr_t>(sg.m) | reinterpret_cast<uintptr_t>(sg.v)) & 15) == 0;
+            const int items = vec ? sg.len >> 2 : sg.len;
+            f.vec_mask |= (int)vec << s;
+            nb += items / kAdamThreads + (items % kAdamThreads != 0);
+        }
+        f.blk_end[s] = nb;
+    }
+    for (int s = a.n_seg; s < SFGPI_MAX_SEGMENTS; ++s) f.blk_end[s] = nb;
+    f.n_own = nb;
+    const int warps = (shared_len + a.n_pol - 1) / a.n_pol;                  // warps per grid row: one element each
+    f.n_shared = shared_len > 0 ? (warps + kAdamThreads / 32 - 1) / (kAdamThreads / 32) : 0;
+    if (f.n_shared > 296) f.n_shared = 296;
+    if (a.losses_host != nullptr) {                          // the kernel needs the device-visible address of the pinned buffer
         cudaPointerAttributes at;
-        if (a_host.loss_part == nullptr || cudaPointerGetAttributes(&at, a_host.losses_host) != cudaSuccess || at.type != cudaMemoryTypeHost ||
+        if (a.loss_part == nullptr || cudaPointerGetAttributes(&at, a.losses_host) != cudaSuccess || at.type != cudaMemoryTypeHost ||
             !at.devicePointer) {
             cudaGetLastError();
             set_error("sfgpi_adam_step: losses_host must be pinned host memory (and needs loss_part)");
             return SFGPI_E_INVALID;
         }
-        a_host.losses_host = reinterpret_cast<float *>(at.devicePointer);
+        a.losses_host = reinterpret_cast<float *>(at.devicePointer);
     }
-    const sfgpi_adam_args &a = a_host;
-    if (a.n_seg < 1 || a.n_seg > SFGPI_MAX_SEGMENTS || a.n_pol < 1 || (a.step == nullptr && !a.fresh)) {
-        set_error("sfgpi_adam_step: invalid arguments");
-        return SFGPI_E_INVALID;
-    }
-    if (a.consts_next != nullptr && (a.consts == nullptr || a.consts_next == a.consts)) {
-        set_error("sfgpi_adam_step: consts_next needs a distinct consts buffer to read from");
-        return SFGPI_E_INVALID;
-    }
-    int max_len = 0;
-    for (int s = 0; s < a.n_seg; ++s) {
-        if (a.fresh && a.seg[s].param_stride == 0 && a.n_pol > 1) { set_error("sfgpi_adam_step: fresh optimizers cannot share a tensor"); return SFGPI_E_INVALID; }
-        if (a.seg[s].len < 0 || a.seg[s].n_part < 1) { set_error("sfgpi_adam_step: bad segment %d", s); return SFGPI_E_INVALID; }
-        max_len = a.seg[s].len > max_len ? a.seg[s].len : max_len;
-    }
-    cudaStream_t st = (cudaStream_t)stream;
-    // flattened fast path (see adam_flat_kernel): the train steps' shape -- double-buffered corrections, 128-bit aligned segments
-    if (!a.fresh && a.consts != nullptr && a.consts_next != nullptr) {
-        AdamFlat f;
-        bool ok = true;
-        int nb = 0, shared_len = 0;
-        for (int s = 0; s < SFGPI_MAX_SEGMENTS; ++s) {
-            if (s < a.n_seg) {
-                const sfgpi_adam_segment &sg = a.seg[s];
-                const bool shared = sg.param_stride == 0 && a.n_pol > 1;
-                if (shared) shared_len = sg.len > shared_len ? sg.len : shared_len;
-                else {
-                    const bool vec = ((sg.len | sg.grad_part_stride | sg.grad_pol_stride | sg.param_stride | sg.m_stride | sg.v_stride) & 3) == 0 &&
-                                     ((reinterpret_cast<uintptr_t>(sg.grad_part) | reinterpret_cast<uintptr_t>(sg.param) |
-                                       reinterpret_cast<uintptr_t>(sg.m) | reinterpret_cast<uintptr_t>(sg.v)) & 15) == 0;
-                    if (!vec || sg.clamp_min < sg.clamp_max) { ok = false; break; }
-                    nb += ((sg.len >> 2) + kAdamThreads - 1) / kAdamThreads;
-                }
-            }
-            f.blk_end[s] = nb;
-        }
-        if (ok) {
-            f.n_own = nb;
-            const int warps = (shared_len + a.n_pol - 1) / a.n_pol;                  // warps per grid row: one element each
-            f.n_shared = shared_len > 0 ? (warps + kAdamThreads / 32 - 1) / (kAdamThreads / 32) : 0;
-            if (f.n_shared > 296) f.n_shared = 296;
-            launch_pdl(adam_flat_kernel, dim3(f.n_own + f.n_shared + 1, a.n_pol), dim3(kAdamThreads), 0, st, a, f);
-            return check_launch("sfgpi_adam_step(flat)");
-        }
-    }
-    int blocks = (max_len + kAdamThreads - 1) / kAdamThreads;
-    if (blocks < 1) blocks = 1;
-    const int cap = (148 * 8 + a.n_pol - 1) / a.n_pol;                 // ~8 CTAs per SM over the whole launch
-    if (blocks > cap) blocks = cap < 1 ? 1 : cap;
-    dim3 grid(blocks, a.n_pol);
-    launch_pdl(adam_kernel, grid, dim3(kAdamThreads), 0, st, a, blocks);
-    int rc = check_launch("sfgpi_adam_step");
-    if (rc || a.consts_next != nullptr || a.fresh) return rc;
-    launch_pdl(adam_finish_kernel, dim3((a.n_pol + 127) / 128), dim3(128), 0, st, a.step, a.consts, a.n_pol, a.beta1, a.beta2);
-    return check_launch("sfgpi_adam_step(finish)");
+    trace_bind();
+    launch_pdl(adam_step_kernel, dim3(f.n_own + f.n_shared + 1, a.n_pol), dim3(kAdamThreads), 0, (cudaStream_t)stream, a, f);
+    return check_launch("sfgpi_adam_step");
 }
 
 extern "C" int sfgpi_adam_refresh(const int32_t *step, double *consts_a, double *consts_b, int32_t n, double beta1, double beta2, void *stream) {

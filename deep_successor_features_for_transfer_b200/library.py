@@ -17,6 +17,7 @@ working.  No torch op is on the compute path; torch only owns the memory and the
 """
 import ctypes as C
 import math
+from typing import NamedTuple
 
 import numpy as np
 import torch
@@ -116,6 +117,79 @@ def _stream():
     if _raw_stream is not None:
         return C.c_void_p(_raw_stream(torch.cuda.current_device()))
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
+
+
+# ---- Adam (sfgpi_adam_step): torch.optim.Adam's betas and eps, which every optimizer of the reference uses
+ADAM_BETA1, ADAM_BETA2, ADAM_EPS = 0.9, 0.999, 1e-8
+
+
+class AdamSeg(NamedTuple):
+    """
+    One segment of an Adam launch: `len` parameters at device address `param`, their moments `m` / `v` (None in a fresh launch)
+    and the gradient, the sum of n_part partials at `grad`, grad_part_stride floats apart.  The per-policy strides select
+    optimizer p's slice; param_stride 0 in a launch of several optimizers is a tensor they share (TSF's h).  clamp = (min, max)
+    clamps the stepped parameter.
+    """
+    param: object
+    m: object
+    v: object
+    grad: object
+    len: int
+    lr: float
+    wd: float = 0.0
+    param_stride: int = 0
+    mv_stride: int = 0
+    grad_pol_stride: int = 0
+    grad_part_stride: int = 0
+    n_part: int = 1
+    clamp: tuple = None
+
+
+def adam_args(segments, n_pol=1, step=None, consts=(None, None)):
+    """
+    sfgpi_adam_args of one launch over `segments` (AdamSeg) for optimizers 0..n_pol-1.  step: device address of their int32
+    step counters, with consts = their (current, next) bias-correction buffers from adam_consts_pair (a block that is kept and
+    launched again gets fresh ones before every launch).  step None: a fresh launch, the first step of brand-new optimizers.
+    """
+    ad = _lib.AdamArgs()
+    ad.n_seg, ad.n_pol = len(segments), n_pol
+    ad.beta1, ad.beta2, ad.eps = ADAM_BETA1, ADAM_BETA2, ADAM_EPS
+    if step is None:
+        ad.fresh = 1
+    else:
+        ad.step = step
+        ad.consts, ad.consts_next = consts
+    for k, sg in enumerate(segments):
+        s = ad.seg[k]
+        s.param, s.param_stride, s.m, s.v, s.m_stride, s.v_stride = sg.param, sg.param_stride, sg.m, sg.v, sg.mv_stride, sg.mv_stride
+        s.grad_part, s.grad_pol_stride, s.grad_part_stride, s.n_part = sg.grad, sg.grad_pol_stride, sg.grad_part_stride, sg.n_part
+        s.len, s.lr, s.weight_decay = sg.len, sg.lr, sg.wd
+        if sg.clamp is not None:
+            s.clamp_min, s.clamp_max = sg.clamp
+    return ad
+
+
+def adam_consts_init(n, device):
+    """Bias corrections {1 - beta1^t, sqrt(1 - beta2^t)} of n optimizers' first step (t = 1): [n][2] float64, as torch's host math."""
+    return torch.tensor([[1.0 - ADAM_BETA1, math.sqrt(1.0 - ADAM_BETA2)]], dtype=torch.float64, device=device).repeat(n, 1).contiguous()
+
+
+def adam_consts_pair(step, consts, par, lo, n):
+    """
+    Bias corrections of optimizers [lo, lo+n) for one Adam launch -> (consts, consts_next) pointers.  They are double-buffered:
+    consts holds two adam_consts_init buffers and par[i] says which one is current for optimizer i.  The launch reads the current
+    buffer and writes the next step's corrections into the other one (no finishing launch).  Optimizers stepped together must be
+    in phase: when they are not (single-policy and all-policy steps were mixed), both buffers are refreshed from the step
+    counters first.  Flips their parity.
+    """
+    p = par[lo:lo + n]
+    if len(set(p)) > 1:
+        _lib.call('sfgpi_adam_refresh', step[lo:].data_ptr(), consts[0][lo:].data_ptr(), consts[1][lo:].data_ptr(), n,
+                  ADAM_BETA1, ADAM_BETA2, _stream())
+        p = [0] * n
+    cur, nxt = consts if p[0] == 0 else consts[::-1]
+    par[lo:lo + n] = [p[0] ^ 1] * n
+    return cur[lo:].data_ptr(), nxt[lo:].data_ptr()
 
 
 class _PsiFunction(torch.autograd.Function):
@@ -320,12 +394,10 @@ class PackedSFLibrary:
                    v=z(cap, sp.row_stride), w=z(cap, sp.n_features), w_m=z(cap, sp.n_features), w_v=z(cap, sp.n_features),
                    step=torch.zeros(cap, dtype=torch.int32, device=dev),
                    # Adam bias corrections of every optimizer's NEXT step (t = step + 1), double like torch's host math
-                   adam_consts=torch.tensor([[1.0 - 0.9 ** 1, math.sqrt(1.0 - 0.999 ** 1)]], dtype=torch.float64,
-                                            device=dev).repeat(cap, 1).contiguous(),
-                   # ... and its twin: the train step's Adam launch reads one buffer and writes the next step's corrections
-                   # into the other (sfgpi_adam_args.consts_next); _adam_par[i] says which buffer is current for policy i
-                   adam_consts2=torch.tensor([[1.0 - 0.9 ** 1, math.sqrt(1.0 - 0.999 ** 1)]], dtype=torch.float64,
-                                             device=dev).repeat(cap, 1).contiguous())
+                   adam_consts=adam_consts_init(cap, dev),
+                   # ... and its twin: an Adam launch reads one buffer and writes the next step's corrections into the
+                   # other (sfgpi_adam_args.consts_next); _adam_par[i] says which buffer is current for policy i
+                   adam_consts2=adam_consts_init(cap, dev))
         if self.G is not None:
             gl = self.G * sp.dims[0] + self.G + self.n_flows * (2 * sp.dims[0] + 1)      # W | b | K x (weight | bias | scale)
             hl = sp.n_features * self.G + sp.n_features
@@ -868,38 +940,25 @@ class PackedSFLibrary:
         if variant == 2 and b_op == 'BACKWARD_TC':
             t.defer_expand, b.expand_td = 1, C.addressof(t)            # TSF expand rides in the dgrad launch (idle SMs)
         # (6) Adam over (psi | w | g | h) for all stepped optimizers, + loss reduction    sfdqn.py:362, tsfdqn.py:700
-        ad = _lib.AdamArgs()
-        ad.n_pol, ad.step = n_pol, C.c_void_p(self.step[lo:].data_ptr())
-        ad.consts = C.c_void_p(self.adam_consts[lo:].data_ptr())          # (consts / consts_next: patched per step, see train_step)
-        ad.beta1, ad.beta2, ad.eps = 0.9, 0.999, 1e-8
         rs_, nblk, al = sp.row_stride, ws['nblk'], ws['aux_len']
         npa = 1 if variant == 2 else nblk          # variant 2: the TD step leaves ONE reduced aux-gradient row per policy
-
-        def seg(k, param, pstride, m, v, mstride, grad, gpol, gpart, npart, length, lr, wd):
-            s = ad.seg[k]
-            s.param, s.param_stride, s.m, s.m_stride, s.v, s.v_stride = param, pstride, m, mstride, v, mstride
-            s.grad_part, s.grad_pol_stride, s.grad_part_stride, s.n_part = grad, gpol, gpart, npart
-            s.len, s.lr, s.weight_decay = length, lr, wd
-
-        seg(0, P(self.online), rs_, P(self.m), P(self.v), rs_, ptr(ws['grad_part']), ws['n_split'] * rs_, rs_, ws['n_split'],
-            rs_, self.lr['sf'], self.wd['sf'])
-        nseg = 1
-        aux = ws['aux_part']
+        aux, aux_parts = ws['aux_part'].data_ptr(), dict(grad_pol_stride=nblk * al, grad_part_stride=al, n_part=npa)
+        segs = [AdamSeg(P(self.online), P(self.m), P(self.v), ptr(ws['grad_part']), rs_, self.lr['sf'], self.wd['sf'],
+                        param_stride=rs_, mv_stride=rs_, grad_pol_stride=ws['n_split'] * rs_, grad_part_stride=rs_,
+                        n_part=ws['n_split'])]
         if variant >= 1:
-            seg(1, P(self.w), D, P(self.w_m), P(self.w_v), D, ptr(aux), nblk * al, al, npa, D, self.lr['w'], self.wd['w'])
-            nseg = 2
+            segs.append(AdamSeg(P(self.w), P(self.w_m), P(self.w_v), aux, D, self.lr['w'], self.wd['w'], param_stride=D,
+                                mv_stride=D, **aux_parts))
         if variant == 2:
             gl, hl = self.g.shape[1], self.h.numel()
-            seg(2, P(self.g), gl, P(self.g_m), P(self.g_v), gl, C.c_void_p(aux.data_ptr() + 4 * D), nblk * al, al, npa, gl,
-                self.lr['g'], self.wd['g'])
-            seg(3, ptr(self.h), 0, P(self.h_m), P(self.h_v), hl, C.c_void_p(aux.data_ptr() + 4 * (D + gl)), nblk * al, al, npa,
-                hl, self.lr['h'], self.wd['h'])
-            nseg = 4
-        ad.n_seg = nseg
+            segs.append(AdamSeg(P(self.g), P(self.g_m), P(self.g_v), aux + 4 * D, gl, self.lr['g'], self.wd['g'], param_stride=gl,
+                                mv_stride=gl, **aux_parts))
+            segs.append(AdamSeg(ptr(self.h), P(self.h_m), P(self.h_v), aux + 4 * (D + gl), hl, self.lr['h'], self.wd['h'],
+                                mv_stride=hl, **aux_parts))
+        ad = adam_args(segs, n_pol, C.c_void_p(self.step[lo:].data_ptr()))       # (consts: set per step, see train_step)
         ad.loss_part, ad.n_loss_part = ptr(ws['loss_part']), nblk
         ad.l1_scale, ad.l2_scale = 1.0 / (B * A * D), 1.0 / B
         ad.beta_loss = (float(beta) if variant == 2 else 1.0) if variant >= 1 else 0.0
-        ad.sequential_shared = 1
         return dict(ws=ws, a1=a1, a2=a2, a3=a3, t=t, b=b, b_op=b_op, ad=ad, n_pol=n_pol, lo=lo, tc=tc, st=st_mode, B=B, ring=0, keys=keys, w_all=w_all, sharded=sharded,
                     peer=peer, variant=variant,
                     losses=torch.zeros(64, n_pol, 3, dtype=torch.float32, device=self.device))
@@ -1054,20 +1113,8 @@ class PackedSFLibrary:
         return losses
 
     def _adam_consts(self, lo, n):
-        """
-        Adam bias corrections of optimizers [lo, lo+n) for one Adam launch -> (consts, consts_next) pointers.  They are double-
-        buffered: the launch reads the current buffer of its optimizers and writes the next step's corrections into the other
-        one (no finishing launch).  Optimizers stepped together must be in phase: when they are not (single-policy and
-        all-policy steps were mixed), both buffers are refreshed from the step counters first.  Flips their parity.
-        """
-        par = self._adam_par[lo:lo + n]
-        if len(set(par)) > 1:
-            _lib.call('sfgpi_adam_refresh', self.step[lo:].data_ptr(), self.adam_consts[lo:].data_ptr(),
-                      self.adam_consts2[lo:].data_ptr(), n, 0.9, 0.999, _stream())
-            par = [0] * n
-        cur, nxt = (self.adam_consts, self.adam_consts2) if par[0] == 0 else (self.adam_consts2, self.adam_consts)
-        self._adam_par[lo:lo + n] = [par[0] ^ 1] * n
-        return cur[lo:].data_ptr(), nxt[lo:].data_ptr()
+        """(consts, consts_next) of optimizers [lo, lo+n) for one Adam launch (adam_consts_pair)."""
+        return adam_consts_pair(self.step, (self.adam_consts, self.adam_consts2), self._adam_par, lo, n)
 
     def _exchange(self, xc, with_h):
         """
@@ -1232,7 +1279,7 @@ class PackedSFLibrary:
                     arr[k].p[q] = v
                 for q, v in enumerate(i):
                     arr[k].i[q] = int(v)
-                launches += _lib.OP_LAUNCHES[arr[k].op] - (1 if op == 'BACKWARD_TC' and b.xo_ready else 0) - (1 if op == 'ADAM' else 0) \
+                launches += _lib.OP_LAUNCHES[arr[k].op] - (1 if op == 'BACKWARD_TC' and b.xo_ready else 0) \
                     + (1 if op == 'TD' and t.variant == 2 and not t.defer_expand else 0) \
                     + (_lib.lib().sfgpi_step_prep_launches(C.addressof(plan['prep'])) - 1 if op == 'STEP_PREP' else 0)
             if plan['h2d'] is None:
@@ -1355,23 +1402,14 @@ class PackedSFLibrary:
             b.x, b.actions, b.d_out = x_.data_ptr(), acts_.data_ptr(), d_.data_ptr()
             _lib.call('sfgpi_mlp_backward', C.byref(b), st)
         # (7) one fresh Adam over the four groups (lr 1e-3 each, :159-172), coefficient clamped (:212-215)
-        ad = _lib.AdamArgs()
-        ad.n_pol, ad.fresh, ad.sequential_shared = 1, 1, 1
-        ad.beta1, ad.beta2, ad.eps = 0.9, 0.999, 1e-8
-
-        def seg(k, param, length, grad, n_part, part_stride, clamp=None):
-            s_ = ad.seg[k]
-            s_.param, s_.param_stride, s_.m_stride, s_.v_stride = param, length, length, length
-            s_.grad_part, s_.grad_pol_stride, s_.grad_part_stride, s_.n_part = grad, n_part * part_stride, part_stride, n_part
-            s_.len, s_.lr, s_.weight_decay = length, 1e-3, 0.0
-            if clamp is not None:
-                s_.clamp_min, s_.clamp_max = clamp
-        seg(0, self.online[i].data_ptr(), sp.row_stride, ws['psi']['grad_part'].data_ptr(), ws['psi']['n_split'], sp.row_stride)
-        seg(1, phi_lib.online[0].data_ptr(), psp.row_stride, ws['phi']['grad_part'].data_ptr(), ws['phi']['n_split'], psp.row_stride)
-        seg(2, self.w[i].data_ptr(), D, ws['small'].data_ptr(), 1, D + 2)
-        seg(3, w_bias.data_ptr(), 1, ws['small'].data_ptr() + 4 * D, 1, D + 2)
-        seg(4, coef.data_ptr(), 1, ws['small'].data_ptr() + 4 * (D + 1), 1, D + 2, clamp=(1e-2, 1e6))
-        ad.n_seg = 5
+        small = ws['small'].data_ptr()
+        ad = adam_args([AdamSeg(self.online[i].data_ptr(), None, None, ws['psi']['grad_part'].data_ptr(), sp.row_stride, 1e-3,
+                                grad_part_stride=sp.row_stride, n_part=ws['psi']['n_split']),
+                        AdamSeg(phi_lib.online[0].data_ptr(), None, None, ws['phi']['grad_part'].data_ptr(), psp.row_stride, 1e-3,
+                                grad_part_stride=psp.row_stride, n_part=ws['phi']['n_split']),
+                        AdamSeg(self.w[i].data_ptr(), None, None, small, D, 1e-3),
+                        AdamSeg(w_bias.data_ptr(), None, None, small + 4 * D, 1, 1e-3),
+                        AdamSeg(coef.data_ptr(), None, None, small + 4 * (D + 1), 1, 1e-3, clamp=(1e-2, 1e6))])
         _lib.call('sfgpi_adam_step', C.byref(ad), st)
         return losses
 

@@ -245,7 +245,7 @@ class PackedAdamView:
     def _launch(self, have):
         import ctypes as C
         from . import _lib
-        from .library import _stream
+        from .library import AdamSeg, _stream, adam_args
         L, i = self._library, self.index
         sp = L.spec
         keep = []                                    # tensors that must outlive the launch call
@@ -257,41 +257,32 @@ class PackedAdamView:
             keep.append(g)
             return g.data_ptr()
 
-        ad = _lib.AdamArgs()
-        ad.n_pol, ad.step = 1, L.step[i:].data_ptr()
-        ad.beta1, ad.beta2, ad.eps = 0.9, 0.999, 1e-8
-        ad.sequential_shared = 1
         segs = []
         if have['sf']:
-            rs = sp.row_stride
             row = L.online.grad[i]
             for (W, b), lin in zip(sp.views(row), L._views[i]['online']):      # .grad rebound by the user: copy it back
                 for view, p in ((W, lin.weight), (b, lin.bias)):
                     if p.grad.data_ptr() != view.data_ptr():
                         view.copy_(p.grad)
-            segs.append((L.online.detach()[i].data_ptr(), 0, L.m[i].data_ptr(), L.v[i].data_ptr(), row.data_ptr(), rs, 'sf'))
+            segs.append(AdamSeg(L.online.detach()[i].data_ptr(), L.m[i].data_ptr(), L.v[i].data_ptr(), row.data_ptr(), sp.row_stride,
+                                L.lr['sf'], L.wd['sf']))
         if have['w']:
-            segs.append((L.w[i].data_ptr(), 0, L.w_m[i].data_ptr(), L.w_v[i].data_ptr(), grad_of(self._groups[1][1][0]), sp.n_features, 'w'))
+            segs.append(AdamSeg(L.w[i].data_ptr(), L.w_m[i].data_ptr(), L.w_v[i].data_ptr(), grad_of(self._groups[1][1][0]),
+                                sp.n_features, L.lr['w'], L.wd['w']))
         if L.G is not None:
             S, G, D = sp.dims[0], L.G, sp.n_features
             if have['g']:
                 gW, gb = self._groups[2][1]
-                segs.append((L.g[i].data_ptr(), 0, L.g_m[i].data_ptr(), L.g_v[i].data_ptr(), grad_of(gW), G * S, 'g'))
-                o = 4 * G * S
-                segs.append((L.g[i].data_ptr() + o, 0, L.g_m[i].data_ptr() + o, L.g_v[i].data_ptr() + o, grad_of(gb), G, 'g'))
+                p, m, v, o = L.g[i].data_ptr(), L.g_m[i].data_ptr(), L.g_v[i].data_ptr(), 4 * G * S
+                segs.append(AdamSeg(p, m, v, grad_of(gW), G * S, L.lr['g'], L.wd['g']))
+                segs.append(AdamSeg(p + o, m + o, v + o, grad_of(gb), G, L.lr['g'], L.wd['g']))
             if have['h']:
                 hW, hb = self._groups[3][1]
-                segs.append((L.h.data_ptr(), 0, L.h_m[i].data_ptr(), L.h_v[i].data_ptr(), grad_of(hW), D * G, 'h'))
-                o = 4 * D * G
-                segs.append((L.h.data_ptr() + o, 0, L.h_m[i].data_ptr() + o, L.h_v[i].data_ptr() + o, grad_of(hb), D, 'h'))
-        for k, (param, pstride, m, v, grad, length, kind) in enumerate(segs):
-            s = ad.seg[k]
-            s.param, s.param_stride, s.m, s.m_stride, s.v, s.v_stride = param, pstride, m, 0, v, 0
-            s.grad_part, s.grad_pol_stride, s.grad_part_stride, s.n_part = grad, 0, length, 1
-            s.len, s.lr, s.weight_decay = length, L.lr[kind], L.wd[kind]
-        ad.n_seg = len(segs)
+                p, m, v, o = L.h.data_ptr(), L.h_m[i].data_ptr(), L.h_v[i].data_ptr(), 4 * D * G
+                segs.append(AdamSeg(p, m, v, grad_of(hW), D * G, L.lr['h'], L.wd['h']))
+                segs.append(AdamSeg(p + o, m + o, v + o, grad_of(hb), D, L.lr['h'], L.wd['h']))
         # bias corrections: the same double-buffered pair the fused step reads and advances (library.train_step)
-        ad.consts, ad.consts_next = L._adam_consts(i, 1)
+        ad = adam_args(segs, 1, L.step[i:].data_ptr(), L._adam_consts(i, 1))
         _lib.call('sfgpi_adam_step', C.byref(ad), _stream())
         L.weights_gen += 1
 

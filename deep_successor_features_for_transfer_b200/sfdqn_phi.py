@@ -12,13 +12,12 @@ the layer widths are not the 256-wide tensor-core shape, and at B = 32 the step 
 The replay ring, the random-policy rollout and the task protocol stay host-side Python, as in the reference.
 """
 import ctypes as C
-import math
 import random
 
 import torch
 
 from . import _lib
-from .library import PackedSFLibrary, _stream
+from .library import AdamSeg, PackedSFLibrary, _stream, adam_args, adam_consts_init, adam_consts_pair
 from .sfdqn import DeepSF, ReplayBuffer, _device
 
 
@@ -35,7 +34,11 @@ class _RewardHead:
         lin.weight.data = self.weight.view(1, -1)
         self.m, self.v = torch.zeros_like(self.weight), torch.zeros_like(self.weight)
         self.step = torch.zeros(1, dtype=torch.int32, device=device)
-        self.consts = torch.tensor([[1.0 - 0.9 ** 1, math.sqrt(1.0 - 0.999 ** 1)]], dtype=torch.float64, device=device)
+        self._consts, self._consts_par = (adam_consts_init(1, device), adam_consts_init(1, device)), [0]
+
+    def adam_consts(self):
+        """(consts, consts_next) for the next step of the head's Adam (adam_consts_pair)."""
+        return adam_consts_pair(self.step, self._consts, self._consts_par, 0, 1)
 
 
 class PhiFunction:
@@ -107,22 +110,10 @@ class PhiFunction:
         lib._save_acts(a, ws['acts'], ws['masks'])
         b, _, _ = lib._backward_args(ws, 0, 1, B)
         b.x, b.actions, b.d_out = buf['x'].data_ptr(), buf['zeros'].data_ptr(), buf['d_out'].data_ptr()
-
-        def adam(param, m, v, length, grad, n_part, part_stride, lr, step, consts):
-            ad = _lib.AdamArgs()
-            ad.n_seg, ad.n_pol, ad.step, ad.consts = 1, 1, step.data_ptr(), consts.data_ptr()
-            ad.beta1, ad.beta2, ad.eps = 0.9, 0.999, 1e-8
-            s = ad.seg[0]
-            s.param, s.m, s.v, s.param_stride, s.m_stride, s.v_stride = param, m, v, length, length, length
-            s.grad_part, s.grad_pol_stride, s.grad_part_stride, s.n_part = grad, n_part * part_stride, part_stride, n_part
-            s.len, s.lr, s.weight_decay = length, lr, 0.0
-            ad.sequential_shared = 1
-            return ad
-
         rs = sp.row_stride
-        ad_phi = adam(lib.online.data_ptr(), lib.m.data_ptr(), lib.v.data_ptr(), rs, ws['grad_part'].data_ptr(), ws['n_split'], rs,
-                      self.alpha_phi, lib.step, lib.adam_consts)
-        plan = self._plans[B] = dict(buf=buf, a=a, b=b, ad_phi=ad_phi, nblk=nblk, B=B, ws=ws, adam=adam)
+        ad_phi = adam_args([AdamSeg(lib.online.data_ptr(), lib.m.data_ptr(), lib.v.data_ptr(), ws['grad_part'].data_ptr(), rs,
+                                    self.alpha_phi, grad_part_stride=rs, n_part=ws['n_split'])], 1, lib.step.data_ptr())
+        plan = self._plans[B] = dict(buf=buf, a=a, b=b, ad_phi=ad_phi, nblk=nblk, B=B, ws=ws)
         return plan
 
     def regression_step(self, state, action, reward, next_state, head, loss_slot=None):
@@ -145,14 +136,16 @@ class PhiFunction:
         _lib.call('sfgpi_phi_head', buf['phi'].data_ptr(), head.weight.data_ptr(), buf['r'].data_ptr(), B, D, buf['d_out'].data_ptr(),
                   buf['dw'].data_ptr(), buf['lp'].data_ptr(), st)
         _lib.call('sfgpi_mlp_backward', C.byref(plan['b']), st)
-        _lib.call('sfgpi_adam_step', C.byref(plan['ad_phi']), st)
+        ad_phi = plan['ad_phi']
+        ad_phi.consts, ad_phi.consts_next = self._library._adam_consts(0, 1)              # (phi_theta's optimizer: row 0)
+        _lib.call('sfgpi_adam_step', C.byref(ad_phi), st)
         if loss_slot is None:
             buf['ring'] = (buf['ring'] + 1) % 64
             losses = buf['losses'][buf['ring']]
         else:
             losses = loss_slot
-        ad_w = plan['adam'](head.weight.data_ptr(), head.m.data_ptr(), head.v.data_ptr(), D, buf['dw'].data_ptr(), plan['nblk'], D,
-                            head.lr, head.step, head.consts)
+        ad_w = adam_args([AdamSeg(head.weight.data_ptr(), head.m.data_ptr(), head.v.data_ptr(), buf['dw'].data_ptr(), D, head.lr,
+                                  grad_part_stride=D, n_part=plan['nblk'])], 1, head.step.data_ptr(), head.adam_consts())
         ad_w.loss_part, ad_w.n_loss_part = buf['lp'].data_ptr(), plan['nblk']
         ad_w.l1_scale, ad_w.l2_scale, ad_w.beta_loss, ad_w.losses = 0.0, 1.0 / B, 1.0, losses.data_ptr()
         _lib.call('sfgpi_adam_step', C.byref(ad_w), st)

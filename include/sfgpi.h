@@ -185,10 +185,12 @@ int sfgpi_mlp_backward(const sfgpi_backward_args *args, void *stream);
 
 /*
  * Fused multi-tensor Adam (torch/optim/adam.py::_single_tensor_adam order; sfdqn.py:282-286, tsfdqn.py:255-270) for
- * n_pol optimizers in one launch.  A segment is a contiguous parameter range with its own lr / weight decay and its
- * own gradient source (sum of n_part partials).  Per-policy strides select optimizer p's slice; stride 0 = shared
- * tensor (TSF's h, whose moments are nevertheless per optimizer).  `step` [n_pol] int32 is incremented on device.
- * Also reduces loss_part -> losses [n_pol][3] = (loss, l1, l2) when loss_part != NULL.
+ * n_pol optimizers; every call is exactly one kernel launch.  A segment is a contiguous parameter range with its own
+ * lr / weight decay and its own gradient source (sum of n_part partials).  Per-policy strides select optimizer p's
+ * slice; param_stride 0 with n_pol > 1 = shared tensor (TSF's h, whose moments are nevertheless per optimizer).  A
+ * shared tensor follows the frozen-snapshot rule: every optimizer steps it from the same pre-step value, and the
+ * n_pol deltas are summed in a fixed order.  `step` [n_pol] int32 is incremented on device.  Also reduces
+ * loss_part -> losses [n_pol][3] = (loss, l1, l2) when loss_part != NULL.
  */
 typedef struct {
     float *param;  int64_t param_stride;
@@ -208,16 +210,15 @@ typedef struct {
     double beta1, beta2, eps;       /* doubles: torch derives 1-beta and beta**t in double before the fp32 cast */
     const float *loss_part; int32_t n_loss_part; float l1_scale, l2_scale, beta_loss;
     float *losses;
-    int32_t sequential_shared;      /* 1: segments with param_stride 0 are stepped by optimizer 0..n_pol-1 in order */
-    double *consts;                 /* optional [n_pol][2]: {1 - beta1^t, sqrt(1 - beta2^t)} for t = step + 1; must be consistent
-                                       with `step` on entry, refreshed on device after the step.  NULL: computed in-kernel */
-    double *consts_next;            /* optional second [n_pol][2] buffer (needs consts): the update kernel itself advances `step`
-                                       and writes the NEXT step's corrections here (nothing reads this buffer or `step` during the
-                                       launch), so the one-block finishing launch drops off the step's dependent chain; the caller
-                                       swaps the two buffers for the next call */
+    double *consts;                 /* [n_pol][2]: {1 - beta1^t, sqrt(1 - beta2^t)} for t = step + 1, consistent with `step` on
+                                       entry; read, not written */
+    double *consts_next;            /* a second [n_pol][2] buffer, distinct from consts: the launch advances `step` and writes
+                                       the NEXT step's corrections here (nothing reads this buffer or `step` during the launch);
+                                       the caller swaps the two buffers for the next call.  A call that is not fresh needs
+                                       step, consts and consts_next, else SFGPI_E_INVALID */
     int32_t fresh;                  /* nonzero: every call is the FIRST step of a brand-new optimizer (features/deep_phi.py:170 builds a
-                                       new torch.optim.Adam per update): moments start at 0 and are not stored, t = 1, `step` / consts
-                                       are neither read nor written; m / v pointers of the segments may be NULL */
+                                       new torch.optim.Adam per update): moments start at 0 and are not stored, t = 1, `step`, consts and
+                                       consts_next are neither read nor written; m / v pointers of the segments may be NULL */
     float *losses_host;             /* optional: PINNED host buffer [n_pol][3]; the block that reduces the losses also stores them
                                        there (a zero-copy store over PCIe: the step's result reaches the host without a copy
                                        command between two kernels of the launch chain).  Valid once the launch has completed.

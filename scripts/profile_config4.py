@@ -1,5 +1,5 @@
 """Three all-task steps of BASELINE config 4 (ii) (256 policies, beta = 30, B = 4096, GPI over 256 reward vectors) for ncu:
-   ncu --set full --clock-control none --import-source on -k regex:'step_prep|fold_gpi|mlp_forward_tc|td_kernel|dgrad_tc|wgrad_tc|adam_flat' \
+   ncu --set full --clock-control none --import-source on -k regex:'step_prep|fold_gpi|mlp_forward_tc|td_kernel|dgrad_tc|wgrad_tc|adam_step' \
        -s 14 -c 7 -o gpurun_out/r02_config4 python scripts/profile_config4.py"""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))

@@ -69,7 +69,7 @@ def test_negative_sizes_are_rejected_without_a_gpu():
 
 
 def test_new_entry_points_validate_before_touching_cuda():
-    """sfgpi_step_prep / sfgpi_phi_head / peer exchange: bad arguments -> rc < 0 with an error text, no CUDA call needed."""
+    """sfgpi_step_prep / sfgpi_phi_head / peer exchange / sfgpi_adam_step: bad arguments -> rc < 0 with an error text, no CUDA call needed."""
     import ctypes as C
     L = _lib.lib()
     pr = _lib.StepPrepArgs()                                        # zeroed descriptor: not a tensor-core shape
@@ -88,6 +88,15 @@ def test_new_entry_points_validate_before_touching_cuda():
     t.peer_keys = C.addressof(ka2)                                  # peer keys without next_psi / a valid context
     assert L.sfgpi_td_step(C.byref(t), None) < 0 and b'peer_keys' in L.sfgpi_last_error()
     assert _lib.MAX_PEERS == 16 and C.sizeof(_lib.Cmd) == 80
+    # sfgpi_adam_step: a step that is not fresh reads `consts` and writes the next step's corrections into a distinct `consts_next`
+    host = (C.c_double * 8)(), (C.c_double * 8)(), (C.c_int32 * 2)()
+    ad = _lib.AdamArgs()
+    ad.n_seg, ad.n_pol, ad.step = 1, 1, C.addressof(host[2])
+    ad.seg[0].len, ad.seg[0].n_part = 4, 1
+    for consts, consts_next, missing in ((None, C.addressof(host[1]), b'needs consts'), (C.addressof(host[0]), None, b'needs consts_next'),
+                                         (C.addressof(host[0]), C.addressof(host[0]), b'distinct from consts')):
+        ad.consts, ad.consts_next = consts, consts_next
+        assert L.sfgpi_adam_step(C.byref(ad), None) < 0 and L.sfgpi_last_error().endswith(missing)
 
 
 def test_shard_range_partitions_exactly():

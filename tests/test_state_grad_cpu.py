@@ -17,7 +17,7 @@ _HOST = (C.c_float * 64)()                           # stands in for device poin
 def test_input_grad_struct_mirrors_header():
     assert c_struct_fields('sfgpi_input_grad_args') == [f[0] for f in _lib.InputGradArgs._fields_]
     assert 'sfgpi_mlp_input_grad' in _lib.SYMBOLS
-    assert _lib.lib().sfgpi_version() == 103
+    assert _lib.lib().sfgpi_version() == 104
 
 
 def _args(S=4, precision='bf16', hidden=256, B=64, n_pol=2):
