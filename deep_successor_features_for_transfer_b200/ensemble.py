@@ -52,6 +52,10 @@ class DeepSF(_DeepSF):
         super().reset()
         self._w_holders = []
 
+    def load_state_dict(self, sd):
+        super().load_state_dict(sd)
+        self.fit_w = [h.weight.data.view(-1, 1) for h in self._w_holders]
+
     def update_reward(self, phi, r, task_index, exact=False):
         """LMS rule w += alpha_w (r - phi.w) phi, in place on the packed row (features/successor.py:146-167): one tiny kernel
         (sfgpi_lms_update) -- this is the per-environment-step op of main_sfdqn_torch.py."""

@@ -27,6 +27,7 @@ from . import _lib
 from ._lib import ACT, MAX_LAYERS, ptr
 
 INT64_MIN = -(1 << 63)
+STATE_FORMAT = 1            # version of PackedSFLibrary.state_dict()
 
 
 class NetSpec:
@@ -529,6 +530,86 @@ class PackedSFLibrary:
         for k in ('online', 'target', 'm', 'v', 'w', 'w_m', 'w_v', 'step', 'adam_consts', 'adam_consts2', 'g', 'g_m', 'g_v', 'h_m', 'h_v'):
             if hasattr(self, k):
                 delattr(self, k)
+
+    # ------------------------------------------------------------------ checkpoints
+    def _state_rows(self):
+        """Names of the per-policy buffers a checkpoint holds (rows [:n]); TSF adds the shared h, saved whole."""
+        rows = ('online', 'target', 'm', 'v', 'w', 'w_m', 'w_v', 'step')
+        return rows + ('g', 'g_m', 'g_v', 'h_m', 'h_v') if self.G is not None else rows
+
+    def state_dict(self):
+        """
+        The training state of the library: format version, architecture, learning rates / weight decays, and detached CLONES
+        of rows [:n] of the online and target nets, their Adam moments, w and its moments, the int32 step counters, and for TSF
+        g, its moments, the shared h and its per-optimizer moments.  Clones, not views: adding a policy re-packs the storage,
+        which would leave a view reading a dead buffer.  The master weights are fp32 in every precision mode, so the dict does
+        not depend on the mode; the mode's operand shadows, the workspaces and the Adam bias corrections are derived on load.
+        """
+        if self._sharded:
+            raise NotImplementedError('state_dict() does not support sharded libraries')
+        if self.spec is None:
+            raise RuntimeError('the library holds no policy: nothing to save')
+        sp = self.spec
+        sd = dict(version=STATE_FORMAT, dims=list(sp.dims), acts=list(sp.acts), n_actions=sp.n_actions, n_features=sp.n_features,
+                  G=self.G, n_flows=self.n_flows, lr=dict(self.lr), wd=dict(self.wd))
+        for k in self._state_rows():
+            sd[k] = getattr(self, k).detach()[:self.n].clone()
+        if self.G is not None:
+            sd['h'] = self.h.detach().clone()
+        return sd
+
+    def load_state_dict(self, sd):
+        """
+        Restore a state_dict() into this library, which must already hold the same number of policies of the same architecture
+        (its capacity and precision mode may differ).  The data are copied into the existing buffers, so the nn.Module views and
+        the cached step plans keep valid pointers.  Everything derived is reset: operand shadows and workspaces (re-packed and
+        rebuilt by the next call), the online rows' gradient, and the bias corrections of every optimizer, recomputed from its
+        step counter as the Adam launch does.  A psi() forward recorded before the load cannot be differentiated afterwards.
+        """
+        if self._sharded:
+            raise NotImplementedError('load_state_dict() does not support sharded libraries')
+        for k in ('version', 'dims', 'acts', 'n_actions', 'n_features', 'G', 'n_flows', 'lr', 'wd') + self._state_rows():
+            if k not in sd:
+                raise ValueError(f"library state_dict: missing key '{k}'")
+        if sd['version'] > STATE_FORMAT:
+            raise ValueError(f"library state_dict: format version {sd['version']} is newer than this library's ({STATE_FORMAT})")
+        if self.spec is None:
+            raise ValueError('library state_dict: the library holds no policy; add the policies first, then load')
+        sp = self.spec
+        for k, mine in (('dims', list(sp.dims)), ('acts', list(sp.acts)), ('n_actions', sp.n_actions),
+                        ('n_features', sp.n_features), ('G', self.G), ('n_flows', self.n_flows)):
+            got = list(sd[k]) if isinstance(mine, list) else sd[k]
+            if got != mine:
+                raise ValueError(f"library state_dict: '{k}' is {sd[k]!r}, this library has {mine!r}")
+        if sd['online'].shape[0] != self.n:
+            raise ValueError(f"library state_dict: it holds {sd['online'].shape[0]} policies, this library holds {self.n}")
+        if self.G is not None and 'h' not in sd:
+            raise ValueError("library state_dict: missing key 'h'")
+        pairs = [(getattr(self, k).detach()[:self.n], k) for k in self._state_rows()]
+        pairs += [(self.h, 'h')] if self.G is not None else []
+        for dst, k in pairs:
+            if tuple(sd[k].shape) != tuple(dst.shape):
+                raise ValueError(f"library state_dict: '{k}' has shape {tuple(sd[k].shape)}, this library needs {tuple(dst.shape)}")
+        with torch.no_grad():
+            for dst, k in pairs:
+                dst.copy_(sd[k])
+        self.lr, self.wd = dict(sd['lr']), dict(sd['wd'])
+        self._shadow, self._ws = {}, {}               # the step plans bake in lr / wd and the shadows' contents
+        self.weights_gen += 1
+        self._grad_rows, self._bound_rows = set(), set()
+        if self.autograd and self.online.grad is not None:
+            self.online.grad.zero_()
+        for i, mods in enumerate(self._views):        # (same storage: only the psi Linear .grad bindings are cleared)
+            self._point_views(i, mods)
+        self.invalidate_exchange()
+        self._refresh_adam(0, self.n)
+
+    def _refresh_adam(self, lo, n):
+        """Both bias-correction buffers of optimizers [lo, lo+n) from their step counters, after the counters were written
+        outside an Adam launch (the launch's own consts_next formula, so the next step reads the same bits)."""
+        _lib.call('sfgpi_adam_refresh', self.step[lo:].data_ptr(), self.adam_consts[lo:].data_ptr(),
+                  self.adam_consts2[lo:].data_ptr(), n, ADAM_BETA1, ADAM_BETA2, _stream())
+        self._adam_par[lo:lo + n] = [0] * n
 
     # ------------------------------------------------------------------ workspaces
     def _f(self, *shape):

@@ -7,11 +7,12 @@ TD target, backward, Adam) executed by hand-written sm_100a kernels through libs
 What stays host-side Python (as in the reference): the replay ring, epsilon-greedy, environment stepping, logging.
 """
 import random
+from collections import OrderedDict
 
 import numpy as np
 import torch
 
-from .library import PackedSFLibrary
+from .library import ADAM_BETA1, ADAM_BETA2, ADAM_EPS, PackedSFLibrary
 
 
 def _device():
@@ -52,6 +53,38 @@ class ReplayBuffer:
         self.buffer[self.index] = (state, action, reward, phi, next_state, gamma)
         self.size = min(self.size + 1, self.n_samples)
         self.index = (self.index + 1) % self.n_samples
+
+    def state_dict(self):
+        """Slots [:size] as stacked tensors (states / next_states [size][S], actions int64, rewards / gammas [size], phis
+        [size][D]) with the write index and the size: the format DeviceReplayBuffer uses too, so either ring loads the other's."""
+        cols = list(zip(*self.buffer[:self.size])) if self.size else [()] * 6
+        stack = lambda c: torch.vstack([torch.as_tensor(v) for v in c]) if c else torch.empty(0)
+        return dict(n_samples=self.n_samples, index=self.index, size=self.size, states=stack(cols[0]),
+                    actions=torch.as_tensor([int(v) for v in cols[1]], dtype=torch.int64), rewards=stack(cols[2]).reshape(-1),
+                    phis=stack(cols[3]), next_states=stack(cols[4]),
+                    gammas=torch.as_tensor([float(v) for v in cols[5]], dtype=torch.float64))
+
+    def load_state_dict(self, sd):
+        _check_ring_dict(self, sd)
+        self.reset()
+        cpu = {k: sd[k].detach().cpu() for k in _RING_FIELDS}
+        for k in range(sd['size']):
+            self.buffer[k] = (cpu['states'][k:k + 1], int(cpu['actions'][k]), cpu['rewards'][k].float(), cpu['phis'][k],
+                              cpu['next_states'][k:k + 1], float(cpu['gammas'][k]))
+        self.index, self.size = int(sd['index']), int(sd['size'])
+
+
+_RING_FIELDS = ('states', 'actions', 'rewards', 'phis', 'next_states', 'gammas')
+
+
+def _check_ring_dict(ring, sd):
+    for k in ('n_samples', 'index', 'size') + _RING_FIELDS:
+        if k not in sd:
+            raise ValueError(f"replay state_dict: missing key '{k}'")
+    if int(sd['n_samples']) != ring.n_samples:
+        raise ValueError(f"replay state_dict: saved from a ring of {sd['n_samples']} samples, this ring holds {ring.n_samples}")
+    if any(sd[k].shape[0] != sd['size'] for k in _RING_FIELDS) or not 0 <= sd['index'] < ring.n_samples:
+        raise ValueError('replay state_dict: inconsistent sizes')
 
 
 class DeviceReplayBuffer:
@@ -142,6 +175,30 @@ class DeviceReplayBuffer:
         _lib.call('sfgpi_replay_gather', C.byref(self._args), C.c_void_p(torch.cuda.current_stream().cuda_stream))
         return self._out
 
+    def state_dict(self):
+        """ReplayBuffer.state_dict()'s format: clones of the packed rows [:size], split into fields (fp32, actions int64)."""
+        n, sd = self.size, dict(n_samples=self.n_samples, index=self.index, size=self.size)
+        if self.ring is None:
+            return dict(sd, **{k: torch.empty(0) for k in _RING_FIELDS})
+        S, D, rows = self.S, self.D, self.ring[:n]
+        return dict(sd, states=rows[:, :S].clone(), next_states=rows[:, S:2 * S].clone(), phis=rows[:, 2 * S:2 * S + D].clone(),
+                    rewards=rows[:, 2 * S + D].clone(), gammas=rows[:, 2 * S + D + 1].clone(),
+                    actions=rows[:, 2 * S + D + 2].to(torch.int64))
+
+    def load_state_dict(self, sd):
+        _check_ring_dict(self, sd)
+        self.reset()
+        n = int(sd['size'])
+        if n:
+            dev = _device()
+            col = lambda k: sd[k].detach().to(device=dev, dtype=torch.float32).reshape(n, -1)
+            S, D = col('states').shape[1], col('phis').shape[1]
+            if int(sd['actions'].max()) >= (1 << 24):
+                raise ValueError('action index too large for the packed fp32 row')
+            self._alloc(S, D)
+            self.ring[:n].copy_(torch.cat([col(k) for k in ('states', 'next_states', 'phis', 'rewards', 'gammas', 'actions')], 1))
+        self.index, self.size = int(sd['index']), n
+
 
 class PackedPsi(torch.nn.Module):
     """
@@ -181,19 +238,80 @@ class PackedAdamView:
         L = self._library
         return [dict(params=p, lr=L.lr[k], weight_decay=L.wd[k], betas=(0.9, 0.999), eps=1e-8) for k, p in self._groups]
 
+    _MOMENTS = {'sf': ('m', 'v'), 'w': ('w_m', 'w_v'), 'g': ('g_m', 'g_v'), 'h': ('h_m', 'h_v')}
+
+    def _moments(self, src):
+        """[(param, exp_avg, exp_avg_sq)] in param-id order: views of row i of the moment buffers src(name) (the library's, or
+        those of its state_dict), at each parameter's offset into its packed row."""
+        L, i, out = self._library, self.index, []
+        base = {'sf': L.online.detach()[i], 'w': L.w[i], 'h': L.h, 'g': L.g[i] if L.G is not None else None}
+        for k, params in self._groups:
+            m, v = (src(name)[i] for name in self._MOMENTS[k])
+            for p in params:
+                off = (p.data.data_ptr() - base[k].data_ptr()) // 4
+                out.append((p, m[off:off + p.numel()].view_as(p), v[off:off + p.numel()].view_as(p)))
+        return out
+
     @property
     def state(self):
-        L, i, out = self._library, self.index, {}
-        step = L.step[i]
-        for k, params in self._groups:
-            for p in params:
-                base, m, v = {'sf': (L.online[i], L.m[i], L.v[i]), 'w': (L.w[i], L.w_m[i], L.w_v[i]),
-                              'g': (getattr(L, 'g', [None] * (i + 1))[i], getattr(L, 'g_m', [None] * (i + 1))[i],
-                                    getattr(L, 'g_v', [None] * (i + 1))[i]),
-                              'h': (L.h, getattr(L, 'h_m', [None] * (i + 1))[i], getattr(L, 'h_v', [None] * (i + 1))[i])}[k]
-                off = (p.data.data_ptr() - base.data_ptr()) // 4
-                out[p] = dict(step=step, exp_avg=m[off:off + p.numel()].view_as(p), exp_avg_sq=v[off:off + p.numel()].view_as(p))
-        return out
+        L = self._library
+        step = L.step[self.index]
+        return {p: dict(step=step, exp_avg=m, exp_avg_sq=v) for p, m, v in self._moments(lambda name: getattr(L, name))}
+
+    def state_dict(self):
+        """torch.optim.Adam.state_dict() of optimizer i: one param group per kind in the reference's order (psi, w, and for TSF
+        g's W and b, h's W and b), integer param ids, and per parameter a 0-dim float32 `step` with clones of its moments (no
+        state before the first step).  Loads into a stock torch.optim.Adam over the same parameters, and back."""
+        L = self._library
+        return self._torch_dict(lambda name: getattr(L, name), int(L.step[self.index]), clone=True)
+
+    def _torch_dict(self, src, step, clone=False):
+        state = {}
+        if step > 0:
+            for pid, (_, m, v) in enumerate(self._moments(src)):
+                state[pid] = dict(step=torch.tensor(float(step)), exp_avg=m.clone() if clone else m,
+                                  exp_avg_sq=v.clone() if clone else v)
+        groups, pid = [], 0
+        for g in self.param_groups:
+            n = len(g['params'])
+            groups.append(dict(g, amsgrad=False, maximize=False, params=list(range(pid, pid + n))))
+            pid += n
+        return dict(state=state, param_groups=groups)
+
+    def load_state_dict(self, sd):
+        """Load a torch.optim.Adam.state_dict() over the same parameters (or this class's own): the moments go into the packed
+        rows at the parameters' offsets.  Each group's lr / weight decay must be the library's, which steps every optimizer's
+        group of that kind alike.  The packed step counter is one per optimizer, so every parameter with state must carry the
+        same step; parameters without state are allowed only when no parameter has any (a fresh optimizer)."""
+        L, i = self._library, self.index
+        groups = sd['param_groups']
+        if [len(g['params']) for g in groups] != [len(p) for _, p in self._groups]:
+            raise ValueError(f'optimizer {i}: the state_dict\'s parameter groups {[len(g["params"]) for g in groups]} do not '
+                             f'match this optimizer\'s {[len(p) for _, p in self._groups]}')
+        for (k, _), g in zip(self._groups, groups):
+            if tuple(g.get('betas', (ADAM_BETA1, ADAM_BETA2))) != (ADAM_BETA1, ADAM_BETA2) or g.get('eps', ADAM_EPS) != ADAM_EPS \
+                    or g.get('amsgrad', False) or g.get('maximize', False):
+                raise ValueError(f'optimizer {i}: the packed Adam runs betas=(0.9, 0.999), eps=1e-8 without amsgrad / maximize')
+            if g['lr'] != L.lr[k] or g.get('weight_decay', 0.0) != L.wd[k]:
+                raise ValueError(f"optimizer {i}: group '{k}' has lr={g['lr']}, weight_decay={g.get('weight_decay', 0.0)}; the "
+                                 f"library steps every optimizer's '{k}' group with lr={L.lr[k]}, weight_decay={L.wd[k]}")
+        ids = [pid for g in groups for pid in g['params']]
+        have = [pid in sd['state'] for pid in ids]
+        if any(have) and not all(have):
+            raise ValueError(f'optimizer {i}: only some parameters have Adam state; the packed step counter is one per optimizer')
+        steps = {float(sd['state'][pid]['step']) for pid in ids} if all(have) else {0.0}
+        if len(steps) != 1:
+            raise ValueError(f'optimizer {i}: the parameters carry different Adam steps {sorted(steps)}; the packed step counter '
+                             'is one per optimizer')
+        step = steps.pop()
+        with torch.no_grad():
+            for pid, (p, m, v) in zip(ids, self._moments(lambda name: getattr(L, name))):
+                st = sd['state'].get(pid)
+                m.copy_(st['exp_avg'] if st is not None else torch.zeros_like(m))
+                v.copy_(st['exp_avg_sq'] if st is not None else torch.zeros_like(v))
+            L.step[i] = int(step)
+        L._refresh_adam(i, 1)
+        self._skipped = set()
 
     def zero_grad(self, set_to_none=True):
         """Clears optimizer i's psi row of the packed gradient and the .grad of every parameter it steps (w, g and the
@@ -448,6 +566,42 @@ class DeepSF:
             self._after_update(i)
         return losses
 
+    # ---- checkpoints --------------------------------------------------------------------------------------------------
+    def state_dict(self):
+        """
+        Training state of the library: sd['library'] (PackedSFLibrary.state_dict: every network, reward vector, g / h and Adam
+        state) with gpi_counters, updates_since_target_updated, n_tasks and target_update_ev.  sd['library'] is the source of
+        truth.  sd['psi'][i] = {'model': ..., 'optim': ...} is task i in the layout of the reference's eager objects --
+        psi_model.state_dict() key names and torch.optim.Adam.state_dict() -- built from VIEWS of sd['library']'s tensors, so
+        torch.save stores the data once; load it into a reference psi_model / torch.optim.Adam to continue task i eagerly.
+        load_state_dict reads sd['library'] only.  Everything a TSF library learns (g, h) lives in the library too.
+        """
+        lib = self._library
+        lsd = lib.state_dict()
+        psi = []
+        for i in range(self.n_tasks):
+            (model, _, optim), _ = self.psi[i]
+            names = {p: n for n, p in model.net.named_parameters()}
+            weights = OrderedDict()
+            for (W, b), lin in zip(lib.spec.views(lsd['online'][i]), lib._views[i]['online']):
+                weights[names[lin.weight]], weights[names[lin.bias]] = W, b
+            psi.append(dict(model=weights, optim=optim._torch_dict(lsd.__getitem__, int(lsd['step'][i]))))
+        return dict(library=lsd, psi=psi, gpi_counters=[np.asarray(c).tolist() for c in self.gpi_counters],
+                    updates_since_target_updated=list(self.updates_since_target_updated), n_tasks=self.n_tasks,
+                    target_update_ev=self.target_update_ev)
+
+    def load_state_dict(self, sd):
+        """Restore a state_dict() into a library that already holds the same tasks (add them first, as the saved run did)."""
+        for k in ('library', 'gpi_counters', 'updates_since_target_updated', 'n_tasks', 'target_update_ev'):
+            if k not in sd:
+                raise ValueError(f"SF state_dict: missing key '{k}'")
+        if sd['n_tasks'] != self.n_tasks:
+            raise ValueError(f"SF state_dict: it holds {sd['n_tasks']} tasks, this library holds {self.n_tasks}")
+        self._library.load_state_dict(sd['library'])
+        self.gpi_counters = [np.asarray(c, dtype=int) for c in sd['gpi_counters']]
+        self.updates_since_target_updated = list(sd['updates_since_target_updated'])
+        self.target_update_ev = sd['target_update_ev']
+
 
 class SFDQN:
     """SFDQN agent, sequential variant  [sfdqn.py:374-749].  Host-side RL loop around the fused SF library."""
@@ -571,12 +725,7 @@ class SFDQN:
         for train_task in train_tasks:
             self.add_training_task(train_task)
         for test_task in test_tasks:
-            w_approx = torch.nn.Linear(test_task.feature_dim(), 1, bias=False, device=self.device)
-            with torch.no_grad():
-                w_approx.weight.uniform_(-0.01, 0.01)
-            optim = torch.optim.Adam([{'params': w_approx.parameters(), 'lr': self.hyperparameters['learning_rate_w'],
-                                       'weight_decay': self.hyperparameters['weight_decay_w']}])
-            self.test_tasks_weights.append((w_approx, optim))
+            self.test_tasks_weights.append(self._new_test_task(test_task.feature_dim()))
         return_data = []
         for _ in range(cycles_per_task):
             for index, (train_task, viewer) in enumerate(zip(train_tasks, viewers)):
@@ -592,6 +741,64 @@ class SFDQN:
                             self.logger.log_average_reward(avg_R, self.total_training_steps)
                     self.total_training_steps += 1
         return return_data
+
+    # ---- checkpoints --------------------------------------------------------------------------------------------------
+    _EPISODE = ('s', 's_enc', 'new_episode', 'episode', 'episode_reward', 'steps_since_last_episode', 'reward_since_last_episode',
+                'steps', 'reward', 'episode_reward_hist', 'cum_reward', 'reward_hist', 'cum_reward_hist')
+
+    def state_dict(self):
+        """
+        Training state of the agent: the SF library's state_dict, every task's replay ring, total_training_steps, epsilon, the
+        active task with its episode in progress, and the target tasks' reward vectors with their optimizers.  As in torch, the
+        random streams (Python `random`, numpy, torch) and the environments' own state are the caller's to save and restore.
+        """
+        active = getattr(self, 'task_index', None)
+        return dict(sf=self.sf.state_dict(), buffers=[b.state_dict() for b in self.buffers],
+                    total_training_steps=self.total_training_steps, epsilon=getattr(self, 'epsilon', self.epsilon_init),
+                    task_index=active, episode={k: list(v) if isinstance(v, list) else v
+                                                for k, v in vars(self).items() if k in self._EPISODE},
+                    test_tasks=[self._test_task_state(k) for k in range(len(self.test_tasks_weights))])
+
+    def load_state_dict(self, sd):
+        """Restore a state_dict() into an agent that already holds the same training tasks (reset() + add_training_task, as
+        the saved run did).  Target tasks are rebuilt when the agent has none yet."""
+        if len(sd['buffers']) != len(self.buffers):
+            raise ValueError(f"agent state_dict: it holds {len(sd['buffers'])} tasks, this agent holds {len(self.buffers)}")
+        if self.test_tasks_weights and len(self.test_tasks_weights) != len(sd['test_tasks']):
+            raise ValueError(f"agent state_dict: it holds {len(sd['test_tasks'])} target tasks, this agent holds "
+                             f"{len(self.test_tasks_weights)}")
+        self.sf.load_state_dict(sd['sf'])
+        for buf, bsd in zip(self.buffers, sd['buffers']):
+            buf.load_state_dict(bsd)
+        self.total_training_steps = sd['total_training_steps']
+        if sd['task_index'] is not None:
+            self.set_active_training_task(sd['task_index'])
+            for k, v in sd['episode'].items():
+                setattr(self, k, list(v) if isinstance(v, list) else v)
+        self.epsilon = sd['epsilon']
+        for k, tsd in enumerate(sd['test_tasks']):
+            self._load_test_task(k, tsd)
+
+    def _new_test_task(self, feature_dim):
+        """(w_approx, torch.optim.Adam over it) of one target task, as train() builds them."""
+        w_approx = torch.nn.Linear(feature_dim, 1, bias=False, device=self.device)
+        with torch.no_grad():
+            w_approx.weight.uniform_(-0.01, 0.01)
+        optim = torch.optim.Adam([{'params': w_approx.parameters(), 'lr': self.hyperparameters['learning_rate_w'],
+                                   'weight_decay': self.hyperparameters['weight_decay_w']}])
+        return w_approx, optim
+
+    def _test_task_state(self, k):
+        w, optim = self.test_tasks_weights[k]
+        return dict(w=w.weight.detach().clone(), optim=optim.state_dict())
+
+    def _load_test_task(self, k, tsd):
+        if k == len(self.test_tasks_weights):
+            self.test_tasks_weights.append(self._new_test_task(tsd['w'].numel()))
+        w, optim = self.test_tasks_weights[k]
+        with torch.no_grad():
+            w.weight.copy_(tsd['w'].reshape(w.weight.shape))
+        optim.load_state_dict(tsd['optim'])
 
     # ---- target tasks (host loop; calls the in-scope get_successors) -----------------------------------------------------
     def get_test_action(self, s_enc, w):

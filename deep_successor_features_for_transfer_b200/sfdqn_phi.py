@@ -232,6 +232,14 @@ class DeepSF_PHI(DeepSF):
 
     _eager_step_unsupported = 'DeepSF_PHI (its step is the joint psi / phi update)'
 
+    def state_dict(self):
+        raise NotImplementedError('DeepSF_PHI has no state_dict(): the phi network and the reward heads (fit_w with bias, '
+                                  'the loss coefficients) live outside the SF library and are not captured')
+
+    def load_state_dict(self, sd):
+        raise NotImplementedError('DeepSF_PHI has no load_state_dict(): the phi network and the reward heads live outside the '
+                                  'SF library and are not captured')
+
     def add_training_task(self, task, source=None):
         n_features = task.feature_dim()
         self.psi.append(None)                                                     # (reference order: psi nets first, then fit_w, :262-270)

@@ -48,6 +48,21 @@ class PackedTargetOptim:
                 dict(lr=self.hp['learning_rate_omega'] * (1 - self.hp['learning_rate_omega_decay']) ** epoch,
                      weight_decay=self.hp['weight_decay_omega'])]
 
+    def state_dict(self):
+        """Adam state of (w, omega) -- clones of the moments, the shared step -- and the LambdaLR epoch.  The w and omega tensors
+        themselves belong to the agent (TSFDQN.state_dict)."""
+        step, epoch = (int(v) for v in self.counters.tolist())
+        return dict(w_exp_avg=self.w_m.clone(), w_exp_avg_sq=self.w_v.clone(), omega_exp_avg=self.o_m.clone(),
+                    omega_exp_avg_sq=self.o_v.clone(), step=step, last_epoch=epoch)
+
+    def load_state_dict(self, sd):
+        with torch.no_grad():
+            for dst, k in ((self.w_m, 'w_exp_avg'), (self.w_v, 'w_exp_avg_sq'), (self.o_m, 'omega_exp_avg'), (self.o_v, 'omega_exp_avg_sq')):
+                if tuple(sd[k].shape) != tuple(dst.shape):
+                    raise ValueError(f"target-task optimizer state_dict: '{k}' has shape {tuple(sd[k].shape)}, expected {tuple(dst.shape)}")
+                dst.copy_(sd[k])
+            self.counters.copy_(torch.tensor([int(sd['step']), int(sd['last_epoch'])], dtype=torch.int32))
+
     def step_fused(self, agent, w_approx, omegas, phi, r, s, a, s1, a1):
         lib = agent.sf._library
         sp = lib.spec
@@ -261,6 +276,29 @@ class TSFDQN(SFDQN):
         decay = hp['learning_rate_omega_decay']
         scheduler = torch.optim.lr_scheduler.LambdaLR(optim, [lambda epoch: 1.0, lambda epoch: (1 - decay) ** epoch])
         return w_approx, optim, scheduler, omegas
+
+    def _test_task_state(self, k):
+        """Target task k: w, omega and their optimizer (a PackedTargetOptim, or torch.optim.Adam + LambdaLR)."""
+        w, optim, scheduler = self.test_tasks_weights[k]
+        fused = isinstance(optim, PackedTargetOptim)
+        return dict(w=w.weight.detach().clone(), omegas=self.omegas[k].detach().clone(), fused=fused, optim=optim.state_dict(),
+                    scheduler=None if fused else scheduler.state_dict())
+
+    def _load_test_task(self, k, tsd):
+        if k == len(self.test_tasks_weights):
+            w, optim, scheduler, omegas = self._new_target_task(tsd['w'].numel(), tsd['omegas'].to(self.device), fused=tsd['fused'])
+            self.test_tasks_weights.append((w, optim, scheduler))
+            self.omegas.append(omegas)
+        w, optim, scheduler = self.test_tasks_weights[k]
+        if isinstance(optim, PackedTargetOptim) != tsd['fused']:
+            raise ValueError(f'agent state_dict: target task {k} was saved with a '
+                             f"{'fused' if tsd['fused'] else 'torch.optim.Adam'} optimizer, this agent has the other kind")
+        with torch.no_grad():
+            w.weight.copy_(tsd['w'].reshape(w.weight.shape))
+            self.omegas[k].copy_(tsd['omegas'])
+        optim.load_state_dict(tsd['optim'])
+        if tsd['scheduler'] is not None:
+            scheduler.load_state_dict(tsd['scheduler'])
 
     def train(self, train_tasks, n_samples, viewers=None, n_view_ev=None, test_tasks=[], n_test_ev=1000, cycles_per_task=1):
         if viewers is None:
