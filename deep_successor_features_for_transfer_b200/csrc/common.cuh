@@ -57,6 +57,39 @@ __device__ __forceinline__ void trace_exit(int trace_slot) { trace_mark(trace_sl
 
 bool pdl_enabled();
 
+// Lets `kernel` launch with `bytes` of dynamic shared memory.  CUDA counts the kernel's static shared memory against the same
+// per-block limit (kMaxSmem), so the static size is read from the kernel once (cached in *static_bytes, initialised to -1) and
+// included in the check.  When static + dynamic exceed the default 48 KB the kernel is opted in to exactly `bytes`.
+// SFGPI_E_SMEM, with the sizes in the error text, when the block cannot have that much.
+template <typename K>
+inline int smem_opt_in(K *kernel, size_t bytes, int *static_bytes, const char *what) {
+    if (*static_bytes < 0) {
+        cudaFuncAttributes fa = {};
+        const cudaError_t e = cudaFuncGetAttributes(&fa, kernel);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            set_error("%s: cudaFuncGetAttributes: %s", what, cudaGetErrorString(e));
+            return SFGPI_E_CUDA;
+        }
+        *static_bytes = (int)fa.sharedSizeBytes;
+    }
+    if (bytes + (size_t)*static_bytes > (size_t)kMaxSmem) {
+        set_error("%s: needs %zu B of dynamic + %d B of static shared memory, more than the %d B of a block", what, bytes,
+                  *static_bytes, kMaxSmem);
+        return SFGPI_E_SMEM;
+    }
+    if (bytes + (size_t)*static_bytes > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            set_error("%s: cannot opt in to %zu B of dynamic shared memory (%d B static): %s", what, bytes, *static_bytes,
+                      cudaGetErrorString(e));
+            return SFGPI_E_SMEM;
+        }
+    }
+    return SFGPI_OK;
+}
+
 template <typename... KArgs, typename... Args>
 inline void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args &&...args) {
     cudaLaunchConfig_t cfg = {};

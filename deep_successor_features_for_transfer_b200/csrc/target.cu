@@ -185,8 +185,8 @@ extern "C" int sfgpi_target_adapt(const sfgpi_target_args *args, void *stream) {
     }
     const size_t fl = (size_t)a.N * 2 + (size_t)a.N * a.G + 2 * (size_t)a.G + 4 * (size_t)a.D;
     const size_t bytes = fl * sizeof(float);
-    if (bytes > (size_t)kMaxSmem) { set_error("sfgpi_target_adapt: N * G too large for shared memory (%zu B)", bytes); return SFGPI_E_SMEM; }
-    if (bytes > 48 * 1024) cudaFuncSetAttribute(target_adapt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem);
+    static int adapt_static = -1;
+    if (int rc = smem_opt_in(target_adapt_kernel, bytes, &adapt_static, "sfgpi_target_adapt (N * G too large)")) return rc;
     launch_pdl(target_adapt_kernel, dim3(1), dim3(kTgtThreads), bytes, (cudaStream_t)stream, a);
     return check_launch("sfgpi_target_adapt");
 }

@@ -353,8 +353,6 @@ extern "C" int sfgpi_td_step(const sfgpi_td_args *args, void *stream) {
     if (tsf) fl += (size_t)a.D * a.S + a.D + 2 * (size_t)kTdRows * a.S + (a.tsf_mc ? 0 : (size_t)a.G * a.S + a.G + (size_t)a.D * a.G + a.D);
     if (K > 0) fl += 3 * (size_t)tsf_flow_len(a.S, K) + 2 * (size_t)kTdRows * ((size_t)(K + 1) * a.S + K);
     const size_t bytes = fl * sizeof(float);
-    if (bytes > (size_t)kMaxSmem) { set_error("sfgpi_td_step: D/G too large for shared memory (%zu B)", bytes); return SFGPI_E_SMEM; }
-    if (bytes > 48 * 1024) cudaFuncSetAttribute(td_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem);
     const int nclu = sfgpi_td_partials(a.B);
     dim3 grid(nclu * kTdCluster, a.n_pol);
     sfgpi_peer_keys_args pk = {};
@@ -368,11 +366,15 @@ extern "C" int sfgpi_td_step(const sfgpi_td_args *args, void *stream) {
         for (int r = 0; r < pk.ctx.world; ++r)
             if (!pk.ctx.flags[r] || !pk.keys_all[r]) { set_error("sfgpi_td_step: peer arena of rank %d not mapped", r); return SFGPI_E_INVALID; }
     }
+    // every argument is checked before the first CUDA call; both launches' shared memory before the first launch
+    const size_t ebytes = ((size_t)n_red + (size_t)a.G * a.S + a.G + (size_t)a.D * a.G) * sizeof(float);
+    static int td_static = -1, expand_static = -1;
+    if (int rc = smem_opt_in(td_kernel, bytes, &td_static, "sfgpi_td_step (D/G too large)")) return rc;
+    if (tsf && !a.defer_expand)
+        if (int rc = smem_opt_in(tsf_expand_kernel, ebytes, &expand_static, "sfgpi_td_step(expand)")) return rc;
     launch_pdl(td_kernel, grid, dim3(kTdThreads), bytes, (cudaStream_t)stream, a, pk);
     int rc = check_launch("sfgpi_td_step");
     if (rc || !tsf || a.defer_expand) return rc;              // deferred: the expand rides in sfgpi_mlp_backward_tc's dgrad launch
-    const size_t ebytes = ((size_t)n_red + (size_t)a.G * a.S + a.G + (size_t)a.D * a.G) * sizeof(float);
-    if (ebytes > 48 * 1024) cudaFuncSetAttribute(tsf_expand_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem);
     launch_pdl(tsf_expand_kernel, dim3(a.n_pol), dim3(256), ebytes, (cudaStream_t)stream, a, nclu);
     return check_launch("sfgpi_td_step(expand)");
 }
