@@ -844,7 +844,8 @@ static bool tc_shape_ok(const sfgpi_net_desc &net, const char **why) {
     if (net.n_layers < 3) { *why = "needs >= 3 Linear layers"; return false; }
     for (int l = 1; l < net.n_layers; ++l)
         if (net.dims[l] != kH) { *why = "every hidden width must be 256"; return false; }
-    if (net.dims[0] > 64) { *why = "state dimension must be <= 64"; return false; }
+    // S <= 63, not 64: the backward, the step prologue and the state gradient read xo = [x | 1 | 0...], 64 columns wide
+    if (net.dims[0] > 63) { *why = "needs S <= 63"; return false; }
     if (net.acts[net.n_layers - 1] != SFGPI_ACT_NONE) { *why = "output layer must be linear"; return false; }
     return true;
 }

@@ -234,7 +234,7 @@ int sfgpi_adam_refresh(const int32_t *step, double *consts_a, double *consts_b, 
  * Tensor-core mode (mode 1): bf16 operands on tcgen05 with fp32 accumulation in TMEM, weights streamed by TMA.  Same
  * arguments and epilogues as sfgpi_mlp_forward; needs the bf16 shadow of the library produced by sfgpi_pack_bf16
  * ([n_policies_total][sfgpi_bf16_rows_per_policy()][256] bf16: the hidden 256x256 matrices, then the output matrix padded to
- * a multiple of 16 rows, preceded by the input matrix zero-padded to 256 columns).  Shapes: hidden widths == 256, S <= 64.  Stated tolerance vs fp32: 2e-2 scale-relative on
+ * a multiple of 16 rows, preceded by the input matrix zero-padded to 256 columns).  Shapes: hidden widths == 256, S <= 63.  Stated tolerance vs fp32: 2e-2 scale-relative on
  * psi / q (SURVEY section 7: bf16 inputs, fp32 accumulate), GPI argmax equal wherever the fp32 top-1/top-2 gap exceeds it.
  */
 int sfgpi_bf16_rows_per_policy(const sfgpi_net_desc *net);

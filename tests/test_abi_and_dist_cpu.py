@@ -99,6 +99,27 @@ def test_new_entry_points_validate_before_touching_cuda():
         assert L.sfgpi_adam_step(C.byref(ad), None) < 0 and L.sfgpi_last_error().endswith(missing)
 
 
+def test_bf16_shadow_and_fold_refuse_s64_like_the_backward():
+    """The bf16 backward, the step prologue and the state gradient need S <= 63 (xo = [x | 1 | 0...] is 64 columns wide), so the
+    bf16 pack and GPI fold -- the first calls a bf16 library makes -- refuse S = 64 up front instead of building a library
+    whose every train step fails.  S = 63 passes validation (n_pol = 0: nothing is launched)."""
+    import ctypes as C
+    from deep_successor_features_for_transfer_b200.library import NetSpec
+    L = _lib.lib()
+    for S, ok in ((64, False), (63, True)):
+        desc = NetSpec([S, 256, 256, 256, 108], ['none', 'relu', 'relu', 'none'], 9, 12).desc()
+        n_pol = 0 if ok else 1                                      # S = 64 with one policy: refused before any pointer is read
+        rc_pack = L.sfgpi_pack_bf16(C.byref(desc), None, 0, n_pol, None, None)
+        err_pack = L.sfgpi_last_error()
+        rc_fold = L.sfgpi_fold_gpi(C.byref(desc), None, 0, n_pol, None, 1, 0, None, None, None)
+        err_fold = L.sfgpi_last_error()
+        if ok:
+            assert rc_pack == 0 and rc_fold == 0
+        else:
+            assert rc_pack == -1 and b'sfgpi_pack_bf16' in err_pack and b'S <= 63' in err_pack       # SFGPI_E_INVALID
+            assert rc_fold == -1 and b'sfgpi_fold_gpi' in err_fold and b'S <= 63' in err_fold
+
+
 def test_shard_range_partitions_exactly():
     for n_total in (1, 4, 7, 64, 256):
         for world in (1, 2, 3, 8):

@@ -22,9 +22,9 @@ def fro_err(a, b):
     return float((a - b).norm() / b.norm().clamp_min(1e-30))
 
 
-def make(S, A, D, N, seed, tsf_dim=None, beta=1):
+def make(S, A, D, N, seed, tsf_dim=None, beta=1, hidden=(256, 256), acts=('relu', 'relu')):
     gen = torch.Generator().manual_seed(seed)
-    o = OracleSF(S, A, D, (256, 256), ('relu', 'relu'), tsf_dim=tsf_dim, beta=beta)
+    o = OracleSF(S, A, D, hidden, acts, tsf_dim=tsf_dim, beta=beta)
     for _ in range(N):
         o.add_random_policy(gen)
     return o, gen
@@ -58,20 +58,24 @@ def test_bf16_forward_chain_kernel_multi_tile(S, A, D, N, B, hopper):
         _lib.lib().sfgpi_set_option(b'forward_chain', old)
 
 
-@pytest.mark.parametrize('variant', ['g2', 'g3'])
-def test_bf16_chain_and_pair_kernels_agree_bit_for_bit(variant):
+@pytest.mark.parametrize('variant,net', [pytest.param('g2', 'headline', id='g2'), pytest.param('g3', 'headline', id='g3'),
+                                         pytest.param('g2', 'L8', id='g2-L8')])
+def test_bf16_chain_and_pair_kernels_agree_bit_for_bit(variant, net):
     """Both forward kernels issue the same MMAs in the same k order on the same bf16 operands and share the epilogue arithmetic:
     an all-task train step (online forward with saved activations / ReLU masks, fused GPI with 4 reward vectors, target
-    forward) must leave bit-identical losses, weights and Adam moments whichever kernel ran the forward."""
+    forward) must leave bit-identical losses, weights and Adam moments whichever kernel ran the forward.  'L8': the deepest
+    net (8 Linear layers) at Hopper's shape, (1 + 6) * 256 + 1350 > 3072 bias floats: the chain kernel single-buffers its
+    biases."""
     from deep_successor_features_for_transfer_b200 import _lib
-    S, A, D, N, B = 4, 9, 12, 4, 1000
+    S, A, D, N, B = (11, 27, 50, 4, 1000) if net == 'L8' else (4, 9, 12, 4, 1000)
+    hidden, acts = ((256,) * 6, ('relu',) * 6) if net == 'L8' else ((256, 256), ('relu', 'relu'))
     tsf = variant == 'g3'
-    meta = dict(S=S, A=A, D=D, hidden=[256, 256], acts=['relu', 'relu'], N=N, gdim=100, beta=1, use_gpi=True)
+    meta = dict(S=S, A=A, D=D, hidden=list(hidden), acts=list(acts), N=N, gdim=100, beta=1, use_gpi=True)
     outs = []
     for mode in (0, 2):
         old = _lib.lib().sfgpi_set_option(b'forward_chain', mode)
         try:
-            o, gen = make(S, A, D, N, seed=5, tsf_dim=100 if tsf else None)
+            o, gen = make(S, A, D, N, seed=5, tsf_dim=100 if tsf else None, hidden=hidden, acts=acts)
             if tsf:
                 sf, ag = gu.build_g3(meta, oracle=o)
                 sf._library.set_precision('bf16')

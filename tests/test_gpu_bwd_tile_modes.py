@@ -18,10 +18,11 @@ HYPER_BF16 = dict(gu.HYPER, precision='bf16')
 
 def _lib(S, A, D, acts, N, seed):
     gen = torch.Generator().manual_seed(seed)                      # same seed: the first nets of every N are the same nets
-    o = OracleSF(S, A, D, (256, 256), tuple(acts))
+    hidden = (256,) * len(acts)                                    # one activation per hidden layer
+    o = OracleSF(S, A, D, hidden, tuple(acts))
     for _ in range(N):
         o.add_random_policy(gen)
-    meta = dict(S=S, A=A, D=D, hidden=[256, 256], acts=list(acts), N=N)
+    meta = dict(S=S, A=A, D=D, hidden=list(hidden), acts=list(acts), N=N)
     return gu.build_g2(meta, oracle=o, hyper=HYPER_BF16)._library
 
 
@@ -35,6 +36,8 @@ def _rel(a, b):
     (4, 9, 12, ('relu', 'relu'), 4000),   # ragged last tile
     (4, 9, 12, ('relu', 'relu'), 32),     # one partial tile per policy (both launches one tile per CTA)
     (4, 2, 20, ('tanh', 'tanh'), 4096),   # tanh CartPole net: the epilogue reads the saved activations
+    (4, 9, 12, ('relu',), 4096),          # 3 Linear layers: a dgrad chain of one hidden layer
+    (11, 27, 50, ('tanh',) * 3, 4096),    # 5 Linear layers, Hopper: odd hidden count, tanh only (no ReLU masks), 6 output chunks
 ])
 def test_one_tile_and_paired_backward_agree(S, A, D, acts, B, dense):
     small, large = _lib(S, A, D, acts, 4, seed=5), _lib(S, A, D, acts, 8, seed=5)
