@@ -134,7 +134,9 @@ __global__ void __launch_bounds__(256) gpi_from_psi_kernel(const float *__restri
             }
             if (q_out) q_out[(size_t)b * N * A + cell] = q;
             const int j = cell / A, act = cell - j * A;
-            const long long ka = pack_key(q, (uint32_t)act), kt = pack_key(q, (uint32_t)(task_base + j));
+            // a NaN packs as -inf: never selected, as in the fused epilogues (a packed NaN would order above +inf)
+            const float qk = fmaxf(q, -INFINITY);
+            const long long ka = pack_key(qk, (uint32_t)act), kt = pack_key(qk, (uint32_t)(task_base + j));
             kA = ka > kA ? ka : kA;
             kT = kt > kT ? kt : kT;
         }

@@ -165,8 +165,10 @@ __global__ void __launch_bounds__(kThreads, 1) mlp_forward_kernel(const __grid_c
                 for (int wl = 0; wl < nw; ++wl) {
                     const float *wv = w_s + wl * D;
                     const int wi = a.w_diag ? pl : wl;                      // key row
+                    // (-inf, the chunk's first action): a chunk emits a key even when no q beats -inf (all NaN / -inf), so
+                    // such a state decodes to action 0 as in the tensor-core scans, never to the unwritten key's index
                     float best = -INFINITY;
-                    int best_a = 0x7FFFFFFF;
+                    int best_a = a0;
                     for (int al = sub; al < na; al += 4) {
                         const float *pv = trow + al * D;
                         float q = 0.0f;
@@ -181,7 +183,7 @@ __global__ void __launch_bounds__(kThreads, 1) mlp_forward_kernel(const __grid_c
                         const int oa = __shfl_xor_sync(0xffffffffu, best_a, o);
                         if (ob > best || (ob == best && oa < best_a)) { best = ob; best_a = oa; }
                     }
-                    if (sub == 0 && b < B && best_a != 0x7FFFFFFF) {
+                    if (sub == 0 && b < B) {
                         if (a.key_action) atomicMax(reinterpret_cast<long long *>(a.key_action) + (size_t)wi * B + b,
                                                     pack_key(best, (uint32_t)best_a));
                         if (a.key_task) atomicMax(reinterpret_cast<long long *>(a.key_task) + (size_t)wi * B + b,

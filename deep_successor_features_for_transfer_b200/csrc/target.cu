@@ -44,9 +44,10 @@ __global__ void __launch_bounds__(kTgtThreads) target_q_kernel(const float *__re
     }
     __syncthreads();
     if (threadIdx.x == 0 && action_out) {
+        float best_q = -INFINITY;
         int best = 0;
-        for (int a = 1; a < A; ++a)
-            if (q_s[a] > q_s[best]) best = a;                  // first maximal index (torch.argmax)
+        for (int a = 0; a < A; ++a)                            // first maximal index (torch.argmax); a NaN is never selected,
+            if (q_s[a] > best_q) { best_q = q_s[a]; best = a; }     // all NaN / -inf: 0 (the packed GPI keys' rule)
         action_out[0] = best;
     }
 }

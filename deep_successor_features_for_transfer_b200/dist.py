@@ -22,8 +22,10 @@ def shard_range(n_total, world, rank):
 
 
 def pack_keys(values, indices):
-    """torch mirror of csrc/common.cuh::pack_key: fp32 values [*], integer indices [*] -> int64 keys."""
-    v = (values.float() + 0.0).contiguous()
+    """torch mirror of csrc/common.cuh::pack_key: fp32 values [*], integer indices [*] -> int64 keys.  A NaN value packs as
+    -inf, as the device epilogues treat it: never selected (a packed NaN would order above +inf)."""
+    v = values.float()
+    v = (torch.where(v.isnan(), float('-inf'), v) + 0.0).contiguous()
     bits = v.view(torch.int32).to(torch.int64)
     ordered = torch.where(bits >= 0, bits, bits ^ 0x7FFFFFFF)
     low = (0xFFFFFFFF - indices.to(torch.int64)) & 0xFFFFFFFF

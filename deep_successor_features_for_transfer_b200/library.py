@@ -908,6 +908,8 @@ class PackedSFLibrary:
         With (lo, n_pol) = (i, 1) row 0 is argmax_a q_i: the `use_gpi=False` selection, at the cost of ONE net instead of N.
         Tie clause: the reference takes the first maximal task and then the first maximal action of THAT task's row; the key
         takes the smallest action among all cells holding the maximum -- they differ only under exact fp32 ties across policies.
+        -0 and +0 tie.  A NaN q is never selected, and a state whose q are all NaN or -inf selects action 0 and task lo (torch's
+        argmax would take the first NaN of a row that mixes NaN with numbers).
         The result lives in a per-batch-size workspace and is valid until the next gpi_select call of the same size.
         """
         x = self._check_x(x)

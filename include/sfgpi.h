@@ -92,8 +92,11 @@ int sfgpi_mlp_forward(const sfgpi_forward_args *args, void *stream);
 
 /*
  * Packed (value,index) keys: key = (orderable_i32(q) << 32) | (0xFFFFFFFF - index); signed int64 max == max q, ties
- * -> smallest index (torch.argmax first-index rule, sfdqn.py:239,316).  Signed so that the cross-GPU reduction is a
- * plain NCCL/gloo MAX all-reduce on int64.  Decode: action/task as int64 (torch index dtype), value as fp32.
+ * -> smallest index (torch.argmax first-index rule, sfdqn.py:239,316), -0 == +0.  A NaN q is never selected; when every
+ * q of a (state, reward vector) is NaN or -inf the key decodes to index 0 (action 0, task task_base) with value -inf --
+ * torch.argmax would pick the first NaN of a row that mixes NaN with numbers.  Every GPI entry point writes a key for every
+ * valid state.  Signed so that the cross-GPU reduction is a plain NCCL/gloo MAX all-reduce on int64.  Decode: action/task
+ * as int64 (torch index dtype), value as fp32.
  */
 int sfgpi_keys_fill(int64_t *keys, int64_t n, void *stream);
 int sfgpi_keys_decode(const int64_t *keys, int64_t n, int64_t *index_out, float *value_out, void *stream);
@@ -410,7 +413,7 @@ int sfgpi_g4_head(const sfgpi_g4_args *args, void *stream);
  * Target-task adaptation of the TSF agent, batch 1 (SURVEY 8f N1; tsfdqn.py:859-997).  psi / next_psi: [N][A][D] = get_successors(s)
  * / get_next_successors(s') of sfgpi_mlp_forward* for ONE state.
  *   sfgpi_target_q     q[a] = w . sum_j (omega_j / sum omega) psi_j[a,:]  (get_test_action's greedy branch, :864-871), q_out [A]
- *                      and / or action_out [1] = argmax (first maximal index); A <= 256
+ *                      and / or action_out [1] = argmax (first maximal index; the packed keys' NaN rule); A <= 256
  *   sfgpi_target_adapt update_test_reward_mapper (:917-997) + scheduler.step() (:895) in one kernel: loss = MSE(tsf(s,a),
  *                      phi~ + gamma tsf^-(s',a')) + beta (w.phi~ - r)^2 + l1_coef |omega|_1 with phi~ = phi * (h(sum_j omega^_j g_j(s))
  *                      + h(sum_j omega^_j g_j(s'))); Adam (betas 0.9 / 0.999, eps 1e-8, torch op order) on w (lr_w, wd_w) and omega

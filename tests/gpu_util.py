@@ -77,6 +77,19 @@ def psi_params(sf, i, target=False):
     return [(lin.weight.data.cpu(), lin.bias.data.cpu()) for lin in linears(sf.psi[i][1 if target else 0][0].net)]
 
 
+def gpi_rule(q, index):
+    """
+    The selection rule of the packed GPI keys (include/sfgpi.h, DESIGN.md "Packed keys") in float64: q [..., M] over M cells
+    with index [M] -> the largest q, among the cells holding it the smallest index (-0 == +0); NaN is never selected; when
+    every cell is NaN or -inf, index.min().  Returns (index [...], value [...]: the maximum, -inf in the last case).
+    """
+    v = torch.where(q.isnan(), torch.tensor(float('-inf'), dtype=q.dtype), q)
+    m = v.max(dim=-1).values
+    cand = (v == m.unsqueeze(-1)) & (m.unsqueeze(-1) > float('-inf'))
+    pick = torch.where(cand, index, int(index.max()) + 1).min(dim=-1).values
+    return torch.where(m == float('-inf'), index.min(), pick), m
+
+
 def argmax_mismatch_ok(q_ref, idx_ref, idx_got, dim_pair, tol):
     """
     GPI argmax must be bit-exact except for ties inside tolerance: wherever the indices differ, the reference's top-1 and

@@ -13,6 +13,7 @@ import torch.distributed as dist
 import torch.multiprocessing as mp
 
 from deep_successor_features_for_transfer_b200 import _lib, dist as sdist
+from tests import gpu_util as gu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HEADER = os.path.join(ROOT, 'include', 'sfgpi.h')
@@ -145,6 +146,34 @@ def test_key_packing_orders_like_argmax_first_index():
     v, i = sdist.unpack_keys(sdist.pack_keys(torch.tensor([-1.5, 0.0, 2.0 ** 127, -2.0 ** 127]), torch.tensor([0, 7, 2 ** 31, 5])))
     assert v.tolist() == [-1.5, 0.0, 2.0 ** 127, -2.0 ** 127] and i.tolist() == [0, 7, 2 ** 31, 5]
 
+
+
+def test_key_packing_never_selects_nan():
+    """NaN is never selected, +-inf order as values, a row of NaN / -inf only decodes to index 0 (task: task_base), as on the
+    device (tests/gpu_util.py::gpi_rule)."""
+    g = torch.Generator().manual_seed(5)
+    q = torch.randint(-2, 3, (64, 3, 9), generator=g).float()
+    neg_nan = (torch.tensor(float('nan')).view(torch.int32) | -2 ** 31).view(torch.float32)
+    q[0:8, :, 0] = float('nan')                                     # NaN first, beside finite maxima
+    q[8:16] = float('nan')
+    q[16:24] = neg_nan
+    q[24:32] = float('-inf')
+    q[32:40, 1, 2] = float('inf')
+    q[32:36, 2, 1] = float('inf')
+    q[40:48] = torch.where(torch.rand(8, 3, 9, generator=g) < 0.5, float('nan'), float('-inf'))
+    q[48:56, :, 3:] = neg_nan
+    q[56:64] = torch.where(torch.rand(8, 3, 9, generator=g) < 0.5, 0.0, -0.0)
+    for task_base in (0, 5):
+        ka, kt = sdist.gpi_keys_from_q(q, task_base=task_base)
+        (va, ia), (vt, it) = sdist.unpack_keys(ka), sdist.unpack_keys(kt)
+        cells = q.reshape(64, -1).double()
+        a_ref, m = gu.gpi_rule(cells, torch.arange(9).repeat(3))
+        t_ref, _ = gu.gpi_rule(cells, (task_base + torch.arange(3)).repeat_interleave(9))
+        assert torch.equal(ia, a_ref) and torch.equal(it, t_ref)
+        assert torch.equal(va.double(), m) and torch.equal(vt.double(), m)
+        assert not va.isnan().any()
+    assert int(ia[8]) == 0 and int(it[8]) == 5 and float(va[8]) == float('-inf')      # all NaN
+    assert (int(ia[32]), int(it[32]), int(ia[36]), int(it[36])) == (1, 6, 2, 6)                 # ties at +inf
 
 def _free_port():
     s = socket.socket()
