@@ -58,6 +58,27 @@ def allreduce_max_keys(keys, group=None):
     return keys
 
 
+def gather_rows(t, shard, out=None):
+    """
+    Collective over shard.group: every rank's rows t [n_local, ...] -> [n_total, ...] in global policy order (rank r's rows
+    at [lo_r, lo_r + counts[r])), into `out` when given.  Uneven counts travel padded to the largest shard, so one
+    all-gather serves every backend (gloo has no uneven all-gather).
+    """
+    t = t.contiguous()
+    if out is None:
+        out = t.new_empty((shard.n_total,) + tuple(t.shape[1:]))
+    if shard.uniform:
+        dist.all_gather_into_tensor(out, t, group=shard.group)
+        return out
+    m = max(shard.counts)
+    pad = t.new_zeros((m,) + tuple(t.shape[1:]))
+    pad[:t.shape[0]] = t
+    allp = t.new_empty((shard.world * m,) + tuple(t.shape[1:]))
+    dist.all_gather_into_tensor(allp, pad, group=shard.group)
+    torch.cat([allp[r * m:r * m + c] for r, c in enumerate(shard.counts)], out=out)
+    return out
+
+
 class ShardContext:
     """Rank-local view of a policy-sharded library: which global policy indices live here."""
 

@@ -546,19 +546,39 @@ class PackedSFLibrary:
         g, its moments, the shared h and its per-optimizer moments.  Clones, not views: adding a policy re-packs the storage,
         which would leave a view reading a dead buffer.  The master weights are fp32 in every precision mode, so the dict does
         not depend on the mode; the mode's operand shadows, the workspaces and the Adam bias corrections are derived on load.
+
+        On a policy-sharded library this is a collective over the shard's process group: every rank of the group must call
+        it, in the same order, and every rank returns the same FULL dict -- the rows of all shard.n_total policies in global
+        policy order and h as rank 0 of the group holds it -- which is exactly the dict one library holding all those
+        policies would save.  It records nothing about the world size, so it loads into a library sharded over any number of
+        GPUs, or into one GPU's.  Being full-sized on every rank (256 Reacher policies: about 0.66 GB), it is best saved from
+        one rank.
         """
-        if self._sharded:
-            raise NotImplementedError('state_dict() does not support sharded libraries')
         if self.spec is None:
             raise RuntimeError('the library holds no policy: nothing to save')
+        if self._sharded:
+            self._check_group('state_dict')
         sp = self.spec
         sd = dict(version=STATE_FORMAT, dims=list(sp.dims), acts=list(sp.acts), n_actions=sp.n_actions, n_features=sp.n_features,
                   G=self.G, n_flows=self.n_flows, lr=dict(self.lr), wd=dict(self.wd))
+        from .dist import gather_rows
         for k in self._state_rows():
-            sd[k] = getattr(self, k).detach()[:self.n].clone()
+            rows = getattr(self, k).detach()[:self.n]
+            sd[k] = gather_rows(rows, self.shard) if self._sharded else rows.clone()
         if self.G is not None:
             sd['h'] = self.h.detach().clone()
+            if self._sharded:
+                import torch.distributed as dist
+                dist.broadcast(sd['h'], group=self.shard.group, group_src=0)
         return sd
+
+    def _check_group(self, what):
+        """A sharded library saves and loads inside its process group: after destroy_process_group() the other shards' rows
+        are out of reach."""
+        import torch.distributed as dist
+        if not dist.is_initialized():
+            raise NotImplementedError(f'{what}() of a sharded library is a collective over its process group, and '
+                                      'torch.distributed is not initialized; it is supported while the group is alive')
 
     def load_state_dict(self, sd):
         """
@@ -567,9 +587,14 @@ class PackedSFLibrary:
         the cached step plans keep valid pointers.  Everything derived is reset: operand shadows and workspaces (re-packed and
         rebuilt by the next call), the online rows' gradient, and the bias corrections of every optimizer, recomputed from its
         step counter as the Adam launch does.  A psi() forward recorded before the load cannot be differentiated afterwards.
+
+        On a policy-sharded library every rank of the group passes the same full dict (state_dict() of a library of
+        shard.n_total policies, sharded over any number of GPUs or not at all) and keeps its own rows [shard.lo, shard.lo + n)
+        and the whole h.  The dict is checked in full before anything is copied, so a bad dict raises the same error on every
+        rank.  The next train step gathers the reward vectors of every rank again and restarts the h exchange from the loaded h.
         """
         if self._sharded:
-            raise NotImplementedError('load_state_dict() does not support sharded libraries')
+            self._check_group('load_state_dict')
         for k in ('version', 'dims', 'acts', 'n_actions', 'n_features', 'G', 'n_flows', 'lr', 'wd') + self._state_rows():
             if k not in sd:
                 raise ValueError(f"library state_dict: missing key '{k}'")
@@ -583,18 +608,23 @@ class PackedSFLibrary:
             got = list(sd[k]) if isinstance(mine, list) else sd[k]
             if got != mine:
                 raise ValueError(f"library state_dict: '{k}' is {sd[k]!r}, this library has {mine!r}")
-        if sd['online'].shape[0] != self.n:
-            raise ValueError(f"library state_dict: it holds {sd['online'].shape[0]} policies, this library holds {self.n}")
+        lo, n_total = (self.shard.lo, self.shard.n_total) if self._sharded else (0, self.n)
+        if sd['online'].shape[0] != n_total:
+            have = f'this sharded library holds {n_total} over {self.shard.world} ranks' if self._sharded else \
+                f'this library holds {self.n}'
+            raise ValueError(f"library state_dict: it holds {sd['online'].shape[0]} policies, {have}")
         if self.G is not None and 'h' not in sd:
             raise ValueError("library state_dict: missing key 'h'")
-        pairs = [(getattr(self, k).detach()[:self.n], k) for k in self._state_rows()]
-        pairs += [(self.h, 'h')] if self.G is not None else []
-        for dst, k in pairs:
-            if tuple(sd[k].shape) != tuple(dst.shape):
-                raise ValueError(f"library state_dict: '{k}' has shape {tuple(sd[k].shape)}, this library needs {tuple(dst.shape)}")
+        # (destination, key, source rows): the per-policy buffers take rows [lo, lo + n) of the dict, h is whole
+        pairs = [(getattr(self, k).detach()[:self.n], k, slice(lo, lo + self.n)) for k in self._state_rows()]
+        pairs += [(self.h, 'h', slice(None))] if self.G is not None else []
+        for dst, k, _ in pairs:
+            want = tuple(dst.shape) if k == 'h' else (n_total,) + tuple(dst.shape[1:])
+            if tuple(sd[k].shape) != want:
+                raise ValueError(f"library state_dict: '{k}' has shape {tuple(sd[k].shape)}, this library needs {want}")
         with torch.no_grad():
-            for dst, k in pairs:
-                dst.copy_(sd[k])
+            for dst, k, rows in pairs:
+                dst.copy_(sd[k][rows])
         self.lr, self.wd = dict(sd['lr']), dict(sd['wd'])
         self._shadow, self._ws = {}, {}               # the step plans bake in lr / wd and the shadows' contents
         self.weights_gen += 1
@@ -1499,12 +1529,8 @@ class PackedSFLibrary:
         return losses
 
     def _gather_w(self, w_all):
-        import torch.distributed as dist
-        if self.shard.uniform:
-            dist.all_gather_into_tensor(w_all, self.w[:self.n].contiguous(), group=self.shard.group)
-        else:
-            parts = [w_all[sum(self.shard.counts[:r]):sum(self.shard.counts[:r + 1])] for r in range(self.shard.world)]
-            dist.all_gather(parts, self.w[:self.n].contiguous(), group=self.shard.group)
+        from .dist import gather_rows
+        gather_rows(self.w[:self.n], self.shard, out=w_all)
 
     def target_sync(self, i):
         """update_models_weights(psi_model, target_psi_model) (utils/torch.py:31-33): one contiguous D2D row copy."""

@@ -240,13 +240,13 @@ class PackedAdamView:
 
     _MOMENTS = {'sf': ('m', 'v'), 'w': ('w_m', 'w_v'), 'g': ('g_m', 'g_v'), 'h': ('h_m', 'h_v')}
 
-    def _moments(self, src):
-        """[(param, exp_avg, exp_avg_sq)] in param-id order: views of row i of the moment buffers src(name) (the library's, or
-        those of its state_dict), at each parameter's offset into its packed row."""
+    def _moments(self, src, row=None):
+        """[(param, exp_avg, exp_avg_sq)] in param-id order: views of row `row` (default i) of the moment buffers src(name) (the
+        library's, or those of its state_dict), at each parameter's offset into its packed row."""
         L, i, out = self._library, self.index, []
         base = {'sf': L.online.detach()[i], 'w': L.w[i], 'h': L.h, 'g': L.g[i] if L.G is not None else None}
         for k, params in self._groups:
-            m, v = (src(name)[i] for name in self._MOMENTS[k])
+            m, v = (src(name)[i if row is None else row] for name in self._MOMENTS[k])
             for p in params:
                 off = (p.data.data_ptr() - base[k].data_ptr()) // 4
                 out.append((p, m[off:off + p.numel()].view_as(p), v[off:off + p.numel()].view_as(p)))
@@ -265,10 +265,10 @@ class PackedAdamView:
         L = self._library
         return self._torch_dict(lambda name: getattr(L, name), int(L.step[self.index]), clone=True)
 
-    def _torch_dict(self, src, step, clone=False):
+    def _torch_dict(self, src, step, clone=False, row=None):
         state = {}
         if step > 0:
-            for pid, (_, m, v) in enumerate(self._moments(src)):
+            for pid, (_, m, v) in enumerate(self._moments(src, row)):
                 state[pid] = dict(step=torch.tensor(float(step)), exp_avg=m.clone() if clone else m,
                                   exp_avg_sq=v.clone() if clone else v)
         groups, pid = [], 0
@@ -575,32 +575,55 @@ class DeepSF:
         psi_model.state_dict() key names and torch.optim.Adam.state_dict() -- built from VIEWS of sd['library']'s tensors, so
         torch.save stores the data once; load it into a reference psi_model / torch.optim.Adam to continue task i eagerly.
         load_state_dict reads sd['library'] only.  Everything a TSF library learns (g, h) lives in the library too.
+
+        On a policy-sharded library this is a collective over the shard's process group (PackedSFLibrary.state_dict): every
+        rank returns the same dict of ALL the group's tasks in global task order -- the format of one unsharded library
+        holding them, loadable at any GPU count.  GPI selects global task indices, so a gpi_counters row holds one count per
+        global task; rows shorter than that (built before the library was sharded) are padded with zeros.
         """
         lib = self._library
         lsd = lib.state_dict()
+        lo, n_total = self._task_range()
+        counters = [np.asarray(c).tolist() for c in self.gpi_counters]
+        updates = list(self.updates_since_target_updated)
+        if lib._sharded:
+            import torch.distributed as dist
+            parts = [None] * lib.shard.world
+            dist.all_gather_object(parts, (counters, updates), group=lib.shard.group)
+            counters, updates = [c for p in parts for c in p[0]], [u for p in parts for u in p[1]]
+        counters = [c + [0] * (n_total - len(c)) for c in counters]
         psi = []
-        for i in range(self.n_tasks):
-            (model, _, optim), _ = self.psi[i]
+        for i in range(n_total):
+            k = i - lo if lo <= i < lo + self.n_tasks else 0    # another rank's task: task 0's modules (one architecture)
+            (model, _, optim), _ = self.psi[k]
             names = {p: n for n, p in model.net.named_parameters()}
             weights = OrderedDict()
-            for (W, b), lin in zip(lib.spec.views(lsd['online'][i]), lib._views[i]['online']):
+            for (W, b), lin in zip(lib.spec.views(lsd['online'][i]), lib._views[k]['online']):
                 weights[names[lin.weight]], weights[names[lin.bias]] = W, b
-            psi.append(dict(model=weights, optim=optim._torch_dict(lsd.__getitem__, int(lsd['step'][i]))))
-        return dict(library=lsd, psi=psi, gpi_counters=[np.asarray(c).tolist() for c in self.gpi_counters],
-                    updates_since_target_updated=list(self.updates_since_target_updated), n_tasks=self.n_tasks,
+            psi.append(dict(model=weights, optim=optim._torch_dict(lsd.__getitem__, int(lsd['step'][i]), row=i)))
+        return dict(library=lsd, psi=psi, gpi_counters=counters, updates_since_target_updated=updates, n_tasks=n_total,
                     target_update_ev=self.target_update_ev)
 
     def load_state_dict(self, sd):
-        """Restore a state_dict() into a library that already holds the same tasks (add them first, as the saved run did)."""
+        """Restore a state_dict() into a library that already holds the same tasks (add them first, as the saved run did).
+        On a policy-sharded library every rank passes the same full dict of all the group's tasks and keeps its own."""
         for k in ('library', 'gpi_counters', 'updates_since_target_updated', 'n_tasks', 'target_update_ev'):
             if k not in sd:
                 raise ValueError(f"SF state_dict: missing key '{k}'")
-        if sd['n_tasks'] != self.n_tasks:
-            raise ValueError(f"SF state_dict: it holds {sd['n_tasks']} tasks, this library holds {self.n_tasks}")
+        lo, n_total = self._task_range()
+        if sd['n_tasks'] != n_total:
+            raise ValueError(f"SF state_dict: it holds {sd['n_tasks']} tasks, this library holds {n_total}")
         self._library.load_state_dict(sd['library'])
-        self.gpi_counters = [np.asarray(c, dtype=int) for c in sd['gpi_counters']]
-        self.updates_since_target_updated = list(sd['updates_since_target_updated'])
+        mine = slice(lo, lo + self.n_tasks)
+        self.gpi_counters = [np.asarray(c, dtype=int) for c in sd['gpi_counters'][mine]]
+        self.updates_since_target_updated = list(sd['updates_since_target_updated'][mine])
         self.target_update_ev = sd['target_update_ev']
+
+    def _task_range(self):
+        """(lo, n_total): this object's tasks are tasks [lo, lo + n_tasks) of the n_total of its library's shard group
+        ((0, n_tasks) unsharded)."""
+        lib = self._library
+        return (lib.shard.lo, lib.shard.n_total) if lib._sharded else (0, self.n_tasks)
 
 
 class SFDQN:
@@ -752,6 +775,7 @@ class SFDQN:
         active task with its episode in progress, and the target tasks' reward vectors with their optimizers.  As in torch, the
         random streams (Python `random`, numpy, torch) and the environments' own state are the caller's to save and restore.
         """
+        self._check_unsharded('state_dict')
         active = getattr(self, 'task_index', None)
         return dict(sf=self.sf.state_dict(), buffers=[b.state_dict() for b in self.buffers],
                     total_training_steps=self.total_training_steps, epsilon=getattr(self, 'epsilon', self.epsilon_init),
@@ -762,6 +786,7 @@ class SFDQN:
     def load_state_dict(self, sd):
         """Restore a state_dict() into an agent that already holds the same training tasks (reset() + add_training_task, as
         the saved run did).  Target tasks are rebuilt when the agent has none yet."""
+        self._check_unsharded('load_state_dict')
         if len(sd['buffers']) != len(self.buffers):
             raise ValueError(f"agent state_dict: it holds {len(sd['buffers'])} tasks, this agent holds {len(self.buffers)}")
         if self.test_tasks_weights and len(self.test_tasks_weights) != len(sd['test_tasks']):
@@ -778,6 +803,13 @@ class SFDQN:
         self.epsilon = sd['epsilon']
         for k, tsd in enumerate(sd['test_tasks']):
             self._load_test_task(k, tsd)
+
+    def _check_unsharded(self, what):
+        lib = getattr(self.sf, '_library', None)
+        if lib is not None and lib._sharded:
+            raise NotImplementedError(f'{type(self).__name__}.{what}() does not support policy-sharded libraries: the replay '
+                                      'rings are per rank.  Save and load the SF library with sf.state_dict() / '
+                                      'sf.load_state_dict(), collectively on every rank')
 
     def _new_test_task(self, feature_dim):
         """(w_approx, torch.optim.Adam over it) of one target task, as train() builds them."""
